@@ -15,9 +15,13 @@ throughput (1M = T x S points, sharded by point), the end-to-end numbers through
 the dominant kernel and the CPU baseline.
 
   python bench.py --gpus N --steps K --warmup W            # our arm (torchrun for N > 1)
+  python bench.py ... --dump-outputs DIR                   # also write the last timed step's results to DIR/*.npy
   python bench.py --impl reference --gpus N ...            # CPU arm: the reference's own PyTorch path (oracle/_ref, the
                                                            # unmodified `stnf` package) on the host cores, rank 0 only
   python bench.py --config 1|3|4|5 [--gpus N]              # the other BASELINE configs, one JSON line each (profiles/)
+
+The bench compiles nothing and writes nothing into the tree (it may be read-only): it runs the library that
+`__graft_entry__.build()` left there, so rebuild after changing a kernel.
 """
 import argparse
 import json
@@ -401,15 +405,34 @@ def profile_kernels(fn, iters):
         return None
 
 
+def dump_outputs(out_dir, tr):
+    """Write what the last training step handed its caller as float32 .npy files under out_dir: the step's loss
+    (`loss`), the model's state_dict after the step (`model.<key>`) and the EMA weights (`ema.<key>`).  The bench's
+    inputs are seeded, so two builds run with the same arguments can be compared file by file.  The backward kernels
+    sum gradients with float atomics in a run-dependent order and AdamW at lr 2e-2 amplifies those last bits, so two
+    runs of one build differ per array by up to 5e-7 relative L2 after 4 steps, 6e-6 after 23 and 0.4 after 520
+    (B200): compare builds at a small --steps."""
+    grab = lambda: {k: np.ascontiguousarray(v.detach().cpu().numpy(), dtype=np.float32)
+                    for k, v in tr.model.state_dict().items()}
+    arrays = {"loss": tr.loss_last.cpu().numpy().astype(np.float32)}
+    arrays.update({"model." + k: v for k, v in grab().items()})
+    tr.flat.apply_shadow()          # EMA weights swapped into the parameters by value, then swapped back
+    try:
+        arrays.update({"ema." + k: v for k, v in grab().items()})
+    finally:
+        tr.flat.restore()
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    return sum(a.nbytes for a in arrays.values())
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
-    import __graft_entry__ as ge
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
-    if rank == 0:
-        ge.build()
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
     log = lambda m: print(f"[bench r{rank}] {m}", file=sys.stderr, flush=True)
@@ -480,6 +503,8 @@ def run_ours(args):
     final_loss = tr.pop_loss_sum()
 
     log(f"timed region done: {dev_ms / args.steps:.4f} ms/step")
+    if args.dump_outputs and rank == 0:          # data-parallel replicas hold identical weights
+        log(f"last step's outputs: {dump_outputs(args.dump_outputs, tr)} bytes written to {args.dump_outputs}")
     # ---- end-to-end through the host-buffer API: per step H2D of the batch from pinned memory + D2H of the loss
     hb = 3 * 4 * BATCH + 4 * BATCH                 # coords (8 B) + t (4 B) + y (4 B) per sample
     # (lagged read-back: every step's batch is copied H2D and every step's loss read D2H inside the timed region; the
@@ -718,7 +743,13 @@ def main():
                     help="BASELINE.json config (1-based; 2 = the headline workload, the default)")
     ap.add_argument("--no-graph", action="store_true",
                     help="launch every kernel eagerly (for ncu: kernel replay cannot run inside stream capture)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's loss, weights and EMA weights to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.config != 2):
+        ap.error("--dump-outputs applies to the default workload (--impl ours, --config 2)")
     if args.batch != BATCH:
         WORKLOAD = WORKLOAD.replace(f"batch {BATCH}/GPU", f"batch {args.batch}/GPU").replace(
             "80k train samples", f"{max(N_TRAIN, 4 * args.batch)} train samples")

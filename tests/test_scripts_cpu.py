@@ -214,3 +214,36 @@ def test_gmm_fit_is_shared_between_processes_through_files(tmp_path, monkeypatch
     assert not calls and np.array_equal(m1, m2) and np.array_equal(c1, c2)
     m3, _ = ki._gmm_fit(sub, 4)                 # a different k is a different fit
     assert calls and m3.shape == (4, 2)
+
+
+def test_bench_dump_outputs(tmp_path):
+    """`bench.py --dump-outputs DIR`: the last step's loss, the model's state_dict and the EMA weights as float32 .npy
+    files under the upstream state_dict names, leaving the live weights as they were; the option and --steps are
+    checked before any work starts."""
+    import os
+    import subprocess
+    import sys
+    import types
+    import bench
+    from stnf.models import STInterpMLP
+    from st_dadk_b200.trainer import FlatState
+    torch.manual_seed(0)
+    model = STInterpMLP(k_spatial_centers=[9, 25], k_temporal_centers=[4], hidden_dims=[32, 16])
+    fl = FlatState(model, "cpu")
+    fl.shadow.mul_(0.5)
+    p0 = fl.p.clone()
+    nbytes = bench.dump_outputs(str(tmp_path), types.SimpleNamespace(model=model, flat=fl, loss_last=torch.tensor([0.25])))
+    assert torch.equal(fl.p, p0)
+    keys = set(model.state_dict())
+    assert {f[:-len(".npy")] for f in os.listdir(tmp_path)} == {"loss"} | {"model." + k for k in keys} | {"ema." + k for k in keys}
+    assert nbytes == 4 * (1 + 2 * sum(v.numel() for v in model.state_dict().values()))
+    w = np.load(tmp_path / "model.mlp.0.weight.npy")
+    assert w.dtype == np.float32 and np.array_equal(w, model.mlp[0].weight.detach().numpy())
+    assert np.array_equal(np.load(tmp_path / "ema.mlp.0.weight.npy"), 0.5 * w)
+    assert np.load(tmp_path / "loss.npy").tolist() == [0.25]
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    for bad in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", str(tmp_path / "x")],
+                ["--config", "3", "--dump-outputs", str(tmp_path / "x")]):
+        r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), *bad], capture_output=True, text=True, timeout=60)
+        assert r.returncode == 2 and "error" in r.stderr, (bad, r.stderr)
+    assert not (tmp_path / "x").exists()
