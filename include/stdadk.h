@@ -219,7 +219,7 @@ int stdadk_version(void);
 const char* stdadk_last_error(void);
 /* sizeof() of the argument structs, for bindings to verify their layout:
  * 0 basis, 1 points, 2 layer, 3 dropout, 4 head, 5 fwd_args, 6 bwd_args, 7 wgrad_args, 8 knotgrad_args, 9 adamw_args,
- * 10 pack_desc, 11 sparse_args, 12 predict_args, 13 train_fwd_args, 14 peer_allreduce_args, 15 field_args */
+ * 10 pack_desc, 11 sparse_args, 12 predict_args, 13 unused (returns 0), 14 peer_allreduce_args, 15 field_args */
 size_t stdadk_sizeof(int which);
 
 size_t stdadk_image_floats(int64_t rows, int64_t cols);
@@ -330,20 +330,6 @@ typedef struct {
 } stdadk_field_args;
 int stdadk_predict_field_supported(const stdadk_field_args* a);   /* 1 yes, 0 no (reason in stdadk_last_error) */
 int stdadk_predict_field(const stdadk_field_args* a, void* stream);
-
-/* Forward of a TRAINING step through the same whole-network kernel (STInterpMLP.forward in train mode + the loss of
- * train_st_interp.py:620-631): one launch instead of one stdadk_layer_fwd per block.  Besides y_hat it applies
- * dropout, accumulates the loss, writes dLoss/dy_hat, and leaves what stdadk_layer_bwd / stdadk_wgrad read:
- * h_img[l] = image of block l's output (l < n_layers-1), and per block either x_img[l] (pre-LayerNorm x, see
- * stdadk_fwd_args.x_img) and/or stats[l] (rows x 2 mean, rstd).  Same shape limits as stdadk_predict. */
-typedef struct {
-    stdadk_predict_args net;                 /* net.head carries y, loss_type, taus, inv_count, dyhat, loss_acc */
-    stdadk_dropout drop;
-    float* h_img[STDADK_MAX_HIDDEN];
-    float* x_img[STDADK_MAX_HIDDEN];         /* optional (NULL) */
-    float* stats[STDADK_MAX_HIDDEN];         /* optional (NULL) */
-} stdadk_train_fwd_args;
-int stdadk_train_fwd(const stdadk_train_fwd_args* a, void* stream);
 
 int stdadk_layer_fwd(const stdadk_fwd_args* a, void* stream);
 int stdadk_layer_bwd(const stdadk_bwd_args* a, void* stream);

@@ -117,11 +117,6 @@ class PeerAllreduceArgs(C.Structure):
                 ("sqnorms", fp), ("workspace", fp)]
 
 
-class TrainFwdArgs(C.Structure):
-    _fields_ = [("net", PredictArgs), ("drop", Dropout), ("h_img", fp * MAX_HIDDEN), ("x_img", fp * MAX_HIDDEN),
-                ("stats", fp * MAX_HIDDEN)]
-
-
 _lib = None
 
 _PROTOS = {
@@ -137,7 +132,6 @@ _PROTOS = {
     "stdadk_pack_images": (C.c_int, [C.POINTER(PackDesc), C.c_int, fp]),
     "stdadk_predict_supported": (C.c_int, [C.POINTER(PredictArgs)]),
     "stdadk_predict": (C.c_int, [C.POINTER(PredictArgs), fp]),
-    "stdadk_train_fwd": (C.c_int, [C.POINTER(TrainFwdArgs), fp]),
     "stdadk_predict_field_supported": (C.c_int, [C.POINTER(FieldArgs)]),
     "stdadk_predict_field": (C.c_int, [C.POINTER(FieldArgs), fp]),
     "stdadk_peer_allreduce": (C.c_int, [C.POINTER(PeerAllreduceArgs), fp]),
@@ -171,9 +165,11 @@ def lib():
             fn = getattr(L, name)
             fn.restype = res
             fn.argtypes = args
-        structs = [Basis, Points, Layer, Dropout, Head, FwdArgs, BwdArgs, WgradArgs, KnotGradArgs, AdamWArgs, PackDesc, SparseArgs,
-                   PredictArgs, TrainFwdArgs, PeerAllreduceArgs, FieldArgs]
-        for i, st in enumerate(structs):
+        # (stdadk_sizeof index, struct); index 13 is unused
+        structs = [(0, Basis), (1, Points), (2, Layer), (3, Dropout), (4, Head), (5, FwdArgs), (6, BwdArgs), (7, WgradArgs),
+                   (8, KnotGradArgs), (9, AdamWArgs), (10, PackDesc), (11, SparseArgs), (12, PredictArgs),
+                   (14, PeerAllreduceArgs), (15, FieldArgs)]
+        for i, st in structs:
             if L.stdadk_sizeof(i) != C.sizeof(st):
                 raise RuntimeError(f"libstdadk ABI mismatch: {st.__name__} is {C.sizeof(st)} B in the binding, "
                                    f"{L.stdadk_sizeof(i)} B in the library")

@@ -3,7 +3,6 @@
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
-#include <cstdlib>
 
 #include "layer.cuh"
 #include "misc.cuh"
@@ -166,7 +165,6 @@ size_t stdadk_sizeof(int which) {
         case 10: return sizeof(stdadk_pack_desc);
         case 11: return sizeof(stdadk_sparse_args);
         case 12: return sizeof(stdadk_predict_args);
-        case 13: return sizeof(stdadk_train_fwd_args);
         case 14: return sizeof(stdadk_peer_allreduce_args);
         case 15: return sizeof(stdadk_field_args);
         default: return 0;
@@ -318,52 +316,46 @@ int stdadk_layer_fwd(const stdadk_fwd_args* a, void* stream) {
     REQUIRE(sp.total <= 227 * 1024, "layer_fwd: needs %u B of shared memory (> 227 KB): too many knots for the dense path",
             sp.total);
     K.n_tiles = tiles;
-    // Optional (STDADK_CLUSTER=1): clusters of 4 CTAs share every weight slab by multicast (L2 -> SM weight traffic / 4).
-    // Bit-identical output, but measured SLOWER on B200 (1M-point prediction 2.25 ms vs 2.03 ms): the kernels are
-    // issue/latency-bound, not L2-bound, and the cluster couples four tiles' pipelines.  Kept for L2-bound shapes.
-    constexpr int FCL = 4;
 #define LAUNCH_FWD(B, C)                                                                                     \
     do {                                                                                                     \
-        if (int r = set_smem(layer_fwd_kernel<B, C, (C == 2 ? 2 : 4), 1>, sp.total)) return r;               \
-        layer_fwd_kernel<B, C, (C == 2 ? 2 : 4), 1><<<tiles, n_threads(C), sp.total, (cudaStream_t)stream>>>(K); \
+        if (int r = set_smem(layer_fwd_kernel<B, C, (C == 2 ? 2 : 4)>, sp.total)) return r;                  \
+        layer_fwd_kernel<B, C, (C == 2 ? 2 : 4)><<<tiles, n_threads(C), sp.total, (cudaStream_t)stream>>>(K); \
     } while (0)
-#define LAUNCH_FWD_CLUSTER(B)                                                                                \
-    do {                                                                                                     \
-        if (int r = set_smem(layer_fwd_kernel<B, 2, 2, FCL>, sp.total)) return r;                            \
-        cudaLaunchConfig_t cfg{};                                                                            \
-        cfg.gridDim = dim3((unsigned)((tiles + FCL - 1) / FCL * FCL));                                       \
-        cfg.blockDim = dim3(n_threads(2));                                                                   \
-        cfg.dynamicSmemBytes = sp.total;                                                                     \
-        cfg.stream = (cudaStream_t)stream;                                                                   \
-        cudaLaunchAttribute at[1];                                                                           \
-        at[0].id = cudaLaunchAttributeClusterDimension;                                                      \
-        at[0].val.clusterDim.x = FCL;                                                                        \
-        at[0].val.clusterDim.y = 1;                                                                          \
-        at[0].val.clusterDim.z = 1;                                                                          \
-        cfg.attrs = at;                                                                                      \
-        cfg.numAttrs = 1;                                                                                    \
-        cudaError_t e = cudaLaunchKernelEx(&cfg, layer_fwd_kernel<B, 2, 2, FCL>, K);                         \
-        if (e != cudaSuccess) return fail((int)e, "layer_fwd (cluster launch): %s", cudaGetErrorString(e));  \
-    } while (0)
-    const char* cl_env = getenv("STDADK_CLUSTER");
-    const bool use_cluster = cg == 2 && cl_env != nullptr && cl_env[0] == '1';
     if (basis) {
-        if (use_cluster) LAUNCH_FWD_CLUSTER(true);
-        else if (cg == 2) LAUNCH_FWD(true, 2);
+        if (cg == 2) LAUNCH_FWD(true, 2);
         else LAUNCH_FWD(true, 4);
     } else {
-        if (use_cluster) LAUNCH_FWD_CLUSTER(false);
-        else if (cg == 2) LAUNCH_FWD(false, 2);
+        if (cg == 2) LAUNCH_FWD(false, 2);
         else LAUNCH_FWD(false, 4);
     }
 #undef LAUNCH_FWD
-#undef LAUNCH_FWD_CLUSTER
     return check_launch("layer_fwd");
 }
 
 // Development aid (not part of include/stdadk.h): 16 device counters of cycles the fused prediction kernel's roles spend
 // waiting; see tools/prof_predict.py.
 extern "C" void stdadk_debug_counters(void* dev_u64x16) { g_predict_dbg = static_cast<unsigned long long*>(dev_u64x16); }
+
+// The hidden blocks of the whole-network kernels: each block's n_in must be the previous block's n_out.
+static int fill_pred_layers(const stdadk_layer* layers, int n_layers, PredLayerP* out, const char* who) {
+    for (int l = 0; l < n_layers; ++l) {
+        const stdadk_layer& y = layers[l];
+        if (int r = check_layer(y, who)) return r;
+        REQUIRE(l == 0 || y.n_in == layers[l - 1].n_out, "%s: block %d n_in=%d != previous n_out=%d", who, l, y.n_in,
+                layers[l - 1].n_out);
+        PredLayerP& L = out[l];
+        L.w_img = y.w_img;
+        L.bias = y.bias;
+        L.gamma = y.gamma;
+        L.beta = y.beta;
+        L.n_out = y.n_out;
+        L.n_pad = pad32(y.n_out);
+        L.k_slabs = pad32(y.n_in) / SLAB_K;
+        L.has_ln = y.gamma != nullptr;
+        L.eps = y.ln_eps;
+    }
+    return 0;
+}
 
 static int predict_fill(const stdadk_predict_args* a, PredK* K) {
     REQUIRE(a && a->basis && a->head, "predict: NULL args / basis / head");
@@ -380,22 +372,7 @@ static int predict_fill(const stdadk_predict_args* a, PredK* K) {
     K->head_w = a->head->w;
     K->head_b = a->head->b;
     K->yhat = a->head->yhat;
-    for (int l = 0; l < a->n_layers; ++l) {
-        const stdadk_layer& y = a->layers[l];
-        if (int r = check_layer(y, "predict")) return r;
-        REQUIRE(l == 0 || y.n_in == a->layers[l - 1].n_out, "predict: block %d n_in=%d != previous n_out=%d", l, y.n_in,
-                a->layers[l - 1].n_out);
-        PredLayerP& L = K->L[l];
-        L.w_img = y.w_img;
-        L.bias = y.bias;
-        L.gamma = y.gamma;
-        L.beta = y.beta;
-        L.n_out = y.n_out;
-        L.n_pad = pad32(y.n_out);
-        L.k_slabs = pad32(y.n_in) / SLAB_K;
-        L.has_ln = y.gamma != nullptr;
-        L.eps = y.ln_eps;
-    }
+    if (int r = fill_pred_layers(a->layers, a->n_layers, K->L, "predict")) return r;
     uint32_t bytes = plan_predict(*K);
     REQUIRE(bytes <= 227 * 1024, "predict: the fused kernel needs %u B of shared memory (> 227 KB) for this shape", bytes);
     K->n_tiles = (int)ceil_div64(a->pts.n_rows, TILE_M);
@@ -413,10 +390,10 @@ int stdadk_predict(const stdadk_predict_args* a, void* stream) {
     PredK Kl;
     if (int r = predict_fill(a, &Kl)) return r;
     if (a->pts.n_rows <= 0) return 0;
-    if (int r = set_smem(predict_fused_kernel<false>, Kl.sm.total)) return r;
+    if (int r = set_smem(predict_fused_kernel, Kl.sm.total)) return r;
     const int sms = g_sm_count > 0 ? g_sm_count : 148;
     const int grid = Kl.n_tiles < sms ? Kl.n_tiles : sms;
-    predict_fused_kernel<false><<<grid, PF_NT, Kl.sm.total, (cudaStream_t)stream>>>(Kl);
+    predict_fused_kernel<<<grid, PF_NT, Kl.sm.total, (cudaStream_t)stream>>>(Kl);
     return check_launch("predict");
 }
 
@@ -462,22 +439,7 @@ static int field_fill(const stdadk_field_args* a, FieldK* K) {
     K->out_k_stride = a->out_k_stride > 0 ? a->out_k_stride : a->n_sites;
     K->zt = a->zt_ws;
     K->dbg = g_predict_dbg;
-    for (int l = 0; l < a->n_layers; ++l) {
-        const stdadk_layer& y = a->layers[l];
-        if (int r = check_layer(y, "predict_field")) return r;
-        REQUIRE(l == 0 || y.n_in == a->layers[l - 1].n_out, "predict_field: block %d n_in=%d != previous n_out=%d", l, y.n_in,
-                a->layers[l - 1].n_out);
-        PredLayerP& L = K->L[l];
-        L.w_img = y.w_img;
-        L.bias = y.bias;
-        L.gamma = y.gamma;
-        L.beta = y.beta;
-        L.n_out = y.n_out;
-        L.n_pad = pad32(y.n_out);
-        L.k_slabs = pad32(y.n_in) / SLAB_K;
-        L.has_ln = y.gamma != nullptr;
-        L.eps = y.ln_eps;
-    }
+    if (int r = fill_pred_layers(a->layers, a->n_layers, K->L, "predict_field")) return r;
     REQUIRE(K->L[0].k_slabs <= PF_HSLABS, "predict_field: %d spatial knots exceed the resident operand (%d)", b->k_s,
             PF_HSLABS * SLAB_K);
     uint32_t bytes = plan_field(*K);
@@ -526,39 +488,6 @@ int stdadk_predict_field(const stdadk_field_args* a, void* stream) {
     const int grid = K.n_units < sms ? K.n_units : sms;
     predict_field_kernel<<<grid, PF_NT, K.sm.total, (cudaStream_t)stream>>>(K);
     return check_launch("predict_field");
-}
-
-int stdadk_train_fwd(const stdadk_train_fwd_args* a, void* stream) {
-    if (int r = check_device()) return r;
-    REQUIRE(a, "train_fwd: NULL args");
-    PredK Kl;
-    if (int r = predict_fill(&a->net, &Kl)) return r;
-    const stdadk_head* h = a->net.head;
-    REQUIRE(h->loss_type == STDADK_LOSS_NONE || (h->y && h->loss_acc), "train_fwd: loss requested without y / loss_acc");
-    REQUIRE(a->drop.p >= 0.0f && a->drop.p < 1.0f, "train_fwd: dropout p=%f", a->drop.p);
-    for (int l = 0; l < a->net.n_layers; ++l) {
-        REQUIRE(l == a->net.n_layers - 1 || a->h_img[l], "train_fwd: h_img[%d] is NULL (the backward of block %d reads it)", l,
-                l + 1);
-        REQUIRE(((reinterpret_cast<uintptr_t>(a->h_img[l]) | reinterpret_cast<uintptr_t>(a->x_img[l])) & 127) == 0,
-                "train_fwd: images must be 128-byte aligned");
-        Kl.h_img[l] = l < a->net.n_layers - 1 ? a->h_img[l] : nullptr;
-        Kl.x_img[l] = a->x_img[l];
-        Kl.stats[l] = a->stats[l];
-    }
-    if (a->net.pts.n_rows <= 0) return 0;
-    Kl.head = to_head(h);
-    Kl.seed = a->drop.seed;
-    Kl.key_offset = a->drop.key_offset;
-    Kl.step_ptr = a->drop.step_ptr;
-    Kl.step = a->drop.step;
-    Kl.drop_p = a->drop.p;
-    Kl.thresh16 = dropout_thresh16(a->drop.p);
-    Kl.drop_scale = a->drop.p > 0.0f ? 1.0f / (1.0f - a->drop.p) : 1.0f;
-    if (int r = set_smem(predict_fused_kernel<true>, Kl.sm.total)) return r;
-    const int sms = g_sm_count > 0 ? g_sm_count : 148;
-    const int grid = Kl.n_tiles < sms ? Kl.n_tiles : sms;
-    predict_fused_kernel<true><<<grid, PF_NT, Kl.sm.total, (cudaStream_t)stream>>>(Kl);
-    return check_launch("train_fwd");
 }
 
 int stdadk_layer_bwd(const stdadk_bwd_args* a, void* stream) {

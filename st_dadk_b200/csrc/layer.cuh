@@ -373,27 +373,6 @@ __device__ __forceinline__ void stage_knots_async(const BasisP& B, float4* sk, f
     if (B.k_t & 1) st[B.k_t - 1] = B.tknots[B.k_t - 1];
 }
 
-// Cluster variant: the CL CTAs of a cluster work on different row tiles but need the same weight slab; CTA `rank`
-// fetches 1/CL of its rows and multicasts them to all, so the slab crosses L2 -> SM once per cluster instead of once
-// per CTA.  Every CTA's barrier still expects the whole slab (+ its own A slab).
-template <int CL>
-__device__ __forceinline__ void issue_slab_copies_cluster(const float* w_img, int w_slabs, int slab, int n_pad,
-                                                          const float* a_tile_img, float* sA, float* sB, uint64_t* bar,
-                                                          uint32_t rank) {
-    uint32_t bytes = (uint32_t)n_pad * 128u + (a_tile_img ? (uint32_t)SLAB_BYTES : 0u);
-    mbar_arrive_expect_tx(bar, bytes);
-    const int per = n_pad / CL;                    // n_pad is a multiple of 32, CL of {2, 4}
-    int r0 = (int)rank * per;
-    const int r_end = r0 + per;
-    while (r0 < r_end) {                           // split at 128-row image tiles
-        int rows = min(r_end - r0, TILE_M - (r0 % TILE_M));
-        const float* src = w_img + ((size_t)(r0 / TILE_M) * w_slabs + slab) * SLAB_FLOATS + (size_t)(r0 % TILE_M) * SLAB_K;
-        bulk_g2s_mcast(sB + (size_t)r0 * SLAB_K, src, (uint32_t)rows * 128u, bar, (uint16_t)((1u << CL) - 1u));
-        r0 += rows;
-    }
-    if (a_tile_img) bulk_g2s(sA, a_tile_img + (size_t)slab * SLAB_FLOATS, SLAB_BYTES, bar);
-}
-
 // MMA issuer: one 128-byte K slab = 4 MMAs of K=8 (TF32), advancing 32 bytes inside the swizzle atom.
 __device__ __forceinline__ void issue_slab_mma(uint32_t tmem_acc, const float* sA, const float* sB, uint32_t idesc,
                                                bool first) {
@@ -610,7 +589,7 @@ __device__ __forceinline__ void pf_head_partial(const float (&v)[32], const floa
 // =============================================================================================
 // Epilogue of a forward block for one thread = (row, column group): two passes over the accumulator in tensor memory
 // (a thread owns 256 / CG columns, more than the register file holds at two CTAs per SM), each on whole 32-column chunks
-// in registers with packed FP32 math.  Shared by layer_fwd_kernel and layer_fwd_lattice_kernel.
+// in registers with packed FP32 math.
 struct EpiCtx {
     const float* sbias;
     const float* sgam;
@@ -756,10 +735,9 @@ __device__ __forceinline__ void fwd_epilogue(const FwdK& P, const EpiCtx& E) {
     }
 }
 
-template <bool BASIS, int CG, int NS, int CL>
+template <bool BASIS, int CG, int NS>
 __global__ void __launch_bounds__(n_threads(CG), CG <= 2 ? 2 : 1) layer_fwd_kernel(const __grid_constant__ FwdK P) {
     constexpr int NW = n_work(CG), NT = n_threads(CG), NSTAGE = NS;
-    constexpr uint16_t CMASK = (uint16_t)((1u << CL) - 1u);
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = align_smem(smem_raw);
     const SmemPlan sp = plan_smem(P.n_pad, P.has_head ? P.head.q : 0, BASIS ? P.basis.k_s : 0,
@@ -786,9 +764,11 @@ __global__ void __launch_bounds__(n_threads(CG), CG <= 2 ? 2 : 1) layer_fwd_kern
         atomicAdd(P.dbg + 8, 1ull);
     }
 #endif
-    const bool tile_valid = (int)blockIdx.x < P.n_tiles;       // a cluster may be padded with a tile-less CTA
+    // The grid has one CTA per tile, so tile_valid always holds.  It stays, with the tests it feeds, because ptxas
+    // allocates registers better with it: without it the row index of layer_fwd_kernel<true, 2, 2> spills and a
+    // 1M-row launch took 0.812 ms instead of 0.789 ms (B200, 1000 W power limit).
+    const bool tile_valid = (int)blockIdx.x < P.n_tiles;
     const int tile = tile_valid ? (int)blockIdx.x : P.n_tiles - 1;
-    const uint32_t crank = CL > 1 ? cluster_ctarank() : 0u;
     const int n_pad = P.n_pad, n_out = P.L.n_out;
     const bool has_ln = P.L.gamma != nullptr;
     const size_t b_stage_floats = (size_t)n_pad * SLAB_K;
@@ -796,7 +776,7 @@ __global__ void __launch_bounds__(n_threads(CG), CG <= 2 ? 2 : 1) layer_fwd_kern
     if (tid == NW) {
         for (int s = 0; s < NSTAGE; ++s) {
             mbar_init(&full[s], BASIS ? 1 + NW / 32 : 1);
-            mbar_init(&empty[s], CL);        // every CTA of the cluster must have consumed the stage
+            mbar_init(&empty[s], 1);
         }
         mbar_init(accf, 1);
         mbar_fence_init();
@@ -821,7 +801,6 @@ __global__ void __launch_bounds__(n_threads(CG), CG <= 2 ? 2 : 1) layer_fwd_kern
     }
     tc_fence_before();
     __syncthreads();
-    if (CL > 1) cluster_sync_all();                // peers' barriers are initialised before anything remote arrives
     tc_fence_after();
     const uint32_t tmem_base = *tmem_slot;
     FWD_T(0);       // prologue
@@ -837,12 +816,8 @@ __global__ void __launch_bounds__(n_threads(CG), CG <= 2 ? 2 : 1) layer_fwd_kern
                 if (it > 0) FWD_WAIT(7, mbar_wait(&empty[stage], (it - 1) & 1));
                 const float* w_src = pass_b_lo(p) ? P.L.w_img_lo : P.L.w_img;
                 const float* a_tile = BASIS ? nullptr : (pass_a_lo(p) ? P.a_img_lo : P.a_img) + a_off;
-                if (CL > 1)
-                    issue_slab_copies_cluster<CL>(w_src, P.k_slabs, s, n_pad, a_tile, sA + (size_t)stage * SLAB_FLOATS,
-                                                  sB + stage * b_stage_floats, &full[stage], crank);
-                else
-                    issue_slab_copies(w_src, P.k_slabs, s, n_pad, a_tile, sA + (size_t)stage * SLAB_FLOATS,
-                                      sB + stage * b_stage_floats, &full[stage]);
+                issue_slab_copies(w_src, P.k_slabs, s, n_pad, a_tile, sA + (size_t)stage * SLAB_FLOATS,
+                                  sB + stage * b_stage_floats, &full[stage]);
             }
         }
         __syncwarp();
@@ -857,8 +832,7 @@ __global__ void __launch_bounds__(n_threads(CG), CG <= 2 ? 2 : 1) layer_fwd_kern
                 tc_fence_after();
                 issue_slab_mma(tmem_base, sA + (size_t)stage * SLAB_FLOATS, sB + stage * b_stage_floats, idesc,
                                s == 0);
-                if (CL > 1) umma_commit_mcast(&empty[stage], CMASK);
-                else umma_commit(&empty[stage]);
+                umma_commit(&empty[stage]);
             }
             umma_commit(accf);
         }
@@ -917,7 +891,6 @@ __global__ void __launch_bounds__(n_threads(CG), CG <= 2 ? 2 : 1) layer_fwd_kern
         FWD_T(3);   // epilogue
     }
     __syncthreads();
-    if (CL > 1) cluster_sync_all();                // no peer may still multicast into / arrive on this CTA's memory
     if (warp == 4 * CG) tmem_dealloc(tmem_base, (uint32_t)P.tmem_cols);
     FWD_T(4);       // tail
 }

@@ -48,15 +48,6 @@ struct PredK {
     float* yhat;
     int n_layers, q, n_tiles, _pad;
     unsigned long long* dbg;                // optional cycle counters (stdadk_debug_counters), NULL in production
-    // ---- training forward only (predict_fused_kernel<true>): what the backward kernels read
-    float* h_img[PF_MAX_LAYERS];            // image of block l's output (post dropout, TF32), l < n_layers - 1
-    float* x_img[PF_MAX_LAYERS];            // optional image of the pre-LayerNorm x of block l
-    float* stats[PF_MAX_LAYERS];            // optional (rows x 2) LayerNorm mean, rstd of block l
-    HeadP head;                             // y, loss, dyhat, loss_acc
-    unsigned long long seed, key_offset;
-    const int* step_ptr;
-    unsigned int step, thresh16;
-    float drop_scale, drop_p;
 };
 
 // Development aid, compiled in with -DSTDADK_PF_DEBUG: cycles each role spends waiting / per phase, accumulated
@@ -115,15 +106,6 @@ __device__ __forceinline__ void pf_gen_slab(const BasisP& B, const float4* sk, c
     }
 }
 
-// the TF32-rounded chunk into a global operand image (what the next block / wgrad of the layered path read)
-__device__ __forceinline__ void pf_store_image_tf32(float* img, int tile, int slabs, int c0, uint32_t row, const float (&v)[32]) {
-    uint8_t* dst = reinterpret_cast<uint8_t*>(img + ((size_t)tile * slabs + (c0 / SLAB_K)) * SLAB_FLOATS);
-#pragma unroll
-    for (int c = 0; c < 8; ++c)
-        *reinterpret_cast<float4*>(dst + swz_off(row, c)) =
-            make_float4(to_tf32(v[4 * c]), to_tf32(v[4 * c + 1]), to_tf32(v[4 * c + 2]), to_tf32(v[4 * c + 3]));
-}
-
 __device__ __forceinline__ void pf_store_slab(const float (&v)[32], uint32_t slab_saddr, uint32_t rowoff, uint32_t rx) {
 #pragma unroll
     for (int c = 0; c < 8; ++c)
@@ -131,10 +113,7 @@ __device__ __forceinline__ void pf_store_slab(const float (&v)[32], uint32_t sla
                      to_tf32(v[4 * c + 2]), to_tf32(v[4 * c + 3]));
 }
 
-// TRAIN = false: prediction (eval mode, nothing but y_hat leaves the SM).  TRAIN = true: the forward of a training
-// step -- same pipeline, plus dropout, the loss / dLoss/dy_hat of the fused head and the tensors the backward kernels
-// read (activation images, pre-LayerNorm x or LayerNorm statistics) -- one launch instead of one per block.
-template <bool TRAIN>
+// Eval mode: no dropout, and nothing but y_hat leaves the SM.
 __global__ void __launch_bounds__(PF_NT, 1) predict_fused_kernel(const __grid_constant__ PredK P) {
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = align_smem(smem_raw);
@@ -317,8 +296,6 @@ __global__ void __launch_bounds__(PF_NT, 1) predict_fused_kernel(const __grid_co
         mbar_wait(kbar, 0);
         long long lrow = 0, nxt_lrow = 0;
         bool rvalid = false, nxt_valid = false, have_cur = false;
-        int cur_tile = 0;
-        const uint32_t drop_step = (TRAIN && P.drop_p > 0.0f) ? (P.step_ptr ? (uint32_t)(*P.step_ptr) : P.step) : 0u;
         uint32_t it = 0;                                   // iteration index of the current tile
         for (int next = blockIdx.x; have_cur || next < P.n_tiles; next += gridDim.x) {
             const bool have_next = next < P.n_tiles;
@@ -371,13 +348,6 @@ __global__ void __launch_bounds__(PF_NT, 1) predict_fused_kernel(const __grid_co
                 const bool ha = c0a < Ly.n_pad, hb = c0b < Ly.n_pad;
                 const int nva = min(32, Ly.n_out - c0a), nvb = min(32, Ly.n_out - c0b);
                 float4* redl = red + (size_t)(accn & 1u) * (PF_CG * TILE_M);
-                const bool drop = TRAIN && P.drop_p > 0.0f;
-                uint32_t keep_a = 0xFFFFFFFFu, keep_b = 0xFFFFFFFFu;
-                if (drop) {
-                    const unsigned long long key_row = P.key_offset + (unsigned long long)lrow;
-                    if (ha) keep_a = pf_keep_mask(P.seed, drop_step, (uint32_t)l, key_row, c0a, P.thresh16);
-                    if (hb) keep_b = pf_keep_mask(P.seed, drop_step, (uint32_t)l, key_row, c0b, P.thresh16);
-                }
                 PF_TIMED_WAIT(w_acc, mbar_wait(&accf[it & 1u], ((it >> 1) * (uint32_t)nl + (uint32_t)l) & 1u));
                 PF_DBG(if (P.dbg) t_last = clock64();)
                 ++accn;
@@ -405,10 +375,6 @@ __global__ void __launch_bounds__(PF_NT, 1) predict_fused_kernel(const __grid_co
                 float K = 0.0f, S1 = 0.0f, S2 = 0.0f;
                 if (ha) pf_bias_stats(va, sb + c0a, nva, have, K, S1, S2);
                 if (hb) pf_bias_stats(vb, sb + c0b, nvb, have, K, S1, S2);
-                if (TRAIN && P.x_img[l]) {         // x = A W^T + b, FP32: a backward that gets it skips its recompute GEMM
-                    if (ha) image_store_chunk(P.x_img[l], cur_tile, Ly.n_pad / SLAB_K, c0a, (uint32_t)row, va);
-                    if (hb) image_store_chunk(P.x_img[l], cur_tile, Ly.n_pad / SLAB_K, c0b, (uint32_t)row, vb);
-                }
                 float rstd = 1.0f, nmr = 0.0f;
                 if (Ly.has_ln) {
                     const float cntv = (float)((ha ? max(nva, 0) : 0) + (hb ? max(nvb, 0) : 0));
@@ -434,29 +400,20 @@ __global__ void __launch_bounds__(PF_NT, 1) predict_fused_kernel(const __grid_co
                         }
                         rstd = 1.0f / sqrtf(fmaxf(m2 * inv_n, 0.0f) + Ly.eps);
                         nmr = -mean * rstd;
-                        if (TRAIN && P.stats[l] && rvalid && cg == 0) {
-                            P.stats[l][2 * lrow] = mean;
-                            P.stats[l][2 * lrow + 1] = rstd;
-                        }
                     }
                 } else {
                     worker_barrier(PF_NW);   // every thread has seen this accumulator phase before the next can complete
                 }
-                const int nva_e = (TRAIN && !rvalid) ? 0 : nva, nvb_e = (TRAIN && !rvalid) ? 0 : nvb;   // padding rows -> 0
                 if (l + 1 < nl) {
                     if (ha) {
-                        pf_normalize(va, sg + c0a, sbt + c0a, Ly.has_ln != 0, rstd, nmr, nva_e);
-                        if (drop) pf_dropout(va, keep_a, P.drop_scale);
-                        if (TRAIN && P.h_img[l]) pf_store_image_tf32(P.h_img[l], cur_tile, Ly.n_pad / SLAB_K, c0a, (uint32_t)row, va);
+                        pf_normalize(va, sg + c0a, sbt + c0a, Ly.has_ln != 0, rstd, nmr, nva);
                         pf_store_slab(va, sH_addr + (uint32_t)cg * SLAB_BYTES, rowoff, rx);
                         fence_proxy_async_smem();
                         tc_fence_before();
                         mbar_arrive_warp(&hfull[cg]);
                     }
                     if (hb) {
-                        pf_normalize(vb, sg + c0b, sbt + c0b, Ly.has_ln != 0, rstd, nmr, nvb_e);
-                        if (drop) pf_dropout(vb, keep_b, P.drop_scale);
-                        if (TRAIN && P.h_img[l]) pf_store_image_tf32(P.h_img[l], cur_tile, Ly.n_pad / SLAB_K, c0b, (uint32_t)row, vb);
+                        pf_normalize(vb, sg + c0b, sbt + c0b, Ly.has_ln != 0, rstd, nmr, nvb);
                         pf_store_slab(vb, sH_addr + (uint32_t)(cg + 4) * SLAB_BYTES, rowoff, rx);
                         fence_proxy_async_smem();
                         tc_fence_before();
@@ -468,48 +425,27 @@ __global__ void __launch_bounds__(PF_NT, 1) predict_fused_kernel(const __grid_co
 #pragma unroll
                     for (int k = 0; k < STDADK_MAX_Q; ++k) yh[k] = 0.0f;
                     if (ha) {
-                        pf_normalize(va, sg + c0a, sbt + c0a, Ly.has_ln != 0, rstd, nmr, nva_e);
-                        if (drop) pf_dropout(va, keep_a, P.drop_scale);
+                        pf_normalize(va, sg + c0a, sbt + c0a, Ly.has_ln != 0, rstd, nmr, nva);
                         pf_head_partial(va, shw, Ly.n_pad, c0a, P.q, yh);
                     }
                     if (hb) {
-                        pf_normalize(vb, sg + c0b, sbt + c0b, Ly.has_ln != 0, rstd, nmr, nvb_e);
-                        if (drop) pf_dropout(vb, keep_b, P.drop_scale);
+                        pf_normalize(vb, sg + c0b, sbt + c0b, Ly.has_ln != 0, rstd, nmr, nvb);
                         pf_head_partial(vb, shw, Ly.n_pad, c0b, P.q, yh);
                     }
                     float* mine = hscr + ((size_t)cg * TILE_M + row) * STDADK_MAX_Q;
                     *reinterpret_cast<float4*>(mine) = make_float4(yh[0], yh[1], yh[2], yh[3]);
                     *reinterpret_cast<float4*>(mine + 4) = make_float4(yh[4], yh[5], yh[6], yh[7]);
                     worker_barrier(PF_NW);
-                    if (cg == 0) {
-                        float yq[STDADK_MAX_Q];
-                        float loss = 0.0f;
-                        if (rvalid) {
+                    if (cg == 0 && rvalid) {
 #pragma unroll
-                            for (int k = 0; k < STDADK_MAX_Q; ++k) {
-                                yq[k] = 0.0f;
-                                if (k < P.q) {
-                                    float acc_k = shb[k];
+                        for (int k = 0; k < STDADK_MAX_Q; ++k) {
+                            if (k < P.q) {
+                                float acc_k = shb[k];
 #pragma unroll
-                                    for (int g = 0; g < PF_CG; ++g)
-                                        acc_k += hscr[((size_t)g * TILE_M + row) * STDADK_MAX_Q + k];
-                                    yq[k] = acc_k;
-                                    P.yhat[lrow * P.q + k] = acc_k;
-                                }
+                                for (int g = 0; g < PF_CG; ++g)
+                                    acc_k += hscr[((size_t)g * TILE_M + row) * STDADK_MAX_Q + k];
+                                P.yhat[lrow * P.q + k] = acc_k;
                             }
-                            if (TRAIN && P.head.loss_type != STDADK_LOSS_NONE) {
-                                float dy[STDADK_MAX_Q];
-                                loss = row_loss(P.head, yq, P.head.y[sample_of(P.pts, P.pts.row_begin + lrow)], dy);
-                                if (P.head.dyhat) {
-#pragma unroll
-                                    for (int k = 0; k < STDADK_MAX_Q; ++k)
-                                        if (k < P.q) P.head.dyhat[lrow * P.q + k] = dy[k];
-                                }
-                            }
-                        }
-                        if (TRAIN && P.head.loss_type != STDADK_LOSS_NONE) {
-                            loss = warp_sum(loss);
-                            if (lane == 0) atomicAdd(P.head.loss_acc, loss);
                         }
                     }
                     PF_PHASE(ph_head);
@@ -519,7 +455,6 @@ __global__ void __launch_bounds__(PF_NT, 1) predict_fused_kernel(const __grid_co
             have_cur = have_next;
             lrow = nxt_lrow;
             rvalid = nxt_valid;
-            cur_tile = next;
         }
         PF_DBG(if (P.dbg && tid == 0) {
             atomicAdd(&P.dbg[3], w_acc);

@@ -73,25 +73,6 @@ __device__ __forceinline__ void bulk_g2s(void* smem_dst, const void* gsrc, uint3
                  : "memory");
 }
 
-// Multicast variant: the bytes land at the same shared-memory offset in every CTA of `cta_mask`, and each of those
-// CTAs' mbarrier (same offset) receives the complete_tx.
-__device__ __forceinline__ void bulk_g2s_mcast(void* smem_dst, const void* gsrc, uint32_t bytes, uint64_t* bar,
-                                               uint16_t cta_mask) {
-    asm volatile(
-        "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1], %2, [%3], %4;"
-        ::"r"(smem_u32(smem_dst)), "l"(gsrc), "r"(bytes), "r"(smem_u32(bar)), "h"(cta_mask)
-        : "memory");
-}
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-    uint32_t r;
-    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-    return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-    asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-    asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-
 // ---------------------------------------------------------------- TMEM
 __device__ __forceinline__ void tmem_alloc(uint32_t* smem_dst, uint32_t ncols) {
     asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(smem_dst)),
@@ -199,15 +180,6 @@ __device__ __forceinline__ void umma_tf32_ts(uint32_t taddr, uint32_t a_taddr, u
 __device__ __forceinline__ void umma_commit(uint64_t* bar) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
                  : "memory");
-}
-
-// commit that arrives on the same-offset mbarrier of every CTA in `cta_mask` (stage release in a multicast pipeline)
-__device__ __forceinline__ void umma_commit_mcast(uint64_t* bar, uint16_t cta_mask) {
-    asm volatile(
-        "tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
-            smem_u32(bar)),
-        "h"(cta_mask)
-        : "memory");
 }
 
 // ---------------------------------------------------------------- operand image addressing

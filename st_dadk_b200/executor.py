@@ -130,11 +130,6 @@ class Executor:
         self._knots_ready = False
         self._side = None
         self.fused_predict = True      # forward-only calls use the whole-network kernel when the shape fits
-        # The forward of a training step can run through the same kernel (stdadk_train_fwd: one launch, activations
-        # stay on the SM between blocks).  Measured 3-5 % SLOWER than three layer_fwd launches at batch 4096 / 16384 /
-        # 65536 (0.202 vs 0.191 ms, 0.268 vs 0.263, 0.825 vs 0.790): training has to write every activation and x
-        # image anyway, and one CTA per SM leaves less parallelism than the per-block kernels.  Off by default.
-        self.fused_train = False
         self._fused_ok = None
         self._field_ok = None
         self._cell_ws = None
@@ -318,11 +313,6 @@ class Executor:
         basis = self._basis()
         drop = L.Dropout(s.dropout if train else 0.0, step & 0xFFFFFFFF, seed,
                          step_ptr.data_ptr() if step_ptr is not None else None, key_offset)
-        head = None
-        if self.fused_train and not self.sparse and not self.x3 and self._train_fwd_fused(pts, ws, yhat, drop, y, loss, inv_count, save):
-            if save:
-                self._ctx = (pts, drop, ws)
-            return yhat
         if self.sparse:
             ops.sparse_l1_fwd(self._sparse_args(pts, ws, w1t=self._w1t, zs=ws.zs))
         for l in range(s.n_hidden):
@@ -349,12 +339,7 @@ class Executor:
                 if self.x3:
                     a.out_img_lo = ws.h_lo[l].data_ptr()
             else:
-                if loss is not None:
-                    code = L.LOSS_MSE if loss.kind == "mse" else L.LOSS_PINBALL
-                    head = ops.make_head(s.head_w, s.head_b, s.q, yhat, code, y, list(loss.taus), inv_count,
-                                         ws.dyhat, self.loss_acc, loss.nc_weight, loss.nc_power)
-                else:
-                    head = ops.make_head(s.head_w, s.head_b, s.q, yhat)
+                head = self._make_head(yhat, ws, y, loss, inv_count)
                 a.head = C.pointer(head)
             ops.layer_fwd(a)
         if save:
@@ -369,34 +354,17 @@ class Executor:
                                  self.loss_acc, loss.nc_weight, loss.nc_power)
         return ops.make_head(s.head_w, s.head_b, s.q, yhat)
 
-    def _train_fwd_fused(self, pts, ws, yhat, drop, y, loss, inv_count, save: bool) -> bool:
-        """Training-mode forward in ONE launch (stdadk_train_fwd): dropout, fused head + loss, and the activation /
-        x / statistics tensors the backward kernels read.  False when the shape does not fit the fused kernel."""
+    def _predict_args(self, pts: L.Points, yhat: torch.Tensor) -> L.PredictArgs:
+        """Arguments of the whole-network kernel (stdadk_predict) for this network; needs n_hidden <= MAX_HIDDEN."""
         s = self.spec
-        if s.n_hidden > L.MAX_HIDDEN:
-            return False
-        basis = self._basis()
-        head = self._make_head(yhat, ws, y, loss, inv_count)
-        a = L.TrainFwdArgs()
-        a.net.basis = C.pointer(basis)
-        a.net.pts = pts
-        a.net.n_layers = s.n_hidden
+        a = L.PredictArgs()
+        a.basis = C.pointer(self._basis())
+        a.pts = pts
+        a.n_layers = s.n_hidden
         for l in range(s.n_hidden):
-            a.net.layers[l] = self._layer(l)
-            if l < s.n_hidden - 1:
-                a.h_img[l] = ws.h[l].data_ptr()
-            if save and ws.stats[l] is not None:
-                a.stats[l] = ws.stats[l].data_ptr()
-            if save and ws.x is not None:
-                a.x_img[l] = ws.x[l].data_ptr()
-        a.net.head = C.pointer(head)
-        a.drop = drop
-        if self._fused_ok is None:
-            self._fused_ok = ops.predict_supported(a.net)
-        if not self._fused_ok:
-            return False
-        ops.train_fwd(a)
-        return True
+            a.layers[l] = self._layer(l)
+        a.head = C.pointer(ops.make_head(s.head_w, s.head_b, s.q, yhat))
+        return a
 
     def fused_supported(self) -> bool:
         """Whether forward-only calls on this network run through the whole-network kernel (decided once per binding;
@@ -406,33 +374,16 @@ class Executor:
             return False
         if self._fused_ok is None:
             probe = torch.empty(1, s.q, dtype=torch.float32, device=self.device)
-            basis = self._basis()
-            head = ops.make_head(s.head_w, s.head_b, s.q, probe)
-            a = L.PredictArgs()
-            a.basis = C.pointer(basis)
-            a.pts = ops.make_points(grid=(1, 1, 1), row_begin=0, n_rows=1)
-            a.n_layers = s.n_hidden
-            for l in range(s.n_hidden):
-                a.layers[l] = self._layer(l)
-            a.head = C.pointer(head)
-            self._fused_ok = ops.predict_supported(a)
+            self._fused_ok = ops.predict_supported(
+                self._predict_args(ops.make_points(grid=(1, 1, 1), row_begin=0, n_rows=1), probe))
         return bool(self._fused_ok)
 
     def _predict_fused(self, pts: L.Points, yhat: torch.Tensor) -> bool:
         """Forward-only path: the whole network in one persistent kernel (stdadk_predict), no activation images.
         Returns False when the shape does not fit the fused kernel; the caller then chains layer_fwd."""
-        s = self.spec
-        if s.n_hidden > L.MAX_HIDDEN:
+        if self.spec.n_hidden > L.MAX_HIDDEN:
             return False
-        basis = self._basis()
-        head = ops.make_head(s.head_w, s.head_b, s.q, yhat)
-        a = L.PredictArgs()
-        a.basis = C.pointer(basis)
-        a.pts = pts
-        a.n_layers = s.n_hidden
-        for l in range(s.n_hidden):
-            a.layers[l] = self._layer(l)
-        a.head = C.pointer(head)
+        a = self._predict_args(pts, yhat)
         if self._fused_ok is None:
             self._fused_ok = ops.predict_supported(a)
         if not self._fused_ok:

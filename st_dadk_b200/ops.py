@@ -184,11 +184,6 @@ def predict_field(args: L.FieldArgs):
     L.check(L.lib().stdadk_predict_field(C.byref(args), _stream()), "predict_field")
 
 
-def train_fwd(args: L.TrainFwdArgs):
-    """Forward of a training step (dropout, loss, saved tensors for the backward) in one launch."""
-    L.check(L.lib().stdadk_train_fwd(C.byref(args), _stream()), "train_fwd")
-
-
 def layer_bwd(args: L.BwdArgs):
     L.check(L.lib().stdadk_layer_bwd(C.byref(args), _stream()), "layer_bwd")
 

@@ -246,7 +246,6 @@ class Predictor:
         rec = []
         orig = _ops.layer_fwd
         fused, self.ex.fused_predict = self.ex.fused_predict, False     # profile the layer-by-layer kernels
-        fused_t, self.ex.fused_train = self.ex.fused_train, False
 
         def timed(a):
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -265,7 +264,6 @@ class Predictor:
         finally:
             _ops.layer_fwd = orig
             self.ex.fused_predict = fused
-            self.ex.fused_train = fused_t
         res = {}
         nl = self.ex.spec.n_hidden
         for lid, n_in, n_out, has_head, e0, e1 in rec[nl:]:          # first pass = warm-up

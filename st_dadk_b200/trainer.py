@@ -581,8 +581,7 @@ class Trainer:
         """libstdadk kernel launches in one optimisation step (counted from the launch sequence)."""
         nh = self.ex.spec.n_hidden
         n = 1                               # all weight images (W, W^T, W1s) in one pack_images launch
-        fused = self.ex.fused_train and not self.ex.sparse and self.ex._fused_ok is not False
-        n += (1 if fused else nh) + nh + nh   # forward (one whole-network launch, or one per block), layer_bwd, wgrad
+        n += nh + nh + nh                   # layer_fwd, layer_bwd, wgrad per block
         if self.learnable:
             n += 3                          # knot + temporal tables (knots move), knot_grad
         n += 1 if not self._norm_fused() else 2    # fused tail {norm, step counter, clip + AdamW + EMA}; or step counter + update
@@ -610,10 +609,7 @@ class Trainer:
         f_fwd = lambda a: 2.0 * rows * a.layer.n_in * a.layer.n_out
         f_bwd = lambda a: 2.0 * rows * a.layer.n_out * (a.layer.n_in + (a.n_next if not a.head else 0))
         f_wg = lambda a: 2.0 * rows * a.n_in * a.n_out
-        f_net = lambda a: 2.0 * rows * (sum(a.net.layers[l].n_in * a.net.layers[l].n_out for l in range(a.net.n_layers))
-                                        + a.net.layers[a.net.n_layers - 1].n_out * a.net.head.contents.q)
         patches = {
-            "train_fwd": ("train_fwd", f_net),
             "layer_fwd": (lambda a: f"layer_fwd[{a.layer.layer_id}]", f_fwd),
             "layer_bwd": (lambda a: f"layer_bwd[{a.layer.layer_id}]", f_bwd),
             "wgrad": (lambda a: f"wgrad[{a.n_in}x{a.n_out}]", f_wg),

@@ -294,13 +294,13 @@ def _default_oracle_model(seed, q=1, fn="wendland", hidden=(256, 256, 128)):
                            basis_fn=fn)
 
 
-@pytest.mark.parametrize("q,loss,taus,p,fused_train", [(1, "mse", None, 0.0, False),
-                                                       (5, "pinball", [0.05, 0.25, 0.5, 0.75, 0.95], 0.1, False),
-                                                       (5, "pinball", [0.05, 0.25, 0.5, 0.75, 0.95], 0.1, True),
-                                                       (1, "mse", None, 0.0, True),
-                                                       (1, "mse", None, 0.1, "x3"),
-                                                       (5, "pinball", [0.05, 0.25, 0.5, 0.75, 0.95], 0.1, "x3")])
-def test_default_size_network_with_dropout_vs_oracle(q, loss, taus, p, fused_train):
+@pytest.mark.parametrize("q,loss,taus,p,precision", [(1, "mse", None, 0.0, "tf32"),
+                                                     (1, "mse", None, 0.1, "tf32"),
+                                                     (5, "pinball", [0.05, 0.25, 0.5, 0.75, 0.95], 0.1, "tf32"),
+                                                     (1, "mse", None, 0.0, "tf32x3"),
+                                                     (1, "mse", None, 0.1, "tf32x3"),
+                                                     (5, "pinball", [0.05, 0.25, 0.5, 0.75, 0.95], 0.1, "tf32x3")])
+def test_default_size_network_with_dropout_vs_oracle(q, loss, taus, p, precision):
     """Default architecture 297-256-256-128-Q, ragged batch, dropout masks drawn in-kernel (Philox keyed on the
     global row) and replayed by the oracle: outputs, loss and all gradients."""
     L, ops, Executor, NetSpec, LossSpec = _mods()
@@ -320,16 +320,13 @@ def test_default_size_network_with_dropout_vs_oracle(q, loss, taus, p, fused_tra
     # isolates implementation errors from precision (tolerance 3e-3 instead of 2e-2)
     yemu, cache_e = orc.forward(m, None, coords, t, train=True, keep_masks=masks, return_cache=True, rnd=orc.tf32_round)
     gemu = orc.backward(m, cache_e, orc.loss_and_grad(yemu, y, loss, taus)[1])
-    x3 = fused_train == "x3"          # precision "tf32x3": compared with the FP64 oracle directly (no TF32 emulation)
-    fused_train = bool(fused_train) and not x3
-    spec = spec_from_oracle(m, dropout=p, precision="tf32x3" if x3 else "tf32")
+    x3 = precision == "tf32x3"        # compared with the FP64 oracle directly (no TF32 emulation)
+    spec = spec_from_oracle(m, dropout=p, precision=precision)
     ex = Executor(spec)
-    ex.fused_train = fused_train      # stdadk_train_fwd (whole forward in one launch) vs one layer_fwd per block
     ex.loss_acc.zero_()
     pts = ops.make_points(T(coords), T(t))
     yhat = ex.forward(pts, train=True, step=step, seed=seed, y=T(y), loss=LossSpec(loss, taus or ()),
                       inv_count=1.0 / (n * q), save=True)
-    assert not fused_train or ex._fused_ok is True
     grads = ex.backward()
     torch.cuda.synchronize()
     print("x3" if x3 else "tf32", "yhat err", rel_err(yhat.cpu().numpy(), yref), "dW0 err vs fp64",
@@ -472,29 +469,6 @@ def test_large_knot_regime_support_walk_vs_oracle(fn, sides):
     assert np.all(gw[:, ~mask] == 0) and np.all(np.abs(gw[:, mask]).sum(axis=0) > 0)
 
 
-def test_cluster_multicast_prediction_matches_plain_path():
-    """Optional throughput variant (STDADK_CLUSTER=1): clusters of 4 CTAs multicast every weight slab.  Its output
-    must be bit-identical to the plain launch (same arithmetic, only the slab delivery differs), for a tile count
-    that is not a multiple of the cluster size, and match the oracle."""
-    import os
-    L, ops, Executor, NetSpec, LossSpec = _mods()
-    m = _default_oracle_model(3, q=5)
-    ex = Executor(spec_from_oracle(m))
-    nx, ny, nt = 211, 181, 1            # 38191 points = 299 tiles (not a multiple of 4), last tile ragged
-    n = nx * ny * nt
-    ex.fused_predict = False            # the layer-by-layer kernels are the ones with a cluster variant
-    plain = ex.forward(ops.make_points(grid=(nx, ny, nt)), train=False).clone()
-    os.environ["STDADK_CLUSTER"] = "1"
-    try:
-        got = ex.forward(ops.make_points(grid=(nx, ny, nt)), train=False).clone()
-    finally:
-        del os.environ["STDADK_CLUSTER"]
-    assert torch.equal(got, plain)
-    idx = np.r_[0:300, n - 300:n]
-    coords, t = orc.grid_points(nx, ny, nt, 0, n)
-    assert rel_l2(got.cpu().numpy()[idx], orc.forward(m, None, coords[idx], t[idx])) < 1e-3
-
-
 @pytest.mark.parametrize("hidden,q,fn,ln,n", [((256, 256, 128), 5, "wendland", True, 38191),
                                               ((256, 256, 128), 1, "wendland", True, 1000),
                                               ((128, 128), 3, "triangular", True, 20000),
@@ -529,6 +503,7 @@ def test_fused_prediction_kernel_vs_layered_path_and_oracle(hidden, q, fn, ln, n
     idx = np.r_[0:min(n, 400), max(0, n - 400):n]
     ref = orc.forward(m, None, coords[idx], t[idx])
     assert rel_l2(f[idx], ref) < 1e-3 and rel_err(f[idx], ref) < 3e-3
+    assert rel_l2(l[idx], ref) < 1e-3
     emu = orc.forward(m, None, coords[idx], t[idx], rnd=orc.tf32_round)
     assert rel_l2(f[idx], emu) < 1e-4, rel_l2(f[idx], emu)
 
