@@ -58,6 +58,9 @@ static int pow2_cols(int n) {
     while (c < n) c <<= 1;
     return c;
 }
+// A 64-row tile's warps read the accumulator 64 columns at a time (two 32-column chunks, one per half-warp), so the
+// allocation covers n_pad rounded up to 64.
+static int tmem_cols_m64(int n_pad) { return pow2_cols((n_pad + 63) & ~63); }
 template <typename K>
 static int set_smem(K kernel, uint32_t bytes) {
     cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
@@ -301,7 +304,6 @@ int stdadk_layer_fwd(const stdadk_fwd_args* a, void* stream) {
     K.has_head = a->head ? 1 : 0;
     K.k_slabs = pad32(a->layer.n_in) / SLAB_K;
     K.n_pad = pad32(a->layer.n_out);
-    K.tmem_cols = pow2_cols(K.n_pad);
     K.thresh16 = dropout_thresh16(a->drop.p);
     K.drop_scale = a->drop.p > 0.0f ? 1.0f / (1.0f - a->drop.p) : 1.0f;
     const bool basis = a->basis != nullptr;
@@ -310,23 +312,31 @@ int stdadk_layer_fwd(const stdadk_fwd_args* a, void* stream) {
     // (dense prediction): 8 worker warps and two CTAs per SM so one tile's epilogue overlaps the other's MMAs
     const int sms = g_sm_count > 0 ? g_sm_count : 148;
     const int cg = tiles >= 2 * sms ? 2 : 4;
+    // a batch that fits in one wave of 64-row tiles runs on twice the SMs, each walking half the rows.  Both halves of
+    // every 128-row image tile get a CTA, so the padding rows of the last tile are written (zeros) as on the 128-row
+    // path: wgrad and the knot gradient read whole 128-row tiles.
+    const bool half_tiles = 2 * tiles <= sms;
+    if (half_tiles) tiles *= 2;
+    K.tmem_cols = half_tiles ? tmem_cols_m64(K.n_pad) : pow2_cols(K.n_pad);
     const int ns = cg == 2 ? 2 : 4;   // 1 CTA/SM in the latency configuration: spend the shared memory on pipeline depth
     SmemPlan sp = plan_smem(K.n_pad, K.has_head ? K.head.q : 0, basis ? K.basis.k_s : 0, basis ? K.basis.k_t : 0, false, cg, ns,
                             basis ? K.k_slabs * 8 : 0);
     REQUIRE(sp.total <= 227 * 1024, "layer_fwd: needs %u B of shared memory (> 227 KB): too many knots for the dense path",
             sp.total);
     K.n_tiles = tiles;
-#define LAUNCH_FWD(B, C)                                                                                     \
-    do {                                                                                                     \
-        if (int r = set_smem(layer_fwd_kernel<B, C, (C == 2 ? 2 : 4)>, sp.total)) return r;                  \
-        layer_fwd_kernel<B, C, (C == 2 ? 2 : 4)><<<tiles, n_threads(C), sp.total, (cudaStream_t)stream>>>(K); \
+#define LAUNCH_FWD(B, TM, C)                                                                                     \
+    do {                                                                                                         \
+        if (int r = set_smem(layer_fwd_kernel<B, TM, C, (C == 2 ? 2 : 4)>, sp.total)) return r;                  \
+        layer_fwd_kernel<B, TM, C, (C == 2 ? 2 : 4)><<<tiles, n_threads(C), sp.total, (cudaStream_t)stream>>>(K); \
     } while (0)
     if (basis) {
-        if (cg == 2) LAUNCH_FWD(true, 2);
-        else LAUNCH_FWD(true, 4);
+        if (half_tiles) LAUNCH_FWD(true, 64, 4);
+        else if (cg == 2) LAUNCH_FWD(true, 128, 2);
+        else LAUNCH_FWD(true, 128, 4);
     } else {
-        if (cg == 2) LAUNCH_FWD(false, 2);
-        else LAUNCH_FWD(false, 4);
+        if (half_tiles) LAUNCH_FWD(false, 64, 4);
+        else if (cg == 2) LAUNCH_FWD(false, 128, 2);
+        else LAUNCH_FWD(false, 128, 4);
     }
 #undef LAUNCH_FWD
     return check_launch("layer_fwd");
@@ -540,7 +550,6 @@ int stdadk_layer_bwd(const stdadk_bwd_args* a, void* stream) {
     K.k_slabs = a->x_img ? 0 : pad32(a->layer.n_in) / SLAB_K;      // x saved by the forward: no recomputation GEMM
     K.k_slabs2 = a->head ? 0 : pad32(a->n_next) / SLAB_K;
     K.n_pad = pad32(a->layer.n_out);
-    K.tmem_cols = 2 * pow2_cols(K.n_pad);
     K.thresh16 = dropout_thresh16(a->drop.p);
     K.drop_scale = a->drop.p > 0.0f ? 1.0f / (1.0f - a->drop.p) : 1.0f;
     const bool basis = a->basis != nullptr && a->x_img == nullptr;
@@ -549,22 +558,32 @@ int stdadk_layer_bwd(const stdadk_bwd_args* a, void* stream) {
                             basis ? K.k_slabs * 8 : 0);
     REQUIRE(sp.total <= 227 * 1024, "layer_bwd: needs %u B of shared memory (> 227 KB)", sp.total);
     int tiles = (int)ceil_div64(a->pts.n_rows, TILE_M);
+    // one wave of 64-row tiles (as in layer_fwd), only with x saved by the forward: there is no recompute GEMM then
+    const int sms = g_sm_count > 0 ? g_sm_count : 148;
+    const bool half_tiles = a->x_img && 2 * tiles <= sms;
+    if (half_tiles) tiles *= 2;
+    K.tmem_cols = 2 * (half_tiles ? tmem_cols_m64(K.n_pad) : pow2_cols(K.n_pad));
     const bool ln = a->layer.gamma != nullptr, hd = a->head != nullptr;
-#define LAUNCH_BWD(B, LNV, HD)                                                                              \
-    do {                                                                                                    \
-        if (int r = set_smem(layer_bwd_kernel<B, BCG, BNS, LNV, HD>, sp.total)) return r;                   \
-        layer_bwd_kernel<B, BCG, BNS, LNV, HD><<<tiles, n_threads(BCG), sp.total, (cudaStream_t)stream>>>(K); \
+#define LAUNCH_BWD(B, TM, LNV, HD)                                                                              \
+    do {                                                                                                        \
+        if (int r = set_smem(layer_bwd_kernel<B, TM, BCG, BNS, LNV, HD>, sp.total)) return r;                   \
+        layer_bwd_kernel<B, TM, BCG, BNS, LNV, HD><<<tiles, n_threads(BCG), sp.total, (cudaStream_t)stream>>>(K); \
     } while (0)
-    if (basis) {
-        if (ln && hd) LAUNCH_BWD(true, true, true);
-        else if (ln) LAUNCH_BWD(true, true, false);
-        else if (hd) LAUNCH_BWD(true, false, true);
-        else LAUNCH_BWD(true, false, false);
+    if (half_tiles) {
+        if (ln && hd) LAUNCH_BWD(false, 64, true, true);
+        else if (ln) LAUNCH_BWD(false, 64, true, false);
+        else if (hd) LAUNCH_BWD(false, 64, false, true);
+        else LAUNCH_BWD(false, 64, false, false);
+    } else if (basis) {
+        if (ln && hd) LAUNCH_BWD(true, 128, true, true);
+        else if (ln) LAUNCH_BWD(true, 128, true, false);
+        else if (hd) LAUNCH_BWD(true, 128, false, true);
+        else LAUNCH_BWD(true, 128, false, false);
     } else {
-        if (ln && hd) LAUNCH_BWD(false, true, true);
-        else if (ln) LAUNCH_BWD(false, true, false);
-        else if (hd) LAUNCH_BWD(false, false, true);
-        else LAUNCH_BWD(false, false, false);
+        if (ln && hd) LAUNCH_BWD(false, 128, true, true);
+        else if (ln) LAUNCH_BWD(false, 128, true, false);
+        else if (hd) LAUNCH_BWD(false, 128, false, true);
+        else LAUNCH_BWD(false, 128, false, false);
     }
 #undef LAUNCH_BWD
     return check_launch("layer_bwd");

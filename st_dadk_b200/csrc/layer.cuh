@@ -10,10 +10,14 @@
 //                      LayerNorm backward and writes the dz image + bias/LN/head gradients.
 //   wgrad_kernel     : dW += dz^T A, reduction over rows, both operands MN-major from the same images.
 //
-// One CTA = one 128-row tile (128 TMEM lanes).  Worker warps 0 .. 4*CG-1 (operand generation and epilogue):
-// warp w owns TMEM lane quarter q = w & 3 (the hardware ties a warp to lanes 32*(w%4)..) and column group
-// cg = w >> 2, i.e. thread = (row, 1/CG of the columns); then one producer warp (bulk copies) and one MMA
-// issuer warp (one elected thread).  CG = 4 for latency (few tiles), CG = 2 with two CTAs per SM for throughput.
+// One CTA = one tile of TM rows: TM = 128 (128 TMEM lanes) or, for the forward and the x_img backward, TM = 64 (an
+// M = 64 MMA, whose accumulator fills lanes 0-15 of each 32-lane quarter).  The operand images stay in 128-row slab
+// tiles either way: a 64-row CTA i owns rows (i & 1) * 64 .. +63 of image tile i >> 1.  Worker warps 0 .. 4*CG-1
+// (operand generation and epilogue): warp w owns TMEM lane quarter q = w & 3 (the hardware ties a warp to lanes
+// 32*(w%4)..) and column group cg = w >> 2, i.e. thread = (row, 1/CG of the columns); at TM = 64 the two half-warps
+// take alternate 32-column chunks, so thread = (row, 1/(2 CG) of the columns).  Then one producer warp (bulk copies)
+// and one MMA issuer warp (one elected thread).  CG = 4 for latency (few tiles), CG = 2 with two CTAs per SM for
+// throughput.  TM = 64 is for batches that fit in one wave of 64-row tiles: twice the SMs, half the rows per CTA.
 #pragma once
 #include "common.cuh"
 
@@ -24,6 +28,55 @@ constexpr int RED_STRIDE = 4 + STDADK_MAX_Q;   // per (cg, row) scratch: four La
 __host__ __device__ constexpr int n_work(int cg) { return 128 * cg; }
 __host__ __device__ constexpr int n_threads(int cg) { return 128 * cg + 64; }
 __device__ __forceinline__ void worker_barrier(int nw) { asm volatile("bar.sync 1, %0;" ::"r"(nw) : "memory"); }
+
+// Worker-thread geometry of a TM-row tile (see the header).  The column loops of the epilogues run over the WARP's
+// chunks (wc, and at TM = 64 also wc + 32), so every tcgen05.ld and shuffle is executed by the whole warp; a thread's
+// own chunk is c0 = wc + chunk_off, which at TM = 64 can lie at n_pad when n_pad is an odd multiple of 32.
+template <int TM>
+struct TileGeo {
+    static_assert(TM == 128 || TM == 64, "tile height");
+    static constexpr int ROWS_PER_WARP = TM / 4;                 // rows of a lane quarter
+    static constexpr int WARP_COLS = TM == 128 ? 32 : 64;        // columns one warp covers per step of its loop
+    __device__ static int row(int q4, int lane) { return q4 * ROWS_PER_WARP + (TM == 128 ? lane : (lane & 15)); }
+    __device__ static int chunk_off(int lane) { return TM == 128 ? 0 : (lane >> 4) * 32; }
+    // column group of the thread, 0 .. groups-1, in the order LayerNorm partials are combined
+    __device__ static int group(int cg, int lane) { return TM == 128 ? cg : 2 * cg + (lane >> 4); }
+    __host__ __device__ static constexpr int groups(int cg) { return TM == 128 ? cg : 2 * cg; }
+};
+// accumulator columns [wc, wc + 32) (TM = 128), or [wc, wc + 32) for half-warp 0 and [wc + 32, wc + 64) for half-warp 1
+template <int TM>
+__device__ __forceinline__ void acc_ld(uint32_t taddr, float (&v)[32]) {
+    if (TM == 128) tmem_ld32(taddr, v);
+    else tmem_ld16x2<32>(taddr, v);
+}
+// warp_transpose_sum within each half-warp: on return lane l holds the column sums of indices 2 (l & 15) and +1
+__device__ __forceinline__ float2 halfwarp_transpose_sum(float (&v)[32], int lane) {
+#pragma unroll
+    for (int off = 8, n = 16; off >= 1; off >>= 1, n >>= 1) {
+        bool upper = (lane & off) != 0;
+#pragma unroll
+        for (int i = 0; i < n; ++i) {
+            float send = upper ? v[i] : v[i + n];
+            float keep = upper ? v[i + n] : v[i];
+            v[i] = keep + __shfl_xor_sync(0xffffffffu, send, off);
+        }
+    }
+    return make_float2(v[0], v[1]);
+}
+// Column sums of a 32-column chunk over the rows of the warp, added into cs[c0 ..]; skipped for chunks at n_pad.
+template <int TM>
+__device__ __forceinline__ void colsum_chunk(float* cs, int c0, bool cvalid, float (&v)[32], int lane) {
+    if (TM == 128) {
+        const float s = warp_transpose_sum(v, lane);
+        atomicAdd(&cs[c0 + lane], s);
+    } else {
+        const float2 s = halfwarp_transpose_sum(v, lane);
+        if (cvalid) {
+            atomicAdd(&cs[c0 + 2 * (lane & 15)], s.x);
+            atomicAdd(&cs[c0 + 2 * (lane & 15) + 1], s.y);
+        }
+    }
+}
 
 // ---------------------------------------------------------------- shared-memory carve-up
 struct SmemPlan {
@@ -348,17 +401,20 @@ __device__ __forceinline__ void gen_basis_slab(const BasisP& B, const float4* sk
     }
 }
 
-// Producer: B slab (n_pad rows of the weight image, split over its 128-row tiles) [+ A slab].
+// Producer: B slab (n_pad rows of the weight image, split over its 128-row tiles) [+ A slab: a_bytes from a_tile_img,
+// the whole 128-row slab or, for a 64-row tile, its half: 64 rows are 8 whole swizzle periods, so either half of an
+// image slab is already in the MMA's layout].
 __device__ __forceinline__ void issue_slab_copies(const float* w_img, int w_slabs, int slab, int n_pad,
-                                                  const float* a_tile_img, float* sA, float* sB, uint64_t* bar) {
-    uint32_t bytes = (uint32_t)n_pad * 128u + (a_tile_img ? (uint32_t)SLAB_BYTES : 0u);
+                                                  const float* a_tile_img, float* sA, float* sB, uint64_t* bar,
+                                                  uint32_t a_bytes = SLAB_BYTES) {
+    uint32_t bytes = (uint32_t)n_pad * 128u + (a_tile_img ? a_bytes : 0u);
     mbar_arrive_expect_tx(bar, bytes);
     for (int r0 = 0; r0 < n_pad; r0 += TILE_M) {
         int rows = min(TILE_M, n_pad - r0);
         const float* src = w_img + ((size_t)(r0 / TILE_M) * w_slabs + slab) * SLAB_FLOATS;
         bulk_g2s(sB + (size_t)r0 * SLAB_K, src, (uint32_t)rows * 128u, bar);
     }
-    if (a_tile_img) bulk_g2s(sA, a_tile_img + (size_t)slab * SLAB_FLOATS, SLAB_BYTES, bar);
+    if (a_tile_img) bulk_g2s(sA, a_tile_img + (size_t)slab * SLAB_FLOATS, a_bytes, bar);
 }
 
 // Knot tables (knots4: cx, cy, theta'^2, 1/theta'; tknots2: c, 1/bw) -> shared memory with bulk async copies (TMA 1-D)
@@ -596,15 +652,16 @@ struct EpiCtx {
     const float* sbet;
     const float* shw;
     const float* shb;
-    float* red;                    // CG x 128 x RED_STRIDE floats of scratch
+    float* red;                    // (groups x TM) x RED_STRIDE floats of scratch
     uint32_t trow;                 // accumulator address of this warp's lane quarter
-    int tile, row, cg, lane;
+    int tile, row, irow, cg, lane; // tile / irow: image tile and row in it; row: row of the CTA's tile
     long long lrow, grow;
     bool rvalid, tile_valid;
 };
-template <int CG>
+template <int CG, int TM>
 __device__ __forceinline__ void fwd_epilogue(const FwdK& P, const EpiCtx& E) {
-    constexpr int NW = n_work(CG);
+    using G = TileGeo<TM>;
+    constexpr int NW = n_work(CG), NG = G::groups(CG), WSTEP = G::WARP_COLS * CG;
     const float* sbias = E.sbias;
     const float* sgam = E.sgam;
     const float* sbet = E.sbet;
@@ -612,45 +669,48 @@ __device__ __forceinline__ void fwd_epilogue(const FwdK& P, const EpiCtx& E) {
     const float* shb = E.shb;
     float* red = E.red;
     const uint32_t trow = E.trow;
-    const int tile = E.tile, row = E.row, cg = E.cg, lane = E.lane;
+    const int tile = E.tile, row = E.row, irow = E.irow, cg = E.cg, lane = E.lane;
     const long long lrow = E.lrow, grow = E.grow;
     const bool rvalid = E.rvalid, tile_valid = E.tile_valid;
     const int n_pad = P.n_pad, n_out = P.L.n_out;
     const bool has_ln = P.L.gamma != nullptr;
-    float* myred = red + ((size_t)cg * TILE_M + row) * RED_STRIDE;
+    const int coff = G::chunk_off(lane), grp = G::group(cg, lane);
+    float* myred = red + ((size_t)grp * TM + row) * RED_STRIDE;
     const float* arow = (P.addend && rvalid) ? P.addend + (size_t)lrow * n_out : nullptr;
     float v[32];
     float mean = 0.0f, rstd = 1.0f;
     if (has_ln) {
         // pass 1: shifted moments of x = A W^T + b (+ addend): per-thread shift K (the thread's first value) removes
-        // the cancellation of the raw-moment formula; the CG column groups of a row publish (K, S1, S2, count) and
+        // the cancellation of the raw-moment formula; the NG column groups of a row publish (K, S1, S2, count) and
         // every thread combines them exactly:
         //   mean = sum_g (n_g K_g + S1_g) / n,   M2 = sum_g [S2_g - 2 (mean - K_g) S1_g + n_g (mean - K_g)^2]
         float K = 0.0f, S1 = 0.0f, S2 = 0.0f, cntv = 0.0f;
         bool have = false;
-        for (int c0 = 32 * cg; c0 < n_pad; c0 += 32 * CG) {
-            const int nv = n_out - c0;
-            if (nv <= 0) break;
-            tmem_ld32(trow + c0, v);
-            if (arow) add_addend_chunk(v, arow, c0, n_out);
-            pf_bias_stats(v, sbias + c0, min(nv, 32), have, K, S1, S2);
-            cntv += (float)min(nv, 32);
+        for (int wc = G::WARP_COLS * cg; wc < n_pad; wc += WSTEP) {
+            const int c0 = wc + coff, nv = n_out - c0;
+            if ((TM == 128 ? nv : n_out - wc) <= 0) break;      // warp-uniform: the half-warps' c0 differ at TM = 64
+            acc_ld<TM>(trow + wc, v);
+            if (TM == 128 || nv > 0) {
+                if (arow) add_addend_chunk(v, arow, c0, n_out);
+                pf_bias_stats(v, sbias + c0, min(nv, 32), have, K, S1, S2);
+                cntv += (float)min(nv, 32);
+            }
         }
         const float inv_n = 1.0f / (float)n_out;
-        if (CG > 1) {
+        if (NG > 1) {
             *reinterpret_cast<float4*>(myred) = make_float4(K, S1, S2, cntv);
             worker_barrier(NW);
-            float4 part[CG];
+            float4 part[NG];
             float tot = 0.0f;
 #pragma unroll
-            for (int g = 0; g < CG; ++g) {
-                part[g] = *reinterpret_cast<const float4*>(red + ((size_t)g * TILE_M + row) * RED_STRIDE);
+            for (int g = 0; g < NG; ++g) {
+                part[g] = *reinterpret_cast<const float4*>(red + ((size_t)g * TM + row) * RED_STRIDE);
                 tot += fmaf(part[g].w, part[g].x, part[g].y);
             }
             mean = tot * inv_n;
             float m2 = 0.0f;
 #pragma unroll
-            for (int g = 0; g < CG; ++g) {
+            for (int g = 0; g < NG; ++g) {
                 float dk = mean - part[g].x;
                 m2 += part[g].z - 2.0f * dk * part[g].y + part[g].w * dk * dk;
             }
@@ -660,7 +720,7 @@ __device__ __forceinline__ void fwd_epilogue(const FwdK& P, const EpiCtx& E) {
             mean = K + m1;
             rstd = 1.0f / sqrtf(fmaxf(S2 * inv_n - m1 * m1, 0.0f) + P.L.eps);
         }
-        if (P.stats && rvalid && cg == 0) {
+        if (P.stats && rvalid && grp == 0) {
             P.stats[2 * lrow] = mean;
             P.stats[2 * lrow + 1] = rstd;
         }
@@ -672,12 +732,14 @@ __device__ __forceinline__ void fwd_epilogue(const FwdK& P, const EpiCtx& E) {
     const bool drop = P.L.drop_p > 0.0f;
     const unsigned int drop_step = drop ? dropout_step(P.L) : 0u;
     // pass 2: x -> LayerNorm -> ReLU -> dropout -> operand image (+ head partials, + x image for the backward)
-    for (int c0 = 32 * cg; c0 < n_pad; c0 += 32 * CG) {
+    for (int wc = G::WARP_COLS * cg; wc < n_pad; wc += WSTEP) {
+        const int c0 = wc + coff;
+        const bool cvalid = TM == 128 || c0 < n_pad;
         uint32_t keep = 0xFFFFFFFFu;
-        if (drop)       // masks first: the Philox calls neither sit behind the TMEM load nor hold 32 live values
+        if (drop && cvalid)   // masks first: the Philox calls neither sit behind the TMEM load nor hold 32 live values
             keep = pf_keep_mask(P.L.seed, drop_step, (uint32_t)P.L.layer_id, P.L.key_offset + (unsigned long long)lrow, c0,
                                 P.thresh16);
-        tmem_ld32(trow + c0, v);
+        acc_ld<TM>(trow + wc, v);
         if (arow) add_addend_chunk(v, arow, c0, n_out);
 #pragma unroll
         for (int c = 0; c < 8; ++c) {
@@ -686,33 +748,34 @@ __device__ __forceinline__ void fwd_epilogue(const FwdK& P, const EpiCtx& E) {
             const float2 hi = add2(make_float2(v[4 * c + 2], v[4 * c + 3]), make_float2(b.z, b.w));
             v[4 * c] = lo.x; v[4 * c + 1] = lo.y; v[4 * c + 2] = hi.x; v[4 * c + 3] = hi.y;
         }
-        if (P.x_img && tile_valid)            // training with a single wave of tiles: keep x for the backward
-            image_store_chunk(P.x_img, tile, n_pad / SLAB_K, c0, (uint32_t)row, v);
+        if (P.x_img && tile_valid && cvalid)  // training with a single wave of tiles: keep x for the backward
+            image_store_chunk(P.x_img, tile, n_pad / SLAB_K, c0, (uint32_t)irow, v);
         const int nv = rvalid ? min(32, max(n_out - c0, 0)) : 0;      // padding rows / columns -> 0
         pf_normalize(v, sgam + c0, sbet + c0, has_ln, rstd, nmr, nv);
         if (drop) pf_dropout(v, keep, P.drop_scale);
-        if (P.has_head) pf_head_partial(v, shw, n_pad, c0, P.head.q, yh);
-        if (P.out_img && tile_valid)
-            store_operand_chunk(P.out_img, P.out_img_lo, tile, n_pad / SLAB_K, c0, (uint32_t)row, v);
+        if (P.has_head && cvalid) pf_head_partial(v, shw, n_pad, c0, P.head.q, yh);
+        if (P.out_img && tile_valid && cvalid)
+            store_operand_chunk(P.out_img, P.out_img_lo, tile, n_pad / SLAB_K, c0, (uint32_t)irow, v);
     }
     if (P.has_head) {
-        if (CG > 1) {
+        // head partials after the LayerNorm partials of the same scratch row, which slower threads may still be reading
+        if (NG > 1) {
 #pragma unroll
             for (int k = 0; k < STDADK_MAX_Q; ++k)
-                if (k < P.head.q) myred[2 + k] = yh[k];
+                if (k < P.head.q) myred[4 + k] = yh[k];
             worker_barrier(NW);
         }
         if (cg == 0) {
             float loss = 0.0f;
-            if (rvalid) {
+            if (rvalid && grp == 0) {
                 float dy[STDADK_MAX_Q];
 #pragma unroll
                 for (int k = 0; k < STDADK_MAX_Q; ++k)
                     if (k < P.head.q) {
-                        if (CG > 1) {
+                        if (NG > 1) {
                             float acc = 0.0f;
 #pragma unroll
-                            for (int g = 0; g < CG; ++g) acc += red[((size_t)g * TILE_M + row) * RED_STRIDE + 2 + k];
+                            for (int g = 0; g < NG; ++g) acc += red[((size_t)g * TM + row) * RED_STRIDE + 4 + k];
                             yh[k] = acc;
                         }
                         yh[k] += shb[k];
@@ -735,9 +798,10 @@ __device__ __forceinline__ void fwd_epilogue(const FwdK& P, const EpiCtx& E) {
     }
 }
 
-template <bool BASIS, int CG, int NS>
+template <bool BASIS, int TM, int CG, int NS>
 __global__ void __launch_bounds__(n_threads(CG), CG <= 2 ? 2 : 1) layer_fwd_kernel(const __grid_constant__ FwdK P) {
-    constexpr int NW = n_work(CG), NT = n_threads(CG), NSTAGE = NS;
+    using G = TileGeo<TM>;
+    constexpr int NW = n_work(CG), NT = n_threads(CG), NSTAGE = NS, NG = G::groups(CG);
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = align_smem(smem_raw);
     const SmemPlan sp = plan_smem(P.n_pad, P.has_head ? P.head.q : 0, BASIS ? P.basis.k_s : 0,
@@ -769,6 +833,7 @@ __global__ void __launch_bounds__(n_threads(CG), CG <= 2 ? 2 : 1) layer_fwd_kern
     // 1M-row launch took 0.812 ms instead of 0.789 ms (B200, 1000 W power limit).
     const bool tile_valid = (int)blockIdx.x < P.n_tiles;
     const int tile = tile_valid ? (int)blockIdx.x : P.n_tiles - 1;
+    const int itile = tile / (TILE_M / TM), irow0 = (tile % (TILE_M / TM)) * TM;   // image tile, first row in it
     const int n_pad = P.n_pad, n_out = P.L.n_out;
     const bool has_ln = P.L.gamma != nullptr;
     const size_t b_stage_floats = (size_t)n_pad * SLAB_K;
@@ -808,7 +873,7 @@ __global__ void __launch_bounds__(n_threads(CG), CG <= 2 ? 2 : 1) layer_fwd_kern
     if (warp == 4 * CG) {
         // ---------------- producer
         if (lane == 0) {
-            const size_t a_off = (size_t)tile * P.k_slabs * SLAB_FLOATS;
+            const size_t a_off = (size_t)itile * P.k_slabs * SLAB_FLOATS + (size_t)irow0 * SLAB_K;
             const int n_virt = P.k_slabs * P.passes;
             for (int v = 0; v < n_virt; ++v) {
                 const int s = v / P.passes, p = v - s * P.passes;
@@ -817,14 +882,14 @@ __global__ void __launch_bounds__(n_threads(CG), CG <= 2 ? 2 : 1) layer_fwd_kern
                 const float* w_src = pass_b_lo(p) ? P.L.w_img_lo : P.L.w_img;
                 const float* a_tile = BASIS ? nullptr : (pass_a_lo(p) ? P.a_img_lo : P.a_img) + a_off;
                 issue_slab_copies(w_src, P.k_slabs, s, n_pad, a_tile, sA + (size_t)stage * SLAB_FLOATS,
-                                  sB + stage * b_stage_floats, &full[stage]);
+                                  sB + stage * b_stage_floats, &full[stage], TM * 128u);
             }
         }
         __syncwarp();
     } else if (warp == 4 * CG + 1) {
         // ---------------- MMA issuer
         if (lane == 0) {
-            const uint32_t idesc = umma_idesc_tf32((uint32_t)n_pad, 0, 0);
+            const uint32_t idesc = umma_idesc_tf32((uint32_t)n_pad, 0, 0, TM);
             const int n_virt = P.k_slabs * P.passes;
             for (int s = 0; s < n_virt; ++s) {
                 int stage = s % NSTAGE, it = s / NSTAGE;
@@ -840,8 +905,8 @@ __global__ void __launch_bounds__(n_threads(CG), CG <= 2 ? 2 : 1) layer_fwd_kern
     } else {
         // ---------------- workers: thread = (row, column group)
         const int q4 = warp & 3, cg = warp >> 2;
-        const int row = q4 * 32 + lane;
-        const long long lrow = (long long)tile * TILE_M + row;
+        const int row = G::row(q4, lane), grp = G::group(cg, lane);     // grp: the thread's 8 / NG chunks of each slab
+        const long long lrow = (long long)tile * TM + row;
         const bool rvalid = tile_valid && lrow < P.pts.n_rows;
         const long long grow = P.pts.row_begin + lrow;
         if (BASIS) {
@@ -856,7 +921,9 @@ __global__ void __launch_bounds__(n_threads(CG), CG <= 2 ? 2 : 1) layer_fwd_kern
                 constexpr int FN = decltype(fn_tag)::value;
                 int stage = 0, it = 0;
                 for (int s = 0; s < P.k_slabs; ++s) {
-                    float* gslab = (P.feat_img && tile_valid) ? P.feat_img + ((size_t)tile * P.k_slabs + s) * SLAB_FLOATS : nullptr;
+                    float* gslab = (P.feat_img && tile_valid)
+                                       ? P.feat_img + ((size_t)itile * P.k_slabs + s) * SLAB_FLOATS + (size_t)irow0 * SLAB_K
+                                       : nullptr;
                     for (int p = 0; p < P.passes; ++p) {
                         if (it > 0) {
                             if (tid == 0) FWD_WAIT(5, mbar_wait(&empty[stage], (it - 1) & 1));
@@ -864,11 +931,11 @@ __global__ void __launch_bounds__(n_threads(CG), CG <= 2 ? 2 : 1) layer_fwd_kern
                         }
                         const uint32_t sa = smem_u32(sA + (size_t)stage * SLAB_FLOATS);
                         if (pass_a_lo(p))
-                            gen_basis_slab_soa<FN, true, 2>(P.basis, ctab, s, x, y, t, xrow, sa, (uint32_t)row, cg * (8 / CG),
-                                                         (cg + 1) * (8 / CG), nullptr);
+                            gen_basis_slab_soa<FN, true, 2>(P.basis, ctab, s, x, y, t, xrow, sa, (uint32_t)row, grp * (8 / NG),
+                                                         (grp + 1) * (8 / NG), nullptr);
                         else
-                            gen_basis_slab_soa<FN, false, 2>(P.basis, ctab, s, x, y, t, xrow, sa, (uint32_t)row, cg * (8 / CG),
-                                                          (cg + 1) * (8 / CG), p == 0 ? gslab : nullptr);
+                            gen_basis_slab_soa<FN, false, 2>(P.basis, ctab, s, x, y, t, xrow, sa, (uint32_t)row, grp * (8 / NG),
+                                                          (grp + 1) * (8 / NG), p == 0 ? gslab : nullptr);
                         fence_proxy_async_smem();
                         mbar_arrive_warp(&full[stage]);
                         if (++stage == NSTAGE) { stage = 0; ++it; }
@@ -884,9 +951,9 @@ __global__ void __launch_bounds__(n_threads(CG), CG <= 2 ? 2 : 1) layer_fwd_kern
         mbar_wait(accf, 0);
         tc_fence_after();
         FWD_T(2);   // wait for the accumulator
-        EpiCtx E{sbias, sgam, sbet, shw, shb, red, tmem_base + ((uint32_t)(q4 * 32) << 16), tile, row, cg, lane, lrow, grow,
-                 rvalid, tile_valid};
-        fwd_epilogue<CG>(P, E);
+        EpiCtx E{sbias, sgam, sbet, shw, shb, red, tmem_base + ((uint32_t)(q4 * 32) << 16), itile, row, irow0 + row, cg, lane,
+                 lrow, grow, rvalid, tile_valid};
+        fwd_epilogue<CG, TM>(P, E);
         tc_fence_before();
         FWD_T(3);   // epilogue
     }
@@ -918,10 +985,12 @@ __device__ __forceinline__ void head_dh_chunk(float (&g)[32], const float (&dyh)
 // =============================================================================================
 // LN / HEAD are compile-time so that each instantiation carries only its own epilogue: the generic kernel was
 // 150 KB of SASS and a one-wave launch (32 tiles) spent ~30% of its stall samples on instruction fetch.
-template <bool BASIS, int CG, int NS, bool LN, bool HEAD>
+template <bool BASIS, int TM, int CG, int NS, bool LN, bool HEAD>
 __global__ void __launch_bounds__(n_threads(CG), 1) layer_bwd_kernel(const __grid_constant__ BwdK P) {
-    constexpr int NW = n_work(CG), NT = n_threads(CG), NSTAGE = NS;
-    constexpr int MAXCH = MAX_N / 32 / CG;          // column chunks per thread
+    using G = TileGeo<TM>;
+    constexpr int NW = n_work(CG), NT = n_threads(CG), NSTAGE = NS, NG = G::groups(CG);
+    constexpr int WSTEP = G::WARP_COLS * CG;
+    constexpr int MAXCH = MAX_N / WSTEP;            // column chunks per thread
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = align_smem(smem_raw);
     const int q = HEAD ? P.head.q : 0;
@@ -947,6 +1016,7 @@ __global__ void __launch_bounds__(n_threads(CG), 1) layer_bwd_kernel(const __gri
 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int tile = blockIdx.x;
+    const int itile = tile / (TILE_M / TM), irow0 = (tile % (TILE_M / TM)) * TM;   // image tile, first row in it
     const int n_pad = P.n_pad, n_out = P.L.n_out;
     constexpr bool has_ln = LN;
     const size_t b_stage_floats = (size_t)n_pad * SLAB_K;
@@ -987,7 +1057,8 @@ __global__ void __launch_bounds__(n_threads(CG), 1) layer_bwd_kernel(const __gri
 
     if (warp == 4 * CG) {
         if (lane == 0) {
-            const size_t a_off = (size_t)tile * P.k_slabs * SLAB_FLOATS, dzn_off = (size_t)tile * P.k_slabs2 * SLAB_FLOATS;
+            const size_t a_off = (size_t)itile * P.k_slabs * SLAB_FLOATS + (size_t)irow0 * SLAB_K;
+            const size_t dzn_off = (size_t)itile * P.k_slabs2 * SLAB_FLOATS + (size_t)irow0 * SLAB_K;
             for (int v = 0; v < total_slabs; ++v) {
                 int stage = v % NSTAGE, it = v / NSTAGE;
                 if (it > 0) mbar_wait(&empty[stage], (it - 1) & 1);
@@ -997,18 +1068,19 @@ __global__ void __launch_bounds__(n_threads(CG), 1) layer_bwd_kernel(const __gri
                     const int s = v / P.passes, p = v - s * P.passes;
                     const float* a_tile = BASIS ? nullptr : (pass_a_lo(p) ? P.a_img_lo : P.a_img) + a_off;
                     issue_slab_copies(pass_b_lo(p) ? P.L.w_img_lo : P.L.w_img, P.k_slabs, s, n_pad, a_tile, a_dst, b_dst,
-                                      &full[stage]);
+                                      &full[stage], TM * 128u);
                 } else {
                     const int s = (v - virt1) / P.passes, p = (v - virt1) - s * P.passes;
                     issue_slab_copies(pass_b_lo(p) ? P.wt_next_img_lo : P.wt_next_img, P.k_slabs2, s, n_pad,
-                                      (pass_a_lo(p) ? P.dz_next_img_lo : P.dz_next_img) + dzn_off, a_dst, b_dst, &full[stage]);
+                                      (pass_a_lo(p) ? P.dz_next_img_lo : P.dz_next_img) + dzn_off, a_dst, b_dst, &full[stage],
+                                      TM * 128u);
                 }
             }
         }
         __syncwarp();
     } else if (warp == 4 * CG + 1) {
         if (lane == 0) {
-            const uint32_t idesc = umma_idesc_tf32((uint32_t)n_pad, 0, 0);
+            const uint32_t idesc = umma_idesc_tf32((uint32_t)n_pad, 0, 0, TM);
             for (int s = 0; s < total_slabs; ++s) {
                 int stage = s % NSTAGE, it = s / NSTAGE;
                 mbar_wait(&full[stage], it & 1);
@@ -1023,8 +1095,9 @@ __global__ void __launch_bounds__(n_threads(CG), 1) layer_bwd_kernel(const __gri
         __syncwarp();
     } else {
         const int q4 = warp & 3, cg = warp >> 2;
-        const int row = q4 * 32 + lane;
-        const long long lrow = (long long)tile * TILE_M + row;
+        const int row = G::row(q4, lane), irow = irow0 + row, grp = G::group(cg, lane), coff = G::chunk_off(lane);
+        const int c_begin = grp * (8 / NG), c_end = (grp + 1) * (8 / NG);     // chunks of each slab this thread generates
+        const long long lrow = (long long)tile * TM + row;
         const bool rvalid = lrow < P.pts.n_rows;
         const long long grow = P.pts.row_begin + lrow;
         if (BASIS) {
@@ -1044,11 +1117,11 @@ __global__ void __launch_bounds__(n_threads(CG), 1) layer_bwd_kernel(const __gri
                         const int s = v / P.passes, p = v - s * P.passes;
                         const uint32_t sa = smem_u32(sA + (size_t)stage * SLAB_FLOATS);
                         if (pass_a_lo(p))
-                            gen_basis_slab_soa<FN, true, 2>(P.basis, ctab, s, x, y, t, xrow, sa, (uint32_t)row, cg * (8 / CG),
-                                                            (cg + 1) * (8 / CG), nullptr);
+                            gen_basis_slab_soa<FN, true, 2>(P.basis, ctab, s, x, y, t, xrow, sa, (uint32_t)row, c_begin,
+                                                            c_end, nullptr);
                         else
-                            gen_basis_slab_soa<FN, false, 2>(P.basis, ctab, s, x, y, t, xrow, sa, (uint32_t)row, cg * (8 / CG),
-                                                             (cg + 1) * (8 / CG), nullptr);
+                            gen_basis_slab_soa<FN, false, 2>(P.basis, ctab, s, x, y, t, xrow, sa, (uint32_t)row, c_begin,
+                                                             c_end, nullptr);
                         fence_proxy_async_smem();
                     }
                     mbar_arrive_warp(&full[stage]);
@@ -1061,7 +1134,7 @@ __global__ void __launch_bounds__(n_threads(CG), 1) layer_bwd_kernel(const __gri
         mbar_wait(accf, 0);
         tc_fence_after();
         const uint32_t trow = tmem_base + ((uint32_t)(q4 * 32) << 16);
-        float* myred = red + ((size_t)cg * TILE_M + row) * RED_STRIDE;
+        float* myred = red + ((size_t)grp * TM + row) * RED_STRIDE;
         const float* arow = (P.addend && rvalid) ? P.addend + (size_t)lrow * n_out : nullptr;
         float mean = 0.0f, rstd = 1.0f;
         if (has_ln && rvalid) {
@@ -1080,20 +1153,27 @@ __global__ void __launch_bounds__(n_threads(CG), 1) layer_bwd_kernel(const __gri
         float z[32], g[32], tmp[32];
 
         // pass A: g = dL/dy (after dropout+ReLU backward); LN row sums; dgamma/dbeta/head column sums
+        // a chunk at n_pad (TM = 64, odd number of 32-column chunks) reads zeros and writes nothing: its columns fail
+        // col < n_out below, so it contributes nothing to the row and column sums
         int ch = 0;
-        for (int c0 = 32 * cg; c0 < n_pad; c0 += 32 * CG, ++ch) {
+        for (int wc = G::WARP_COLS * cg; wc < n_pad; wc += WSTEP, ++ch) {
+            const int c0 = wc + coff;
+            const bool cvalid = TM == 128 || c0 < n_pad;
             if (P.x_img) {
-                image_load_chunk(P.x_img, tile, n_pad / SLAB_K, c0, (uint32_t)row, z);    // x saved by the forward
+                if (cvalid) image_load_chunk(P.x_img, itile, n_pad / SLAB_K, c0, (uint32_t)irow, z);    // x saved by the forward
             } else {
-                tmem_ld32(trow + c0, z);
+                acc_ld<TM>(trow + wc, z);
                 if (arow) add_addend_chunk(z, arow, c0, n_out);
 #pragma unroll
                 for (int i = 0; i < 32; ++i) z[i] += sbias[c0 + i];
             }
-            if (!HEAD) tmem_ld32(trow + acc1_off + c0, g);
-            else head_dh_chunk(g, dyh, shw, n_pad, c0, q);
+            if (!cvalid)
+#pragma unroll
+                for (int i = 0; i < 32; ++i) z[i] = 0.0f;
+            if (!HEAD) acc_ld<TM>(trow + acc1_off + wc, g);
+            else head_dh_chunk(g, dyh, shw, n_pad, c0, cvalid ? q : 0);
             uint32_t keep = 0xFFFFFFFFu;
-            if (drop) {
+            if (drop && cvalid) {
                 keep = 0;
 #pragma unroll 1
                 for (int b = 0; b < 4; ++b)
@@ -1125,8 +1205,7 @@ __global__ void __launch_bounds__(n_threads(CG), 1) layer_bwd_kernel(const __gri
                     const float dk = dyh[k];
 #pragma unroll
                     for (int i = 0; i < 32; ++i) hv[i] = dk * tmp[i];
-                    float s = warp_transpose_sum(hv, lane);
-                    atomicAdd(&cs_hw[k * n_pad + c0 + lane], s);
+                    colsum_chunk<TM>(cs_hw + k * n_pad, c0, cvalid, hv, lane);
                 }
             }
             if (has_ln) {
@@ -1137,50 +1216,52 @@ __global__ void __launch_bounds__(n_threads(CG), 1) layer_bwd_kernel(const __gri
                     Sb = fmaf(gy, z[i], Sb);
                     tmp[i] = g[i] * z[i];
                 }
-                float s = warp_transpose_sum(tmp, lane);
-                atomicAdd(&cs_gam[c0 + lane], s);
+                colsum_chunk<TM>(cs_gam, c0, cvalid, tmp, lane);
 #pragma unroll
                 for (int i = 0; i < 32; ++i) tmp[i] = g[i];
-                s = warp_transpose_sum(tmp, lane);
-                atomicAdd(&cs_bet[c0 + lane], s);
+                colsum_chunk<TM>(cs_bet, c0, cvalid, tmp, lane);
             } else {
-                store_operand_chunk(P.dz_img, P.dz_img_lo, tile, n_pad / SLAB_K, c0, (uint32_t)row, g);
-                float s = warp_transpose_sum(g, lane);
-                atomicAdd(&cs_bias[c0 + lane], s);
+                if (cvalid) store_operand_chunk(P.dz_img, P.dz_img_lo, itile, n_pad / SLAB_K, c0, (uint32_t)irow, g);
+                colsum_chunk<TM>(cs_bias, c0, cvalid, g, lane);
             }
         }
         if (HEAD && cg == 0) {
             for (int k = 0; k < q; ++k) {
-                float s = warp_sum(dyh[k]);
+                float s = warp_sum(TM == 128 || lane < 16 ? dyh[k] : 0.0f);    // a TM = 64 row sits in both half-warps
                 if (lane == 0) atomicAdd(&cs_hb[k], s);
             }
         }
         // pass B (LayerNorm): dz = rstd * (gy - mean(gy) - xh * mean(gy * xh))
         if (has_ln) {
-            if (CG > 1) {
+            if (NG > 1) {
                 myred[0] = Sa;
                 myred[1] = Sb;
                 worker_barrier(NW);
                 Sa = Sb = 0.0f;
 #pragma unroll
-                for (int gq = 0; gq < CG; ++gq) {
-                    Sa += red[((size_t)gq * TILE_M + row) * RED_STRIDE];
-                    Sb += red[((size_t)gq * TILE_M + row) * RED_STRIDE + 1];
+                for (int gq = 0; gq < NG; ++gq) {
+                    Sa += red[((size_t)gq * TM + row) * RED_STRIDE];
+                    Sb += red[((size_t)gq * TM + row) * RED_STRIDE + 1];
                 }
             }
             const float ma = Sa * inv_n, mb = Sb * inv_n;
             ch = 0;
-            for (int c0 = 32 * cg; c0 < n_pad; c0 += 32 * CG, ++ch) {
+            for (int wc = G::WARP_COLS * cg; wc < n_pad; wc += WSTEP, ++ch) {
+                const int c0 = wc + coff;
+                const bool cvalid = TM == 128 || c0 < n_pad;
                 if (P.x_img) {
-                    image_load_chunk(P.x_img, tile, n_pad / SLAB_K, c0, (uint32_t)row, z);
+                    if (cvalid) image_load_chunk(P.x_img, itile, n_pad / SLAB_K, c0, (uint32_t)irow, z);
                 } else {
-                    tmem_ld32(trow + c0, z);
+                    acc_ld<TM>(trow + wc, z);
                     if (arow) add_addend_chunk(z, arow, c0, n_out);
 #pragma unroll
                     for (int i = 0; i < 32; ++i) z[i] += sbias[c0 + i];
                 }
-                if (!HEAD) tmem_ld32(trow + acc1_off + c0, g);
-                else head_dh_chunk(g, dyh, shw, n_pad, c0, q);
+                if (!cvalid)
+#pragma unroll
+                    for (int i = 0; i < 32; ++i) z[i] = 0.0f;
+                if (!HEAD) acc_ld<TM>(trow + acc1_off + wc, g);
+                else head_dh_chunk(g, dyh, shw, n_pad, c0, cvalid ? q : 0);
                 uint32_t act = 0;
 #pragma unroll
                 for (int k = 0; k < MAXCH; ++k)
@@ -1194,9 +1275,8 @@ __global__ void __launch_bounds__(n_threads(CG), 1) layer_bwd_kernel(const __gri
                     float dz = rstd * (gy - ma - xh * mb);
                     g[i] = (col < n_out && rvalid) ? dz : 0.0f;
                 }
-                store_operand_chunk(P.dz_img, P.dz_img_lo, tile, n_pad / SLAB_K, c0, (uint32_t)row, g);
-                float s = warp_transpose_sum(g, lane);
-                atomicAdd(&cs_bias[c0 + lane], s);
+                if (cvalid) store_operand_chunk(P.dz_img, P.dz_img_lo, itile, n_pad / SLAB_K, c0, (uint32_t)irow, g);
+                colsum_chunk<TM>(cs_bias, c0, cvalid, g, lane);
             }
         }
         tc_fence_before();

@@ -102,6 +102,27 @@ __device__ __forceinline__ void tmem_ld32(uint32_t taddr, float (&v)[32]) {
     for (int i = 0; i < 32; ++i) v[i] = __uint_as_float(r[i]);
 }
 
+// The accumulator of an M = 64 MMA (cta_group::1) fills lanes 0-15 of each warp's 32-lane quarter.  16 lanes x two
+// runs of 32 consecutive 32-bit columns, the second `split` columns after the first: thread i of the warp receives lane
+// (base_lane + i % 16), run i / 16.
+template <int SPLIT>
+__device__ __forceinline__ void tmem_ld16x2(uint32_t taddr, float (&v)[32]) {
+    uint32_t r[32];
+    asm volatile(
+        "tcgen05.ld.sync.aligned.16x32bx2.x32.b32 "
+        "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
+        "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32], %33;"
+        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]),
+          "=r"(r[8]), "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]),
+          "=r"(r[16]), "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]),
+          "=r"(r[24]), "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
+        : "r"(taddr), "n"(SPLIT)
+        : "memory");
+    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+#pragma unroll
+    for (int i = 0; i < 32; ++i) v[i] = __uint_as_float(r[i]);
+}
+
 // Issue only (no wait): several loads can be in flight before one tmem_ld_wait().
 __device__ __forceinline__ void tmem_ld32_issue(uint32_t taddr, float (&r)[32]) {
     asm volatile(
@@ -148,12 +169,13 @@ __device__ __forceinline__ uint64_t umma_desc_sw128(uint32_t saddr, uint32_t lbo
     return (uint64_t)((saddr & 0x3FFFFu) >> 4) | ((uint64_t)((lbo_bytes >> 4) & 0x3FFFu) << 16) |
            ((uint64_t)((sbo_bytes >> 4) & 0x3FFFu) << 32) | (1ull << 46) | (2ull << 61);
 }
-// Instruction descriptor, kind::tf32, FP32 accumulate, M=128.
+// Instruction descriptor, kind::tf32, FP32 accumulate, M = 128 or 64 (cta_group::1).
 // c_format[4,6)=1 (F32) a_format[7,10)=2 (TF32) b_format[10,13)=2 a_major[15] b_major[16] (1 = MN-major)
 // n_dim[17,23)=N>>3 m_dim[24,29)=M>>4
-__device__ __forceinline__ uint32_t umma_idesc_tf32(uint32_t n, uint32_t a_mn_major, uint32_t b_mn_major) {
+__device__ __forceinline__ uint32_t umma_idesc_tf32(uint32_t n, uint32_t a_mn_major, uint32_t b_mn_major,
+                                                    uint32_t m = 128) {
     return (1u << 4) | (2u << 7) | (2u << 10) | (a_mn_major << 15) | (b_mn_major << 16) | ((n >> 3) << 17) |
-           ((128u >> 4) << 24);
+           ((m >> 4) << 24);
 }
 // D[tmem] (+)= A[smem] * B[smem]; issued by ONE thread.
 __device__ __forceinline__ void umma_tf32(uint32_t taddr, uint64_t adesc, uint64_t bdesc, uint32_t idesc,

@@ -90,8 +90,9 @@ class Executor:
     # walk with the ~20 knots per level inside a support disk.
     DENSE_MAX_KNOTS = 2048
     # Up to this many rows a training forward also stores x = A W^T + b of every block (1 KB/row/block) so that the
-    # backward skips its recomputation GEMM (and, for block 1, regenerating the basis for it): a batch this small is a
-    # single wave of 128-row tiles, bound by per-kernel latency, not by HBM.  Larger batches recompute instead.
+    # backward skips its recomputation GEMM (and, for block 1, regenerating the basis for it): a batch this small is at
+    # most two CTAs of 128 rows per SM, bound by per-kernel latency, not by HBM.  Larger batches recompute instead.
+    # Batches of at most 128 rows per two SMs (9,472 on 148 SMs) run layer_fwd / layer_bwd in one wave of 64-row tiles.
     # (The N x K basis matrix is never stored either way; wgrad regenerates it.)
     SAVE_X_MAX_ROWS = 148 * 2 * 128
     # Beyond that the step is throughput-bound and evaluating the basis three times (forward, the backward's recompute
