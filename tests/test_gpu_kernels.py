@@ -156,10 +156,18 @@ def _run_dense(ops, L, A, W, bias, gamma=None, beta=None, eps=1e-5):
     return ops.unpack_image(out, rows, n_out).cpu().numpy(), stats.cpu().numpy()
 
 
+# Row counts that put layer_fwd on 128-row tiles (148 SMs): 9,473 and 20,000 rows with 4 column groups, 37,765 rows
+# (296 tiles, at least two per SM) with 2; all three end in a ragged tile.
+ROWS_TM128 = (9473, 20000, 37765)
+DENSE_TM128 = [(r, i, o) for r in ROWS_TM128 for i in (32, 297) for o in (16, 48, 96, 160, 256)]
+
+
 @pytest.mark.parametrize("rows,n_in,n_out", [(128, 32, 32), (128, 64, 128), (200, 96, 48), (384, 256, 256),
-                                             (1000, 297, 256), (130, 256, 128), (77, 128, 16), (128, 512, 64)])
+                                             (1000, 297, 256), (130, 256, 128), (77, 128, 16), (128, 512, 64)]
+                         + DENSE_TM128)
 def test_dense_gemm_relu_exact_tf32(rows, n_in, n_out):
-    """K-major tcgen05 path: operands pre-rounded to TF32 => products exact, only FP32 summation order differs."""
+    """K-major tcgen05 path: operands pre-rounded to TF32 => products exact, only FP32 summation order differs.
+    Up to 1,000 rows the launch runs on 64-row tiles; the ROWS_TM128 sizes run on 128-row tiles (148 SMs)."""
     L, ops, *_ = _mods()
     rng = np.random.default_rng(rows + n_in + n_out)
     A = orc.tf32_round(rng.standard_normal((rows, n_in)).astype(np.float32))
@@ -171,8 +179,9 @@ def test_dense_gemm_relu_exact_tf32(rows, n_in, n_out):
     assert np.all(np.abs(got - ref) <= 2e-5 + np.abs(ref) * 2.0 ** -11)
 
 
-@pytest.mark.parametrize("rows,n_in,n_out", [(256, 256, 256), (300, 96, 48), (128, 297, 128)])
+@pytest.mark.parametrize("rows,n_in,n_out", [(256, 256, 256), (300, 96, 48), (128, 297, 128)] + DENSE_TM128)
 def test_dense_layernorm_epilogue(rows, n_in, n_out):
+    """LayerNorm epilogue: 64-row tiles up to 300 rows, 128-row tiles with 4 and 2 column groups at ROWS_TM128."""
     L, ops, *_ = _mods()
     rng = np.random.default_rng(5)
     A = orc.tf32_round(rng.standard_normal((rows, n_in)).astype(np.float32))
@@ -191,9 +200,13 @@ def test_dense_layernorm_epilogue(rows, n_in, n_out):
 
 
 @pytest.mark.parametrize("rows,n_in,n_out", [(128, 32, 32), (256, 256, 256), (1000, 297, 256), (300, 128, 48),
-                                             (4096, 256, 128), (130, 40, 16)])
+                                             (4096, 256, 128), (130, 40, 16), (20000, 297, 256), (65613, 297, 256),
+                                             (20000, 256, 128), (65613, 256, 128)])
 def test_wgrad_mn_major_exact_tf32(rows, n_in, n_out):
-    """MN-major tcgen05 path: dW = dz^T A with both operands read from the forward's images."""
+    """MN-major tcgen05 path: dW = dz^T A with both operands read from the forward's images.  wgrad always reads whole
+    128-row tiles and gives each of its row splits every n_split-th tile: up to 4,096 rows (32 tiles) a split gets at most
+    one tile; at 20,000 and 65,613 rows (157 and 513 tiles, the last ragged) a split accumulates up to 5 and 14 tiles
+    (148 SMs: 37 splits for 297 x 256, 148 for 256 x 128)."""
     L, ops, *_ = _mods()
     rng = np.random.default_rng(rows * 7 + n_in)
     A = orc.tf32_round(rng.standard_normal((rows, n_in)).astype(np.float32))
@@ -617,15 +630,9 @@ def _small_net(rng, k_s, k_t=25, hidden=(64, 32)):
     return ws, bs, gs, be
 
 
-@pytest.mark.parametrize("fn,learnable,precision", [("wendland", True, "tf32x3"), ("wendland", True, "tf32"),
-                                                   ("triangular", False, "tf32"), ("wendland", False, "tf32")])
-def test_cell_list_regime_arbitrary_and_learnable_knots_vs_oracle(fn, learnable, precision):
-    """Support walk over a NON-lattice knot set (data-adaptive placement: clustered centres, per-knot bandwidths, some
-    knots outside [0,1]^2 as drifted learnable knots are) through the device-built per-level cell list: forward, loss,
-    every gradient -- including d centres / d log-bandwidths from the same walk -- vs the FP64 oracle, and the dense
-    path on the same model.  One level is crowded on purpose (> 300 knots inside a support): nothing is truncated."""
-    L, ops, Executor, NetSpec, LossSpec = _mods()
-    rng = np.random.default_rng(33)
+def _cell_list_knots(rng):
+    """1,360 knots in three levels (60, 400, 900) that are not a lattice: clustered centres, per-knot bandwidths, some
+    centres outside [0,1]^2; the 400-knot level is crowded (wide supports around (0.5, 0.5)).  Returns (c, b, sizes)."""
     sizes = [60, 400, 900]
     cen, bw = [], []
     for li, k in enumerate(sizes):
@@ -637,7 +644,19 @@ def test_cell_list_regime_arbitrary_and_learnable_knots_vs_oracle(fn, learnable,
             b = rng.uniform(0.6, 1.0, k) * 2.5 / np.sqrt(k)
         cen.append(c)
         bw.append(b)
-    c, b = np.concatenate(cen).astype(np.float32), np.concatenate(bw).astype(np.float32)
+    return np.concatenate(cen).astype(np.float32), np.concatenate(bw).astype(np.float32), sizes
+
+
+@pytest.mark.parametrize("fn,learnable,precision", [("wendland", True, "tf32x3"), ("wendland", True, "tf32"),
+                                                   ("triangular", False, "tf32"), ("wendland", False, "tf32")])
+def test_cell_list_regime_arbitrary_and_learnable_knots_vs_oracle(fn, learnable, precision):
+    """Support walk over a NON-lattice knot set (data-adaptive placement: clustered centres, per-knot bandwidths, some
+    knots outside [0,1]^2 as drifted learnable knots are) through the device-built per-level cell list: forward, loss,
+    every gradient -- including d centres / d log-bandwidths from the same walk -- vs the FP64 oracle, and the dense
+    path on the same model.  One level is crowded on purpose (> 300 knots inside a support): nothing is truncated."""
+    L, ops, Executor, NetSpec, LossSpec = _mods()
+    rng = np.random.default_rng(33)
+    c, b, sizes = _cell_list_knots(rng)
     tc, tb = orc.temporal_knots([10, 15])
     ws, bs, gs, be = _small_net(rng, c.shape[0])
     m = orc.OracleModel(centers=c, bandwidths=b, t_centers=tc, t_bandwidths=tb, weights=ws, biases=bs, ln_gamma=gs,
