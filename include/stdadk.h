@@ -334,6 +334,17 @@ int stdadk_predict_field(const stdadk_field_args* a, void* stream);
 int stdadk_layer_fwd(const stdadk_fwd_args* a, void* stream);
 int stdadk_layer_bwd(const stdadk_bwd_args* a, void* stream);
 int stdadk_wgrad(const stdadk_wgrad_args* a, void* stream);
+
+/* Whether block 1 can generate its basis densely in shared memory: the block-1 launches fit in 227 KB, by the same
+ * shared-memory plans the launchers check.  training = 0: the forward only (stdadk_layer_fwd in both CTA
+ * configurations), what a prediction runs; training = 1: also stdadk_layer_bwd regenerating the basis and stdadk_wgrad
+ * in basis form, every launch a training step can make.  n_in = p_cov + k_s + k_t inputs, n_out outputs; q_head = Q
+ * when block 1 is also the last hidden block (it carries the head), else 0.  Host-only: no device is needed.  1 yes,
+ * 0 no (the launch that does not fit in stdadk_last_error). */
+int stdadk_dense_basis_supported(int32_t n_in, int32_t n_out, int32_t k_s, int32_t k_t, int32_t q_head, int32_t training);
+/* Largest k_s for which stdadk_dense_basis_supported(p_cov + k_s + k_t, n_out, k_s, k_t, q_head, training) holds, -1 if
+ * none. */
+int32_t stdadk_dense_max_knots(int32_t p_cov, int32_t k_t, int32_t n_out, int32_t q_head, int32_t training);
 int stdadk_knot_grad(const stdadk_knotgrad_args* a, void* stream);
 
 /* sqnorms[g] = sum of squares of g over each group.  Bitwise deterministic (replicas of a data-parallel run must

@@ -138,6 +138,8 @@ _PROTOS = {
     "stdadk_layer_fwd": (C.c_int, [C.POINTER(FwdArgs), fp]),
     "stdadk_layer_bwd": (C.c_int, [C.POINTER(BwdArgs), fp]),
     "stdadk_wgrad": (C.c_int, [C.POINTER(WgradArgs), fp]),
+    "stdadk_dense_basis_supported": (C.c_int, [C.c_int32] * 6),
+    "stdadk_dense_max_knots": (C.c_int32, [C.c_int32] * 5),
     "stdadk_knot_grad": (C.c_int, [C.POINTER(KnotGradArgs), fp]),
     "stdadk_sqnorm_ws_floats": (C.c_size_t, []),
     "stdadk_grad_sqnorm": (C.c_int, [fp, C.c_int64, C.c_int, C.POINTER(C.c_int64), fp, fp, fp]),

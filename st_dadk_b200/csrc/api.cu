@@ -259,6 +259,18 @@ static int check_layer(const stdadk_layer& l, const char* who) {
     return 0;
 }
 
+// Shared memory of the layer_fwd / layer_bwd launches.  stdadk_dense_basis_supported checks block 1's launches with
+// these same functions (and wgrad_smem_bytes), so the executor's regime choice and the launch checks cannot disagree.
+constexpr uint32_t SMEM_LIMIT = 227 * 1024;
+constexpr int BWD_CG = 2, BWD_NS = 4;
+// cg = 4 (latency configuration, 4 stages) or 2 (two CTAs per SM, 2 stages); tab_chunks = k_slabs * 8 with a basis
+static uint32_t fwd_smem(int n_pad, int q, int k_s, int k_t, int tab_chunks, int cg) {
+    return plan_smem(n_pad, q, k_s, k_t, false, cg, cg == 2 ? 2 : 4, tab_chunks).total;
+}
+static uint32_t bwd_smem(int n_pad, int q, int k_s, int k_t, int tab_chunks) {
+    return plan_smem(n_pad, q, k_s, k_t, true, BWD_CG, BWD_NS, tab_chunks).total;
+}
+
 static unsigned long long* g_predict_dbg = nullptr;   // stdadk_debug_counters (profiling builds)
 int stdadk_layer_fwd(const stdadk_fwd_args* a, void* stream) {
     if (int r = check_device()) return r;
@@ -318,16 +330,16 @@ int stdadk_layer_fwd(const stdadk_fwd_args* a, void* stream) {
     const bool half_tiles = 2 * tiles <= sms;
     if (half_tiles) tiles *= 2;
     K.tmem_cols = half_tiles ? tmem_cols_m64(K.n_pad) : pow2_cols(K.n_pad);
-    const int ns = cg == 2 ? 2 : 4;   // 1 CTA/SM in the latency configuration: spend the shared memory on pipeline depth
-    SmemPlan sp = plan_smem(K.n_pad, K.has_head ? K.head.q : 0, basis ? K.basis.k_s : 0, basis ? K.basis.k_t : 0, false, cg, ns,
-                            basis ? K.k_slabs * 8 : 0);
-    REQUIRE(sp.total <= 227 * 1024, "layer_fwd: needs %u B of shared memory (> 227 KB): too many knots for the dense path",
-            sp.total);
+    // 1 CTA/SM in the latency configuration: spend the shared memory on pipeline depth (4 stages, else 2)
+    const uint32_t smem = fwd_smem(K.n_pad, K.has_head ? K.head.q : 0, basis ? K.basis.k_s : 0, basis ? K.basis.k_t : 0,
+                                   basis ? K.k_slabs * 8 : 0, cg);
+    REQUIRE(smem <= SMEM_LIMIT, "layer_fwd: needs %u B of shared memory (> 227 KB): too many knots for the dense path",
+            smem);
     K.n_tiles = tiles;
-#define LAUNCH_FWD(B, TM, C)                                                                                     \
-    do {                                                                                                         \
-        if (int r = set_smem(layer_fwd_kernel<B, TM, C, (C == 2 ? 2 : 4)>, sp.total)) return r;                  \
-        layer_fwd_kernel<B, TM, C, (C == 2 ? 2 : 4)><<<tiles, n_threads(C), sp.total, (cudaStream_t)stream>>>(K); \
+#define LAUNCH_FWD(B, TM, C)                                                                                 \
+    do {                                                                                                     \
+        if (int r = set_smem(layer_fwd_kernel<B, TM, C, (C == 2 ? 2 : 4)>, smem)) return r;                  \
+        layer_fwd_kernel<B, TM, C, (C == 2 ? 2 : 4)><<<tiles, n_threads(C), smem, (cudaStream_t)stream>>>(K); \
     } while (0)
     if (basis) {
         if (half_tiles) LAUNCH_FWD(true, 64, 4);
@@ -553,10 +565,10 @@ int stdadk_layer_bwd(const stdadk_bwd_args* a, void* stream) {
     K.thresh16 = dropout_thresh16(a->drop.p);
     K.drop_scale = a->drop.p > 0.0f ? 1.0f / (1.0f - a->drop.p) : 1.0f;
     const bool basis = a->basis != nullptr && a->x_img == nullptr;
-    constexpr int BCG = 2, BNS = 4;
-    SmemPlan sp = plan_smem(K.n_pad, K.has_head ? K.head.q : 0, basis ? K.basis.k_s : 0, basis ? K.basis.k_t : 0, true, BCG, BNS,
-                            basis ? K.k_slabs * 8 : 0);
-    REQUIRE(sp.total <= 227 * 1024, "layer_bwd: needs %u B of shared memory (> 227 KB)", sp.total);
+    constexpr int BCG = BWD_CG, BNS = BWD_NS;
+    const uint32_t smem = bwd_smem(K.n_pad, K.has_head ? K.head.q : 0, basis ? K.basis.k_s : 0, basis ? K.basis.k_t : 0,
+                                   basis ? K.k_slabs * 8 : 0);
+    REQUIRE(smem <= SMEM_LIMIT, "layer_bwd: needs %u B of shared memory (> 227 KB)", smem);
     int tiles = (int)ceil_div64(a->pts.n_rows, TILE_M);
     // one wave of 64-row tiles (as in layer_fwd), only with x saved by the forward: there is no recompute GEMM then
     const int sms = g_sm_count > 0 ? g_sm_count : 148;
@@ -564,10 +576,10 @@ int stdadk_layer_bwd(const stdadk_bwd_args* a, void* stream) {
     if (half_tiles) tiles *= 2;
     K.tmem_cols = 2 * (half_tiles ? tmem_cols_m64(K.n_pad) : pow2_cols(K.n_pad));
     const bool ln = a->layer.gamma != nullptr, hd = a->head != nullptr;
-#define LAUNCH_BWD(B, TM, LNV, HD)                                                                              \
-    do {                                                                                                        \
-        if (int r = set_smem(layer_bwd_kernel<B, TM, BCG, BNS, LNV, HD>, sp.total)) return r;                   \
-        layer_bwd_kernel<B, TM, BCG, BNS, LNV, HD><<<tiles, n_threads(BCG), sp.total, (cudaStream_t)stream>>>(K); \
+#define LAUNCH_BWD(B, TM, LNV, HD)                                                                          \
+    do {                                                                                                    \
+        if (int r = set_smem(layer_bwd_kernel<B, TM, BCG, BNS, LNV, HD>, smem)) return r;                   \
+        layer_bwd_kernel<B, TM, BCG, BNS, LNV, HD><<<tiles, n_threads(BCG), smem, (cudaStream_t)stream>>>(K); \
     } while (0)
     if (half_tiles) {
         if (ln && hd) LAUNCH_BWD(false, 64, true, true);
@@ -627,7 +639,7 @@ int stdadk_wgrad(const stdadk_wgrad_args* a, void* stream) {
     if (splits > K.n_row_tiles) splits = K.n_row_tiles;
     const bool basis = a->basis != nullptr;
     uint32_t smem = wgrad_smem_bytes(basis ? K.basis.k_s : 0, basis ? K.basis.k_t : 0);
-    REQUIRE(smem <= 227 * 1024, "wgrad: needs %u B of shared memory (> 227 KB)", smem);
+    REQUIRE(smem <= SMEM_LIMIT, "wgrad: needs %u B of shared memory (> 227 KB)", smem);
     dim3 grid(splits, m_tiles, n_tiles_n);
     constexpr int WCG = 2;
     if (basis) {
@@ -638,6 +650,42 @@ int stdadk_wgrad(const stdadk_wgrad_args* a, void* stream) {
         wgrad_kernel<false, WCG><<<grid, n_threads(WCG), smem, (cudaStream_t)stream>>>(K);
     }
     return check_launch("wgrad");
+}
+
+// The block-1 launches of the dense path: layer_fwd in both CTA configurations (every forward), and with `training`
+// also layer_bwd regenerating the basis (batches the forward saves no x for) and the basis-form wgrad.
+static int dense_basis_check(int n_in, int n_out, int k_s, int k_t, int q_head, int training) {
+    REQUIRE(n_out >= 1 && n_out <= MAX_N && k_s >= 0 && k_t >= 0 && n_in >= k_s + k_t && q_head >= 0 &&
+                q_head <= STDADK_MAX_Q,
+            "dense_basis_supported: bad sizes n_in=%d n_out=%d k_s=%d k_t=%d q_head=%d", n_in, n_out, k_s, k_t, q_head);
+    const int n_pad = pad32(n_out), tab_chunks = pad32(n_in) / SLAB_K * 8;
+    for (int cg : {4, 2}) {
+        const uint32_t b = fwd_smem(n_pad, q_head, k_s, k_t, tab_chunks, cg);
+        REQUIRE(b <= SMEM_LIMIT, "layer_fwd: needs %u B of shared memory (> 227 KB): too many knots for the dense path", b);
+    }
+    if (!training) return 0;
+    const uint32_t bb = bwd_smem(n_pad, q_head, k_s, k_t, tab_chunks);
+    REQUIRE(bb <= SMEM_LIMIT, "layer_bwd: needs %u B of shared memory (> 227 KB)", bb);
+    const uint32_t wb = wgrad_smem_bytes(k_s, k_t);
+    REQUIRE(wb <= SMEM_LIMIT, "wgrad: needs %u B of shared memory (> 227 KB)", wb);
+    return 0;
+}
+
+int stdadk_dense_basis_supported(int32_t n_in, int32_t n_out, int32_t k_s, int32_t k_t, int32_t q_head, int32_t training) {
+    return dense_basis_check(n_in, n_out, k_s, k_t, q_head, training) == 0 ? 1 : 0;
+}
+
+int32_t stdadk_dense_max_knots(int32_t p_cov, int32_t k_t, int32_t n_out, int32_t q_head, int32_t training) {
+    if (p_cov < 0 || dense_basis_check(p_cov + k_t, n_out, 0, k_t, q_head, training)) return -1;
+    // shared memory grows with k_s in every launch: bisect for the last k_s that fits.  Each layer_fwd chunk of 4
+    // features takes 64 B of table, so 1 << 14 knots exceed 227 KB in every configuration.
+    int lo = 0, hi = 1 << 14;
+    while (hi - lo > 1) {
+        const int mid = (lo + hi) / 2;
+        if (dense_basis_check(p_cov + mid + k_t, n_out, mid, k_t, q_head, training) == 0) lo = mid;
+        else hi = mid;
+    }
+    return lo;
 }
 
 int stdadk_knot_grad(const stdadk_knotgrad_args* a, void* stream) {

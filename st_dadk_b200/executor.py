@@ -87,7 +87,10 @@ class Executor:
     MAX_WORKSPACES = 4
     # Above this many spatial knots block 1 switches from generating every basis column densely in the tensor-core
     # operand to walking each point's compact support (st_dadk_b200/csrc/sparse.cuh): dense work grows with K_s, the
-    # walk with the ~20 knots per level inside a support disk.
+    # walk with the ~20 knots per level inside a support disk.  This is the performance crossover only.  The dense
+    # kernels keep block 1's knot tables in shared memory, and below it they may already not hold them: at first
+    # width 256 and 70 temporal knots the recompute backward takes at most 1,626 knots
+    # (stdadk_dense_basis_supported).  Such networks walk as well, and raise at construction when they cannot.
     DENSE_MAX_KNOTS = 2048
     # Up to this many rows a training forward also stores x = A W^T + b of every block (1 KB/row/block) so that the
     # backward skips its recomputation GEMM (and, for block 1, regenerating the basis for it): a batch this small is at
@@ -107,7 +110,9 @@ class Executor:
     def __init__(self, spec: NetSpec, force_sparse: bool = False, force_dense: bool = False):
         self.spec = spec
         self.force_sparse = force_sparse
-        self.force_dense = force_dense        # keep the dense operand even above DENSE_MAX_KNOTS (while it fits in SMEM)
+        # keep the dense operand even above DENSE_MAX_KNOTS.  Raises at construction when the dense forward cannot hold
+        # the knots; when only the training launches cannot (predict_only), training calls raise before any launch.
+        self.force_dense = force_dense
         self._setup_regime(spec)
         dev = spec.centers.device
         if dev.type != "cuda":
@@ -145,8 +150,26 @@ class Executor:
     def _setup_regime(self, spec: NetSpec):
         if spec.precision not in ("tf32", "tf32x3"):
             raise ValueError(f"precision must be 'tf32' or 'tf32x3', got {spec.precision!r}")
-        k_s = spec.centers.shape[0]
-        want = (self.force_sparse or k_s > self.DENSE_MAX_KNOTS) and not self.force_dense
+        k_s, k_t = spec.centers.shape[0], spec.t_centers.shape[0]
+        n_out = spec.weights[0].shape[0]
+        q_head = spec.q if spec.n_hidden == 1 else 0        # a single hidden block carries the head
+        fits, why = ops.dense_basis_supported(spec.p_cov, k_s, k_t, n_out, q_head)
+        too_big = ""
+        self.predict_only = None
+        if not fits:
+            limit = ops.dense_max_knots(spec.p_cov, k_t, n_out, q_head)
+            too_big = (f"the dense path holds at most {limit} spatial knots with a first block of {n_out} outputs "
+                       f"and {k_t} temporal knots ({why})")
+            if self.force_dense:
+                # forced dense: predictions need the forward only; training calls are refused before any launch
+                fwd_fits, fwd_why = ops.dense_basis_supported(spec.p_cov, k_s, k_t, n_out, q_head, training=False)
+                if not fwd_fits:
+                    fwd_limit = ops.dense_max_knots(spec.p_cov, k_t, n_out, q_head, training=False)
+                    raise RuntimeError(f"force_dense: {k_s} spatial knots do not fit: the dense forward holds at most "
+                                       f"{fwd_limit} spatial knots with a first block of {n_out} outputs and {k_t} "
+                                       f"temporal knots ({fwd_why})")
+                self.predict_only = f"force_dense: {k_s} spatial knots can be predicted but not trained: {too_big}"
+        want = self.force_sparse or (not self.force_dense and (k_s > self.DENSE_MAX_KNOTS or not fits))
         self.sparse = False
         self.lat = None
         self.level_begin = None
@@ -163,9 +186,10 @@ class Executor:
         if sum(sizes) != k_s or len(sizes) > 8:
             problems.append("level_sizes must be at most 8 contiguous ranges adding up to the number of knots")
         if problems:
-            if self.force_sparse or k_s * 16 > 96 * 1024:
-                raise RuntimeError(f"{k_s} spatial knots need the support-walking path, but " + "; ".join(problems))
-            return
+            if self.force_sparse or not fits:
+                reason = f" ({too_big})" if too_big else ""
+                raise RuntimeError(f"{k_s} spatial knots need the support-walking path{reason}, but " + "; ".join(problems))
+            return          # above DENSE_MAX_KNOTS, but the dense kernels still hold the knots
         if spec.lattice_sides is not None and not spec.learnable_basis:
             # fixed uniform lattice: candidate windows in closed form
             sides = [int(v) for v in spec.lattice_sides]
@@ -301,6 +325,8 @@ class Executor:
         if n == 0:          # empty batch: nothing to launch (empty tensors have no storage to hand to the library)
             self._ctx = None
             return out if out is not None else torch.empty(0, s.q, dtype=torch.float32, device=self.device)
+        if (save or train) and self.predict_only:
+            raise RuntimeError(self.predict_only)
         if not prepared:
             # always rebuild the operand images: parameter storage can be rewritten in place by kernels or by
             # an EMA swap without any version counter the executor could observe (5 tiny launches)

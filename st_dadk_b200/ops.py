@@ -196,6 +196,20 @@ def knot_grad(args: L.KnotGradArgs):
     L.check(L.lib().stdadk_knot_grad(C.byref(args), _stream()), "knot_grad")
 
 
+def dense_basis_supported(p_cov: int, k_s: int, k_t: int, n_out: int, q_head: int, training: bool = True) -> tuple:
+    """(fits, reason): whether the dense block-1 launches of a training step (training=True) or of a prediction hold
+    this shape in shared memory; reason names the launch that does not."""
+    lib = L.lib()
+    if lib.stdadk_dense_basis_supported(p_cov + k_s + k_t, n_out, k_s, k_t, q_head, int(training)):
+        return True, ""
+    return False, lib.stdadk_last_error().decode("utf-8", "replace")
+
+
+def dense_max_knots(p_cov: int, k_t: int, n_out: int, q_head: int, training: bool = True) -> int:
+    """Largest number of spatial knots for which dense_basis_supported holds (-1: none)."""
+    return int(L.lib().stdadk_dense_max_knots(p_cov, k_t, n_out, q_head, int(training)))
+
+
 _sqnorm_ws = {}
 
 

@@ -325,10 +325,11 @@ def test_host_buffer_step_sync_and_lagged_match_device_step():
 
 def test_trainer_learnable_knots_cell_list_path_equals_dense_path_and_scales_to_5000():
     """A learnable, data-adaptive (random_site) model trains through the support walk with the per-step device-built
-    cell list (knots move every step; knot gradients come from the same walk).  At 1,900 knots -- the largest set the
-    dense kernels still hold in shared memory -- the same model forced through the dense operand (all columns generated,
-    knot gradients on the tensor cores) must follow the same losses and reach the same parameters (tf32x3, so operand
-    rounding does not blur the comparison).  The 5,000-knot model (beyond the dense path) must train: finite,
+    cell list (knots move every step; knot gradients come from the same walk).  At 1,900 knots -- which the dense kernels
+    hold at first width 64 (up to 2,134 with its 70 temporal knots, bound by wgrad's knot table; at width 256 the
+    recompute backward holds at most 1,626, test_gpu_dense_knots) -- the same model forced through the dense operand (all columns
+    generated, knot gradients on the tensor cores) must follow the same losses and reach the same parameters (tf32x3, so
+    operand rounding does not blur the comparison).  The 5,000-knot model (beyond the dense path) must train: finite,
     decreasing loss, moving knots."""
     from stnf.models import STInterpMLP
     from stnf.dataio import ObservationTable
