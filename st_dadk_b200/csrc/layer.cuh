@@ -404,9 +404,15 @@ __device__ __forceinline__ void gen_basis_slab(const BasisP& B, const float4* sk
 // Producer: B slab (n_pad rows of the weight image, split over its 128-row tiles) [+ A slab: a_bytes from a_tile_img,
 // the whole 128-row slab or, for a 64-row tile, its half: 64 rows are 8 whole swizzle periods, so either half of an
 // image slab is already in the MMA's layout].
+// With `a_later`, the barrier is armed for both slabs but only the B slab is copied: the A slab comes from the
+// predecessor kernel and is issued after pdl_wait() with issue_a_slab.
+__device__ __forceinline__ void issue_a_slab(int slab, const float* a_tile_img, float* sA, uint64_t* bar,
+                                             uint32_t a_bytes) {
+    bulk_g2s(sA, a_tile_img + (size_t)slab * SLAB_FLOATS, a_bytes, bar);
+}
 __device__ __forceinline__ void issue_slab_copies(const float* w_img, int w_slabs, int slab, int n_pad,
                                                   const float* a_tile_img, float* sA, float* sB, uint64_t* bar,
-                                                  uint32_t a_bytes = SLAB_BYTES) {
+                                                  uint32_t a_bytes = SLAB_BYTES, bool a_later = false) {
     uint32_t bytes = (uint32_t)n_pad * 128u + (a_tile_img ? a_bytes : 0u);
     mbar_arrive_expect_tx(bar, bytes);
     for (int r0 = 0; r0 < n_pad; r0 += TILE_M) {
@@ -414,7 +420,7 @@ __device__ __forceinline__ void issue_slab_copies(const float* w_img, int w_slab
         const float* src = w_img + ((size_t)(r0 / TILE_M) * w_slabs + slab) * SLAB_FLOATS;
         bulk_g2s(sB + (size_t)r0 * SLAB_K, src, (uint32_t)rows * 128u, bar);
     }
-    if (a_tile_img) bulk_g2s(sA, a_tile_img + (size_t)slab * SLAB_FLOATS, a_bytes, bar);
+    if (a_tile_img && !a_later) issue_a_slab(slab, a_tile_img, sA, bar, a_bytes);
 }
 
 // Knot tables (knots4: cx, cy, theta'^2, 1/theta'; tknots2: c, 1/bw) -> shared memory with bulk async copies (TMA 1-D)
@@ -875,7 +881,24 @@ __global__ void __launch_bounds__(n_threads(CG), CG <= 2 ? 2 : 1) layer_fwd_kern
         if (lane == 0) {
             const size_t a_off = (size_t)itile * P.k_slabs * SLAB_FLOATS + (size_t)irow0 * SLAB_K;
             const int n_virt = P.k_slabs * P.passes;
-            for (int v = 0; v < n_virt; ++v) {
+            // blocks 2+: the weight slabs of the first stages (packed at least two launches back) go out before the
+            // wait, the activation slabs (the previous block's output) after it.  Block 1's W1 is packed by the launch
+            // just before this one.
+            const int n_pre = BASIS ? 0 : min(n_virt, NSTAGE);
+            for (int v = 0; v < n_pre; ++v) {
+                const int s = v / P.passes, p = v - s * P.passes;
+                issue_slab_copies(pass_b_lo(p) ? P.L.w_img_lo : P.L.w_img, P.k_slabs, s, n_pad,
+                                  (pass_a_lo(p) ? P.a_img_lo : P.a_img) + a_off, sA + (size_t)v * SLAB_FLOATS,
+                                  sB + v * b_stage_floats, &full[v], TM * 128u, true);
+            }
+            pdl_wait();
+            pdl_launch_dependents();
+            for (int v = 0; v < n_pre; ++v) {
+                const int s = v / P.passes, p = v - s * P.passes;
+                issue_a_slab(s, (pass_a_lo(p) ? P.a_img_lo : P.a_img) + a_off, sA + (size_t)v * SLAB_FLOATS, &full[v],
+                             TM * 128u);
+            }
+            for (int v = n_pre; v < n_virt; ++v) {
                 const int s = v / P.passes, p = v - s * P.passes;
                 int stage = v % NSTAGE, it = v / NSTAGE;
                 if (it > 0) FWD_WAIT(7, mbar_wait(&empty[stage], (it - 1) & 1));
@@ -904,6 +927,9 @@ __global__ void __launch_bounds__(n_threads(CG), CG <= 2 ? 2 : 1) layer_fwd_kern
         __syncwarp();
     } else {
         // ---------------- workers: thread = (row, column group)
+        // The points may have been written by the launch just before this one (a prediction call's inputs), the
+        // addend by the support walk just before block 1, and the epilogue writes global memory: wait first.
+        pdl_wait();
         const int q4 = warp & 3, cg = warp >> 2;
         const int row = G::row(q4, lane), grp = G::group(cg, lane);     // grp: the thread's 8 / NG chunks of each slab
         const long long lrow = (long long)tile * TM + row;
@@ -1059,7 +1085,21 @@ __global__ void __launch_bounds__(n_threads(CG), 1) layer_bwd_kernel(const __gri
         if (lane == 0) {
             const size_t a_off = (size_t)itile * P.k_slabs * SLAB_FLOATS + (size_t)irow0 * SLAB_K;
             const size_t dzn_off = (size_t)itile * P.k_slabs2 * SLAB_FLOATS + (size_t)irow0 * SLAB_K;
+            // Before the wait: the first stages' slabs that come from further back than the previous launch -- both
+            // operands of the recompute GEMM (weights, earlier activations) and W_next^T of the dgrad GEMM.  dz_next
+            // is the previous launch's output: its slabs of those stages are issued after the wait.
+            const int n_pre = min(total_slabs, NSTAGE);
+            auto wait_then_dz_next = [&]() {
+                pdl_wait();
+                pdl_launch_dependents();
+                for (int v = virt1; v < n_pre; ++v) {
+                    const int s = (v - virt1) / P.passes, p = (v - virt1) - s * P.passes;
+                    issue_a_slab(s, (pass_a_lo(p) ? P.dz_next_img_lo : P.dz_next_img) + dzn_off,
+                                 sA + (size_t)v * SLAB_FLOATS, &full[v], TM * 128u);
+                }
+            };
             for (int v = 0; v < total_slabs; ++v) {
+                if (v == n_pre) wait_then_dz_next();
                 int stage = v % NSTAGE, it = v / NSTAGE;
                 if (it > 0) mbar_wait(&empty[stage], (it - 1) & 1);
                 float* a_dst = sA + (size_t)stage * SLAB_FLOATS;
@@ -1073,9 +1113,10 @@ __global__ void __launch_bounds__(n_threads(CG), 1) layer_bwd_kernel(const __gri
                     const int s = (v - virt1) / P.passes, p = (v - virt1) - s * P.passes;
                     issue_slab_copies(pass_b_lo(p) ? P.wt_next_img_lo : P.wt_next_img, P.k_slabs2, s, n_pad,
                                       (pass_a_lo(p) ? P.dz_next_img_lo : P.dz_next_img) + dzn_off, a_dst, b_dst, &full[stage],
-                                      TM * 128u);
+                                      TM * 128u, v < n_pre);
                 }
             }
+            if (total_slabs == n_pre) wait_then_dz_next();
         }
         __syncwarp();
     } else if (warp == 4 * CG + 1) {
@@ -1131,6 +1172,9 @@ __global__ void __launch_bounds__(n_threads(CG), 1) layer_bwd_kernel(const __gri
             else if (P.basis.fn == STDADK_TRIANGULAR) gen_all(std::integral_constant<int, STDADK_TRIANGULAR>{});
             else gen_all(std::integral_constant<int, STDADK_GAUSSIAN>{});
         }
+        // the regenerated operand reads only points and knot tables, which the forward read before; the epilogue
+        // reads the previous launch's output
+        pdl_wait();
         mbar_wait(accf, 0);
         tc_fence_after();
         const uint32_t trow = tmem_base + ((uint32_t)(q4 * 32) << 16);
@@ -1378,6 +1422,31 @@ __device__ __forceinline__ void restage_half_tiles(const float* dz_tile, int msl
     }
 }
 
+// Block 1's wgrad: the basis half (B operand, MN-major) of one stage for (row tile, half, tf32x3 pass), regenerated
+// from the points and the knot tables.  Out of line: the kernel calls it before and after pdl_wait(), and two inlined
+// copies cost the kernel six registers.
+template <int NW>
+__device__ __noinline__ void wgrad_gen_basis_half(const WgradK& P, const float4* sk, const float2* st, int rt, int half,
+                                                  int pass, uint32_t sb, int row64, int par, int n_chunks) {
+    float x = 0.f, y = 0.f, t = 0.f;
+    const float* xrow = nullptr;
+    long long lrow = (long long)rt * TILE_M + half * WG_HALF_ROWS + row64;
+    if (lrow < P.pts.n_rows) {
+        long long grow = P.pts.row_begin + lrow;
+        load_point(P.pts, grow, x, y, t);
+        if (P.basis.p_cov > 0 && P.pts.xcov) xrow = P.pts.xcov + sample_of(P.pts, grow) * P.basis.p_cov;
+    }
+    const int ni = blockIdx.z;
+    for (int c = par; c < n_chunks; c += NW / 64) {
+        const int slab = ni * P.nt_slabs + c;
+#pragma unroll 1
+        for (int c16 = 0; c16 < 8; ++c16) {
+            float4 v = feature_chunk(P.basis, sk, st, slab * SLAB_K + c16 * 4, x, y, t, xrow, pass_b_lo(pass));
+            st_shared_v4(sb + c * WG_CHUNK_BYTES + swz32_off((uint32_t)row64, (uint32_t)c16), v.x, v.y, v.z, v.w);
+        }
+    }
+}
+
 template <bool BASIS, int CG>
 __global__ void __launch_bounds__(n_threads(CG), 1) wgrad_kernel(const __grid_constant__ WgradK P) {
     constexpr int NW = n_work(CG), NT = n_threads(CG);
@@ -1452,22 +1521,27 @@ __global__ void __launch_bounds__(n_threads(CG), 1) wgrad_kernel(const __grid_co
             __syncwarp();
         } else if (warp < 4 * CG) {
             const int row64 = tid & 63, par = tid >> 6;
+            auto gen_basis = [&](int rt, int half, int pass, int stage) {
+                wgrad_gen_basis_half<NW>(P, sk, st, rt, half, pass, smem_u32(stage_base + stage * WG_STAGE_BYTES) + WG_A_BYTES,
+                                         row64, par, n_chunks);
+            };
+            // Before the wait: the basis halves of the first stages (points and knot tables, read by the forward
+            // before).  After it: dz, the previous launch's output.
+            const int n_pre = BASIS ? min(n_iter, WG_NSTAGE) : 0;
             int itn = 0;
-            if (BASIS) mbar_wait(kbar, 0);
+            if (BASIS) {
+                mbar_wait(kbar, 0);
+                for (int rt = split; rt < P.n_row_tiles && itn < n_pre; rt += n_split)
+                    for (int hp = 0; hp < 2 * P.passes && itn < n_pre; ++hp, ++itn)
+                        gen_basis(rt, hp / P.passes, hp % P.passes, itn);
+            }
+            pdl_wait();
+            pdl_launch_dependents();
+            itn = 0;
             for (int rt = split; rt < P.n_row_tiles; rt += n_split)
                 for (int hp = 0; hp < 2 * P.passes; ++hp, ++itn) {
                     const int half = hp / P.passes, pass = hp - half * P.passes;
                     int stage = itn % WG_NSTAGE, it = itn / WG_NSTAGE;
-                    float x = 0.f, y = 0.f, t = 0.f;
-                    const float* xrow = nullptr;
-                    if (BASIS) {
-                        long long lrow = (long long)rt * TILE_M + half * WG_HALF_ROWS + row64;
-                        if (lrow < P.pts.n_rows) {
-                            long long grow = P.pts.row_begin + lrow;
-                            load_point(P.pts, grow, x, y, t);
-                            if (P.basis.p_cov > 0 && P.pts.xcov) xrow = P.pts.xcov + sample_of(P.pts, grow) * P.basis.p_cov;
-                        }
-                    }
                     if (it > 0) mbar_wait(&empty[stage], (it - 1) & 1);
                     uint32_t sa = smem_u32(stage_base + stage * WG_STAGE_BYTES);
                     uint32_t sb = sa + WG_A_BYTES;
@@ -1476,17 +1550,7 @@ __global__ void __launch_bounds__(n_threads(CG), 1) wgrad_kernel(const __grid_co
                                            BASIS ? nullptr
                                                  : (pass_b_lo(pass) ? P.a_img_lo : P.a_img) + (size_t)rt * P.a_slabs * SLAB_FLOATS,
                                            ni * P.nt_slabs, n_chunks, half, sa, sb, tid);
-                    if (BASIS) {
-                        for (int c = par; c < n_chunks; c += NW / 64) {
-                            const int slab = ni * P.nt_slabs + c;
-#pragma unroll 1
-                            for (int c16 = 0; c16 < 8; ++c16) {
-                                float4 v = feature_chunk(P.basis, sk, st, slab * SLAB_K + c16 * 4, x, y, t, xrow, pass_b_lo(pass));
-                                st_shared_v4(sb + c * WG_CHUNK_BYTES + swz32_off((uint32_t)row64, (uint32_t)c16), v.x, v.y,
-                                             v.z, v.w);
-                            }
-                        }
-                    }
+                    if (BASIS && itn >= n_pre) gen_basis(rt, half, pass, stage);
                     fence_proxy_async_smem();
                     mbar_arrive_warp(&full[stage]);
                 }

@@ -37,6 +37,8 @@ struct PackBatch {
 };
 // blockIdx.y selects the matrix; same per-chunk work as pack_image_kernel
 __global__ void pack_images_kernel(PackBatch B) {
+    pdl_wait();                 // the sources are parameters the previous kernel may have written
+    pdl_launch_dependents();
     const stdadk_pack_desc D = B.d[blockIdx.y];
     const int slabs = (int)((D.cols + SLAB_K - 1) / SLAB_K);
     const long long n_chunks = ((D.rows + TILE_M - 1) / TILE_M) * slabs * (long long)(SLAB_FLOATS / 4);
@@ -422,6 +424,7 @@ __global__ void __launch_bounds__(256) adamw_ema_kernel(AdamK A) {
     __shared__ float s_sq[8];
     int step;
     if (FUSED) {
+        pdl_wait();             // every input comes from the backward; the grid barrier below needs its CTAs gone
         // ---- phase 1: squared norm per group.  Deterministic: the element -> thread map is a function of the grid
         // (itself a function of n), in-block reduction and the sum over blocks are ordered.
         step = *A.step_count + 1;                       // read BEFORE the grid barrier; block 0 publishes it after

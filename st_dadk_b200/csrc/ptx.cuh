@@ -54,6 +54,21 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
     }
 }
 
+// ---------------------------------------------------------------- programmatic dependent launch
+// The training step's kernels are launched with programmatic stream serialisation (api.cu, launch_chained): kernel
+// N+1 may become resident while kernel N still runs, does its independent set-up, and blocks in pdl_wait() until N has
+// completed and its writes are visible.  pdl_wait() returns at once when the kernel has no programmatic prerequisite
+// (eager launches after a plain kernel, the first kernel of a graph).  Every kernel that uses them keeps these rules:
+//  1. A CTA calls pdl_launch_dependents() only after it has passed its own pdl_wait() and its own tcgen05.alloc.  So
+//     when kernel N+1 starts, kernel N-1 has completed: code before N+1's wait overlaps kernel N only, and a dependent
+//     CTA that allocates tensor memory before its wait can only contend with CTAs that already hold theirs.
+//  2. Code before the wait reads only data written before the step began or by kernels at least two launches back on
+//     the same stream (parameters, knot tables, weight images, activations of earlier blocks), and writes only
+//     shared and tensor memory.  Every thread that reads a predecessor's output or writes global memory waits first.
+//  3. A grid-wide barrier (the fused step tail) sits after the wait, where the prerequisites have exited.
+__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
+__device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
+
 // ---------------------------------------------------------------- proxies / fences
 __device__ __forceinline__ void fence_proxy_async_smem() {
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");

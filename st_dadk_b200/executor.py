@@ -629,11 +629,16 @@ class Executor:
                 a.dz_img_lo = ws.dz_lo[l].data_ptr()
             a.d_bias = g["biases"][l].data_ptr()
             ops.layer_bwd(a)
-            # dW_l only needs dz_l: it runs on a second stream, concurrently with the rest of the backward chain
-            # (a 4096-row batch is 32 tiles -- one kernel alone leaves most of the 148 SMs idle)
-            side.wait_stream(main)
-            with torch.cuda.stream(side):
+            if l == 0:
+                # block 1's dW is the last kernel of the chain and the step waits for it: it follows layer_bwd on the
+                # launching stream, where it starts early and regenerates its basis operand while layer_bwd runs
                 self._wgrad_block(l, pts, ws, basis, g)
+            else:
+                # dW_l only needs dz_l: it runs on a second stream, concurrently with the rest of the backward chain
+                # (a 4096-row batch is 32 tiles -- one kernel alone leaves most of the 148 SMs idle)
+                side.wait_stream(main)
+                with torch.cuda.stream(side):
+                    self._wgrad_block(l, pts, ws, basis, g)
         main.wait_stream(side)      # join: every weight gradient is complete before the caller continues
         if s.learnable_basis and not self.sparse:
             a = L.KnotGradArgs()
