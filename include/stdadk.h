@@ -127,6 +127,10 @@ typedef struct {
     float* out_img_lo;       /* tf32x3: residual image of out_img (written together with it) */
 } stdadk_fwd_args;
 
+/* stdadk_bwd_args.settled: the dropout step counter (drop.step_ptr) / the saved x image and its stats */
+#define STDADK_SETTLED_STEP 1
+#define STDADK_SETTLED_X 2
+
 /* Backward of one hidden block: recomputes z = A W^T (for block 1 this recomputes the basis),
  * forms dh (from the head, or dz_next * W_next on the tensor cores), and writes dz image + bias /
  * LayerNorm / head gradients (accumulated with atomics into zero-initialised buffers). */
@@ -143,7 +147,9 @@ typedef struct {
     float* d_head_b;           /* (q) += */
     const float* dz_next_img;  /* image (rows x n_next) */
     const float* wt_next_img;  /* image of W_next^T (n_out x n_next): dgrad operand */
-    int32_t n_next, _pad;
+    int32_t n_next;
+    int32_t settled;           /* STDADK_SETTLED_* bits: inputs that the kernel launched just before this one does not
+                                  write, so a one-wave x-image backward may read them while that kernel still runs */
     float* dz_img;             /* out: image (rows x n_out) */
     float* d_bias;             /* (n_out) += */
     float* d_gamma;            /* (n_out) += or NULL */
@@ -211,7 +217,9 @@ typedef struct {
     int32_t fuse_norm;        /* != 0: ONE launch for the whole step tail -- the kernel forms the squared gradient norms
                                  itself (two phases around a grid barrier; bitwise deterministic), writes them to sqnorms
                                  (which then only needs to be non-NULL when clipping is on), and advances step_count */
-    int32_t _pad;
+    int32_t state_early;      /* fuse_norm only, != 0: the kernel launched just before this one writes none of hyper,
+                                 step_count, p, m, v, shadow (it may write g), so they are loaded while it still runs
+                                 and kept in registers across the grid barrier (n <= 8 x 256 x blocks) */
     float* norm_ws;           /* fuse_norm: (148 * 8 + 8) floats, zero-initialised once */
 } stdadk_adamw_args;
 

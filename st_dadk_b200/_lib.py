@@ -18,6 +18,9 @@ CALIBRATION = {"wendland": 1.0, "gaussian": 0.223477, "triangular": 0.654714}
 fp = C.c_void_p  # device pointers travel as integers
 
 
+SETTLED_STEP, SETTLED_X = 1, 2       # stdadk_bwd_args.settled bits (STDADK_SETTLED_*)
+
+
 class Basis(C.Structure):
     _fields_ = [("knots4", fp), ("tknots2", fp), ("k_s", C.c_int32), ("k_t", C.c_int32), ("p_cov", C.c_int32),
                 ("basis_fn", C.c_int32)]
@@ -53,7 +56,7 @@ class FwdArgs(C.Structure):
 class BwdArgs(C.Structure):
     _fields_ = [("basis", C.POINTER(Basis)), ("pts", Points), ("a_img", fp), ("layer", Layer), ("drop", Dropout),
                 ("stats", fp), ("head", C.POINTER(Head)), ("d_head_w", fp), ("d_head_b", fp), ("dz_next_img", fp),
-                ("wt_next_img", fp), ("n_next", C.c_int32), ("_pad", C.c_int32), ("dz_img", fp), ("d_bias", fp),
+                ("wt_next_img", fp), ("n_next", C.c_int32), ("settled", C.c_int32), ("dz_img", fp), ("d_bias", fp),
                 ("d_gamma", fp), ("d_beta", fp), ("addend", fp), ("x_img", fp), ("a_img_lo", fp), ("dz_next_img_lo", fp),
                 ("wt_next_img_lo", fp), ("dz_img_lo", fp)]
 
@@ -74,7 +77,7 @@ class AdamWArgs(C.Structure):
                 ("n_groups", C.c_int32), ("zero_grad", C.c_int32), ("group_end", C.POINTER(C.c_int64)), ("hyper", fp),
                 ("sqnorms", fp), ("step_count", fp), ("beta1", C.c_float), ("beta2", C.c_float), ("eps", C.c_float),
                 ("ema_decay", C.c_float), ("loss_acc", fp), ("loss_sum", fp), ("loss_last", fp), ("fuse_norm", C.c_int32),
-                ("_pad", C.c_int32), ("norm_ws", fp)]
+                ("state_early", C.c_int32), ("norm_ws", fp)]
 
 
 MAX_LEVELS = 8

@@ -380,6 +380,11 @@ int stdadk_layer_fwd(const stdadk_fwd_args* a, void* stream) {
 // Development aid (not part of include/stdadk.h): 16 device counters of cycles the fused prediction kernel's roles spend
 // waiting; see tools/prof_predict.py.
 extern "C" void stdadk_debug_counters(void* dev_u64x16) { g_predict_dbg = static_cast<unsigned long long*>(dev_u64x16); }
+// Phase stamps of the training step (STEP_T, profiling builds): 8 counters per kernel, layer_bwd of layer l at 8 l
+// (l < 7), the fused tail at 56.  Launches read the pointer when they are made, so a graph keeps the one it was
+// captured with.
+static unsigned long long* g_step_dbg = nullptr;
+extern "C" void stdadk_debug_step_counters(void* dev_u64x64) { g_step_dbg = static_cast<unsigned long long*>(dev_u64x64); }
 
 // The hidden blocks of the whole-network kernels: each block's n_in must be the previous block's n_out.
 static int fill_pred_layers(const stdadk_layer* layers, int n_layers, PredLayerP* out, const char* who) {
@@ -572,6 +577,11 @@ int stdadk_layer_bwd(const stdadk_bwd_args* a, void* stream) {
     K.passes = x3 ? 3 : 1;
     K.addend = a->addend;
     K.x_img = a->x_img;
+    K.step_settled = a->x_img && (a->settled & STDADK_SETTLED_STEP) ? 1 : 0;   // only the x-image backward reads
+    K.x_settled = a->x_img && (a->settled & STDADK_SETTLED_X) ? 1 : 0;         // inputs early
+#ifdef STDADK_PF_DEBUG
+    K.dbg = g_step_dbg && a->layer.layer_id < 7 ? g_step_dbg + 8 * a->layer.layer_id : nullptr;
+#endif
     K.stats = a->stats;
     K.dz_next_img = a->dz_next_img;
     K.wt_next_img = a->wt_next_img;
@@ -928,6 +938,8 @@ int stdadk_adamw_ema_step(const stdadk_adamw_args* a, void* stream) {
     K.eps = a->eps;
     K.ema_decay = a->ema_decay;
     K.g_zero = a->zero_grad ? const_cast<float*>(a->g) : nullptr;
+    K.state_early = a->fuse_norm && a->state_early ? 1 : 0;
+    K.dbg = g_step_dbg ? g_step_dbg + 56 : nullptr;
     K.loss_acc = a->loss_acc;
     K.loss_sum = a->loss_sum;
     K.loss_last = a->loss_last;

@@ -9,6 +9,30 @@
 
 namespace stdadk {
 
+// Development aid of the training step's kernels (-DSTDADK_PF_DEBUG builds, stdadk_debug_step_counters): thread 0 of
+// each CTA adds the globaltimer nanoseconds since its previous stamp to dbg[slot] (slots 0-6) and counts the CTA in
+// dbg[7].  Production builds carry none of it.
+#ifdef STDADK_PF_DEBUG
+#define STEP_T_BEGIN(dbg)                                                  \
+    unsigned long long t_prev_ = 0;                                        \
+    if ((dbg) && threadIdx.x == 0) {                                       \
+        asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t_prev_));        \
+        atomicAdd((dbg) + 7, 1ull);                                        \
+    }
+#define STEP_T(dbg, slot)                                                  \
+    do {                                                                   \
+        if ((dbg) && threadIdx.x == 0) {                                   \
+            unsigned long long now_;                                       \
+            asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(now_));       \
+            atomicAdd((dbg) + (slot), now_ - t_prev_);                     \
+            t_prev_ = now_;                                                \
+        }                                                                  \
+    } while (0)
+#else
+#define STEP_T_BEGIN(dbg)
+#define STEP_T(dbg, slot)
+#endif
+
 constexpr int TILE_M = 128;                  // rows (points) per tile = TMEM lanes
 constexpr int SLAB_K = 32;                   // fp32/tf32 elements per 128-byte operand row
 constexpr int SLAB_FLOATS = TILE_M * SLAB_K; // 4096 floats = 16 KB

@@ -173,6 +173,10 @@ struct BwdK {
     float* d_head_w;
     float* d_head_b;
     int has_head, k_slabs, k_slabs2, n_pad, tmem_cols, passes;
+    int step_settled, x_settled;  // stdadk_bwd_args.settled bits (x-image backward only, else 0)
+#ifdef STDADK_PF_DEBUG
+    unsigned long long* dbg;    // phase stamps (STEP_T)
+#endif
     unsigned int thresh16;
     float drop_scale;
 };
@@ -621,6 +625,26 @@ __device__ __forceinline__ uint32_t pf_keep_mask(unsigned long long seed, uint32
     for (int b = 0; b < 4; ++b) keep |= dropout_keep8(seed, step, layer, key_row, (uint32_t)(c0 / 8 + b), thresh16) << (8 * b);
     return keep;
 }
+// keep bits of each of the thread's 32-column chunks (the column loop of the epilogues), indexed by chunk; a chunk at
+// n_pad (TM = 64) keeps everything, as its columns are dropped by col < n_out anyway
+template <int TM, int CG, int MAXCH>
+__device__ __forceinline__ void chunk_keep_masks(const LayerP& L, unsigned int thresh16, long long lrow, int cg, int lane,
+                                                 int n_pad, uint32_t (&keeps)[MAXCH]) {
+    using G = TileGeo<TM>;
+    const bool drop = L.drop_p > 0.0f;
+    const unsigned int step = drop ? dropout_step(L) : 0u;
+    int ch = 0;
+    for (int wc = G::WARP_COLS * cg; wc < n_pad; wc += G::WARP_COLS * CG, ++ch) {
+        const int c0 = wc + G::chunk_off(lane);
+        const uint32_t kb = (drop && (TM == 128 || c0 < n_pad))
+                                ? pf_keep_mask(L.seed, step, (uint32_t)L.layer_id, L.key_offset + (unsigned long long)lrow,
+                                               c0, thresh16)
+                                : 0xFFFFFFFFu;
+#pragma unroll
+        for (int k = 0; k < MAXCH; ++k)
+            if (k == ch) keeps[k] = kb;
+    }
+}
 __device__ __forceinline__ void pf_dropout(float (&v)[32], uint32_t keep, float scale) {
 #pragma unroll
     for (int i = 0; i < 32; ++i) v[i] = ((keep >> i) & 1u) ? v[i] * scale : 0.0f;
@@ -1042,6 +1066,7 @@ __global__ void __launch_bounds__(n_threads(CG), 1) layer_bwd_kernel(const __gri
 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int tile = blockIdx.x;
+    STEP_T_BEGIN(P.dbg);
     const int itile = tile / (TILE_M / TM), irow0 = (tile % (TILE_M / TM)) * TM;   // image tile, first row in it
     const int n_pad = P.n_pad, n_out = P.L.n_out;
     constexpr bool has_ln = LN;
@@ -1080,6 +1105,7 @@ __global__ void __launch_bounds__(n_threads(CG), 1) layer_bwd_kernel(const __gri
     __syncthreads();
     tc_fence_after();
     const uint32_t tmem_base = *tmem_slot;
+    STEP_T(P.dbg, 0);   // prologue
 
     if (warp == 4 * CG) {
         if (lane == 0) {
@@ -1172,29 +1198,75 @@ __global__ void __launch_bounds__(n_threads(CG), 1) layer_bwd_kernel(const __gri
             else if (P.basis.fn == STDADK_TRIANGULAR) gen_all(std::integral_constant<int, STDADK_TRIANGULAR>{});
             else gen_all(std::integral_constant<int, STDADK_GAUSSIAN>{});
         }
+        const uint32_t trow = tmem_base + ((uint32_t)(q4 * 32) << 16);
+        const bool drop = P.L.drop_p > 0.0f;
+        const float inv_n = 1.0f / (float)n_out;
+        float mean = 0.0f, rstd = 1.0f;
+        uint32_t actbits[MAXCH];     // before pass A of a chunk its keep bits (when formed before the wait), after it
+                                     // its activation bits
+        float z[32], g[32], tmp[32];
+        auto load_stats = [&]() {
+            if (has_ln && rvalid) {
+                mean = P.stats[2 * lrow];
+                rstd = P.stats[2 * lrow + 1];
+            }
+        };
+        // Before the wait, when the caller says the inputs are settled (ptx.cuh, rule 2; the launcher passes the bits
+        // to the one-wave x-image backward only, the recompute backward keeps its order): the keep bits and, for a
+        // 64-row tile of a block below the head, whose x image and stats are at least two launches old, x^ and the
+        // activation bits.  x^ goes to the half of tensor memory that the recompute GEMM would use (an x-image backward
+        // has none): the warp's chunk at column wc sits in columns wc / 2 .. +31, one 32x32b lane per thread, so the
+        // epilogue reads it back with one tcgen05.ld instead of two dependent trips to L2.
+        constexpr bool X_EARLY_OK = TM == 64 && !HEAD;
+        const bool keeps_early = P.step_settled != 0;
+        const bool x_early = X_EARLY_OK && keeps_early && P.x_settled != 0;
+        if (keeps_early) chunk_keep_masks<TM, CG, MAXCH>(P.L, P.thresh16, lrow, cg, lane, n_pad, actbits);
+        if (x_early) {
+            load_stats();
+            int ch = 0;
+            for (int wc = G::WARP_COLS * cg; wc < n_pad; wc += WSTEP, ++ch) {
+                const int c0 = wc + coff;
+                const bool cvalid = c0 < n_pad;
+                if (cvalid) image_load_chunk(P.x_img, itile, n_pad / SLAB_K, c0, (uint32_t)irow, z);
+                else
+#pragma unroll
+                    for (int i = 0; i < 32; ++i) z[i] = 0.0f;
+                uint32_t keep = 0, act = 0;
+#pragma unroll
+                for (int k = 0; k < MAXCH; ++k)
+                    if (k == ch) keep = actbits[k];
+#pragma unroll
+                for (int i = 0; i < 32; ++i) {
+                    const int col = c0 + i;
+                    const float xh = has_ln ? (z[i] - mean) * rstd : z[i];
+                    const float yv = has_ln ? fmaf(xh, sgam[col], sbet[col]) : z[i];
+                    const bool on = (yv > 0.0f) && ((keep >> i) & 1u) && (col < n_out) && rvalid;
+                    act |= (on ? 1u : 0u) << i;
+                    z[i] = xh;
+                }
+#pragma unroll
+                for (int k = 0; k < MAXCH; ++k)
+                    if (k == ch) actbits[k] = act;
+                tmem_st32(trow + (uint32_t)(wc / 2), z);
+            }
+            tmem_st_wait();
+        }
+        STEP_T(P.dbg, 1);   // work before the wait
         // the regenerated operand reads only points and knot tables, which the forward read before; the epilogue
         // reads the previous launch's output
         pdl_wait();
+        STEP_T(P.dbg, 2);   // wait for the previous launch
+        if (!x_early) load_stats();
         mbar_wait(accf, 0);
         tc_fence_after();
-        const uint32_t trow = tmem_base + ((uint32_t)(q4 * 32) << 16);
+        STEP_T(P.dbg, 3);   // accumulator ready
         float* myred = red + ((size_t)grp * TM + row) * RED_STRIDE;
         const float* arow = (P.addend && rvalid) ? P.addend + (size_t)lrow * n_out : nullptr;
-        float mean = 0.0f, rstd = 1.0f;
-        if (has_ln && rvalid) {
-            mean = P.stats[2 * lrow];
-            rstd = P.stats[2 * lrow + 1];
-        }
         float dyh[STDADK_MAX_Q];
 #pragma unroll
         for (int k = 0; k < STDADK_MAX_Q; ++k)
             dyh[k] = (HEAD && rvalid && k < q) ? P.head.dyhat[lrow * q + k] : 0.0f;
-        const bool drop = P.L.drop_p > 0.0f;
-        const unsigned int drop_step = drop ? dropout_step(P.L) : 0u;
-        const float inv_n = 1.0f / (float)n_out;
-        uint32_t actbits[MAXCH];
         float Sa = 0.0f, Sb = 0.0f;
-        float z[32], g[32], tmp[32];
 
         // pass A: g = dL/dy (after dropout+ReLU backward); LN row sums; dgamma/dbeta/head column sums
         // a chunk at n_pad (TM = 64, odd number of 32-column chunks) reads zeros and writes nothing: its columns fail
@@ -1203,7 +1275,9 @@ __global__ void __launch_bounds__(n_threads(CG), 1) layer_bwd_kernel(const __gri
         for (int wc = G::WARP_COLS * cg; wc < n_pad; wc += WSTEP, ++ch) {
             const int c0 = wc + coff;
             const bool cvalid = TM == 128 || c0 < n_pad;
-            if (P.x_img) {
+            if (x_early) {
+                tmem_ld32(trow + (uint32_t)(wc / 2), z);       // x^
+            } else if (P.x_img) {
                 if (cvalid) image_load_chunk(P.x_img, itile, n_pad / SLAB_K, c0, (uint32_t)irow, z);    // x saved by the forward
             } else {
                 acc_ld<TM>(trow + wc, z);
@@ -1211,38 +1285,46 @@ __global__ void __launch_bounds__(n_threads(CG), 1) layer_bwd_kernel(const __gri
 #pragma unroll
                 for (int i = 0; i < 32; ++i) z[i] += sbias[c0 + i];
             }
-            if (!cvalid)
+            if (!cvalid && !x_early)
 #pragma unroll
                 for (int i = 0; i < 32; ++i) z[i] = 0.0f;
             if (!HEAD) acc_ld<TM>(trow + acc1_off + wc, g);
             else head_dh_chunk(g, dyh, shw, n_pad, c0, cvalid ? q : 0);
-            uint32_t keep = 0xFFFFFFFFu;
-            if (drop && cvalid) {
-                keep = 0;
-#pragma unroll 1
-                for (int b = 0; b < 4; ++b)
-                    keep |= dropout_keep8(P.L.seed, drop_step, (uint32_t)P.L.layer_id, P.L.key_offset + (unsigned long long)lrow,
-                                          (uint32_t)(c0 / 8 + b), P.thresh16)
-                            << (8 * b);
-            }
-            uint32_t act = 0;
+            if (x_early) {
+                uint32_t act = 0;
 #pragma unroll
-            for (int i = 0; i < 32; ++i) {
-                const int col = c0 + i;
-                float x = z[i];
-                float xh = has_ln ? (x - mean) * rstd : x;
-                float yv = has_ln ? fmaf(xh, sgam[col], sbet[col]) : x;
-                bool on = (yv > 0.0f) && ((keep >> i) & 1u) && (col < n_out) && rvalid;
-                act |= (on ? 1u : 0u) << i;
-                const float dh = g[i];
-                float h = on ? yv * P.drop_scale : 0.0f;  // forward activation (for the head gradient)
-                g[i] = on ? dh * P.drop_scale : 0.0f;
-                z[i] = xh;
-                tmp[i] = h;
-            }
+                for (int k = 0; k < MAXCH; ++k)
+                    if (k == ch) act = actbits[k];
 #pragma unroll
-            for (int k = 0; k < MAXCH; ++k)
-                if (k == ch) actbits[k] = act;
+                for (int i = 0; i < 32; ++i) g[i] = ((act >> i) & 1u) ? g[i] * P.drop_scale : 0.0f;
+            } else {
+                uint32_t keep = 0xFFFFFFFFu, act = 0;
+                if (keeps_early) {
+#pragma unroll
+                    for (int k = 0; k < MAXCH; ++k)
+                        if (k == ch) keep = actbits[k];
+                } else if (drop && cvalid) {
+                    keep = pf_keep_mask(P.L.seed, dropout_step(P.L), (uint32_t)P.L.layer_id,
+                                        P.L.key_offset + (unsigned long long)lrow, c0, P.thresh16);
+                }
+#pragma unroll
+                for (int i = 0; i < 32; ++i) {
+                    const int col = c0 + i;
+                    float x = z[i];
+                    float xh = has_ln ? (x - mean) * rstd : x;
+                    float yv = has_ln ? fmaf(xh, sgam[col], sbet[col]) : x;
+                    bool on = (yv > 0.0f) && ((keep >> i) & 1u) && (col < n_out) && rvalid;
+                    act |= (on ? 1u : 0u) << i;
+                    const float dh = g[i];
+                    float h = on ? yv * P.drop_scale : 0.0f;  // forward activation (for the head gradient)
+                    g[i] = on ? dh * P.drop_scale : 0.0f;
+                    z[i] = xh;
+                    tmp[i] = h;
+                }
+#pragma unroll
+                for (int k = 0; k < MAXCH; ++k)
+                    if (k == ch) actbits[k] = act;
+            }
             if (HEAD) {
                 for (int k = 0; k < q; ++k) {
                     float hv[32];
@@ -1269,6 +1351,7 @@ __global__ void __launch_bounds__(n_threads(CG), 1) layer_bwd_kernel(const __gri
                 colsum_chunk<TM>(cs_bias, c0, cvalid, g, lane);
             }
         }
+        STEP_T(P.dbg, 4);   // pass A
         if (HEAD && cg == 0) {
             for (int k = 0; k < q; ++k) {
                 float s = warp_sum(TM == 128 || lane < 16 ? dyh[k] : 0.0f);    // a TM = 64 row sits in both half-warps
@@ -1293,7 +1376,9 @@ __global__ void __launch_bounds__(n_threads(CG), 1) layer_bwd_kernel(const __gri
             for (int wc = G::WARP_COLS * cg; wc < n_pad; wc += WSTEP, ++ch) {
                 const int c0 = wc + coff;
                 const bool cvalid = TM == 128 || c0 < n_pad;
-                if (P.x_img) {
+                if (x_early) {
+                    tmem_ld32(trow + (uint32_t)(wc / 2), z);   // x^
+                } else if (P.x_img) {
                     if (cvalid) image_load_chunk(P.x_img, itile, n_pad / SLAB_K, c0, (uint32_t)irow, z);
                 } else {
                     acc_ld<TM>(trow + wc, z);
@@ -1301,7 +1386,7 @@ __global__ void __launch_bounds__(n_threads(CG), 1) layer_bwd_kernel(const __gri
 #pragma unroll
                     for (int i = 0; i < 32; ++i) z[i] += sbias[c0 + i];
                 }
-                if (!cvalid)
+                if (!cvalid && !x_early)
 #pragma unroll
                     for (int i = 0; i < 32; ++i) z[i] = 0.0f;
                 if (!HEAD) acc_ld<TM>(trow + acc1_off + wc, g);
@@ -1313,7 +1398,7 @@ __global__ void __launch_bounds__(n_threads(CG), 1) layer_bwd_kernel(const __gri
 #pragma unroll
                 for (int i = 0; i < 32; ++i) {
                     const int col = c0 + i;
-                    float xh = (z[i] - mean) * rstd;
+                    float xh = x_early ? z[i] : (z[i] - mean) * rstd;
                     const float dh = g[i];
                     float gy = ((act >> i) & 1u) ? dh * P.drop_scale * sgam[col] : 0.0f;
                     float dz = rstd * (gy - ma - xh * mb);
@@ -1335,6 +1420,7 @@ __global__ void __launch_bounds__(n_threads(CG), 1) layer_bwd_kernel(const __gri
             for (int k = 0; k < q; ++k) atomicAdd(&P.d_head_w[(size_t)k * n_out + c], cs_hw[k * n_pad + c]);
         }
         if (tid < q) atomicAdd(&P.d_head_b[tid], cs_hb[tid]);
+        STEP_T(P.dbg, 5);   // pass B, column-sum flush
     }
     __syncthreads();
     if (warp == 4 * CG) tmem_dealloc(tmem_base, (uint32_t)P.tmem_cols);

@@ -416,26 +416,74 @@ struct AdamK {
     float* sq_out;
     float* norm_ws;        // gridDim.x * 8 partials, then two uint32: arrival counter, generation
     int* step_rw;
+    int state_early;       // stdadk_adamw_args.state_early (fused tail only)
+    unsigned long long* dbg;   // phase stamps of -DSTDADK_PF_DEBUG builds (STEP_T), else NULL
 };
 // torch.optim.AdamW (decoupled decay, bias correction) + clip_grad_norm_ coefficient + ModelEMA.update
 // in one pass: 20 B read + 16 B written per parameter (28 B without EMA).
+// Fused tail: a thread's float4 of p / m / v / shadow (at most TAIL_RES of them) and of g stay in registers from
+// before the wait and the grid barrier to the update, so the update pass takes no memory round trip after the
+// barrier.  A larger model takes the streaming loop.  Either way element i4 belongs to thread i4 mod (grid x 256) and
+// both norm reductions keep their order, so the results are the same bits.
+constexpr int TAIL_RES = 2;
 template <bool FUSED>
 __global__ void __launch_bounds__(256) adamw_ema_kernel(AdamK A) {
     __shared__ float s_sq[8];
+    const long long n4 = A.n >> 2;
+    const long long i0 = blockIdx.x * (long long)blockDim.x + threadIdx.x, stride = (long long)gridDim.x * blockDim.x;
+    const float4* g4 = reinterpret_cast<const float4*>(A.g);
+    float4* p4 = reinterpret_cast<float4*>(A.p);
+    float4* m4 = reinterpret_cast<float4*>(A.m);
+    float4* v4 = reinterpret_cast<float4*>(A.v);
+    float4* s4 = reinterpret_cast<float4*>(A.shadow);
+    const bool early = FUSED && A.state_early;
+    const bool resident = early && n4 <= TAIL_RES * stride;
+    float4 rg[TAIL_RES], rp[TAIL_RES], rm[TAIL_RES], rv[TAIL_RES], rs[TAIL_RES];
+    float hy[8][3];
     int step;
+    auto load_state = [&]() {
+        step = FUSED ? *A.step_count + 1 : *A.step_count;  // fused: read BEFORE the grid barrier, block 0 publishes it
+#pragma unroll
+        for (int k = 0; k < 8; ++k)
+            if (k < A.G.n) {
+                hy[k][0] = A.hyper[4 * k];
+                hy[k][1] = A.hyper[4 * k + 1];
+                hy[k][2] = A.hyper[4 * k + 2];
+            }
+        if (resident) {
+#pragma unroll
+            for (int r = 0; r < TAIL_RES; ++r) {
+                const long long i = i0 + r * stride;
+                if (i < n4) {
+                    rp[r] = p4[i];
+                    rm[r] = m4[i];
+                    rv[r] = v4[i];
+                    rs[r] = s4 ? s4[i] : make_float4(0.f, 0.f, 0.f, 0.f);
+                }
+            }
+        }
+    };
+    STEP_T_BEGIN(A.dbg);
+    // with state_early, hyper-parameters, the step counter and the optimizer state were written by the previous step's
+    // tail or by copies before this step's first kernel: they are loaded before the wait (ptx.cuh, rule 2)
+    if (early) load_state();
+    STEP_T(A.dbg, 0);   // early loads
     if (FUSED) {
-        pdl_wait();             // every input comes from the backward; the grid barrier below needs its CTAs gone
+        pdl_wait();             // g comes from the backward; the grid barrier below needs its CTAs gone
+        STEP_T(A.dbg, 1);   // wait for the backward
+        if (!early) load_state();
+        if (resident) {
+#pragma unroll
+            for (int r = 0; r < TAIL_RES; ++r)
+                if (i0 + r * stride < n4) rg[r] = __ldg(g4 + i0 + r * stride);
+        }
         // ---- phase 1: squared norm per group.  Deterministic: the element -> thread map is a function of the grid
         // (itself a function of n), in-block reduction and the sum over blocks are ordered.
-        step = *A.step_count + 1;                       // read BEFORE the grid barrier; block 0 publishes it after
         float acc[8];
 #pragma unroll
         for (int k = 0; k < 8; ++k) acc[k] = 0.0f;
         if (A.sqnorms) {                                // (sqnorms != NULL <=> clipping is on)
-            const long long n4q = A.n >> 2;
-            const float4* gq = reinterpret_cast<const float4*>(A.g);
-            for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n4q; i += (long long)gridDim.x * blockDim.x) {
-                const float4 v = __ldg(gq + i);
+            auto add_sq = [&](const float4 v, long long i) {
                 const long long e = i << 2;
                 const float vv[4] = {v.x, v.y, v.z, v.w};
 #pragma unroll
@@ -445,9 +493,16 @@ __global__ void __launch_bounds__(256) adamw_ema_kernel(AdamK A) {
                     for (int k = 0; k < 8; ++k)
                         if (k == gi) acc[k] = fmaf(vv[j], vv[j], acc[k]);
                 }
+            };
+            if (resident) {
+#pragma unroll
+                for (int r = 0; r < TAIL_RES; ++r)
+                    if (i0 + r * stride < n4) add_sq(rg[r], i0 + r * stride);
+            } else {
+                for (long long i = i0; i < n4; i += stride) add_sq(__ldg(g4 + i), i);
             }
             if (blockIdx.x == 0 && threadIdx.x < (A.n & 3)) {
-                const long long i = (n4q << 2) + threadIdx.x;
+                const long long i = (n4 << 2) + threadIdx.x;
                 const float v = A.g[i];
                 const int gi = group_of(A.G, i);
 #pragma unroll
@@ -468,6 +523,7 @@ __global__ void __launch_bounds__(256) adamw_ema_kernel(AdamK A) {
             for (int w = 0; w < 8; ++w) sk += wsum[w][threadIdx.x];
             A.norm_ws[blockIdx.x * 8 + threadIdx.x] = sk;
         }
+        STEP_T(A.dbg, 2);   // g, norm partials
         // ---- grid barrier (the grid is at most one block per SM and every block is resident): arrival counter +
         // generation word; bounded wait
         __threadfence();
@@ -497,8 +553,9 @@ __global__ void __launch_bounds__(256) adamw_ema_kernel(AdamK A) {
         }
         if (blockIdx.x == 0 && threadIdx.x == 0) *A.step_rw = step;
         __syncthreads();
+        STEP_T(A.dbg, 3);   // grid barrier, norms
     } else {
-        step = *A.step_count;
+        load_state();
     }
     const float bc1 = 1.0f - powf(A.beta1, (float)step);
     const float bc2 = 1.0f - powf(A.beta2, (float)step);
@@ -509,9 +566,9 @@ __global__ void __launch_bounds__(256) adamw_ema_kernel(AdamK A) {
         lr[k] = wd[k] = 0.0f;
         clip[k] = 1.0f;
         if (k < A.G.n) {
-            lr[k] = A.hyper[4 * k];
-            wd[k] = A.hyper[4 * k + 1];
-            float mx = A.hyper[4 * k + 2];
+            lr[k] = hy[k][0];
+            wd[k] = hy[k][1];
+            float mx = hy[k][2];
             if (A.sqnorms && mx > 0.0f) clip[k] = fminf(1.0f, mx / (sqrtf(FUSED ? s_sq[k] : A.sqnorms[k]) + 1e-6f));
         }
     }
@@ -529,16 +586,7 @@ __global__ void __launch_bounds__(256) adamw_ema_kernel(AdamK A) {
         p -= (l / bc1) * (m / denom);
         sh = A.ema_decay * sh + (1.0f - A.ema_decay) * p;
     };
-    const long long n4 = A.n >> 2;
-    const float4* g4 = reinterpret_cast<const float4*>(A.g);
-    float4* p4 = reinterpret_cast<float4*>(A.p);
-    float4* m4 = reinterpret_cast<float4*>(A.m);
-    float4* v4 = reinterpret_cast<float4*>(A.v);
-    float4* s4 = reinterpret_cast<float4*>(A.shadow);
-    for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n4;
-         i += (long long)gridDim.x * blockDim.x) {
-        float4 g = __ldg(g4 + i), p = p4[i], m = m4[i], v = v4[i];
-        float4 sh = s4 ? s4[i] : make_float4(0.f, 0.f, 0.f, 0.f);
+    auto update4 = [&](long long i, float4 g, float4 p, float4 m, float4 v, float4 sh) {
         const long long e = i << 2;
         update(e, g.x, p.x, m.x, v.x, sh.x);
         update(e + 1, g.y, p.y, m.y, v.y, sh.y);
@@ -549,7 +597,16 @@ __global__ void __launch_bounds__(256) adamw_ema_kernel(AdamK A) {
         v4[i] = v;
         if (s4) s4[i] = sh;
         if (A.g_zero) reinterpret_cast<float4*>(A.g_zero)[i] = make_float4(0.f, 0.f, 0.f, 0.f);
+    };
+    if (resident) {
+#pragma unroll
+        for (int r = 0; r < TAIL_RES; ++r)
+            if (i0 + r * stride < n4) update4(i0 + r * stride, rg[r], rp[r], rm[r], rv[r], rs[r]);
+    } else {
+        for (long long i = i0; i < n4; i += stride)
+            update4(i, __ldg(g4 + i), p4[i], m4[i], v4[i], s4 ? s4[i] : make_float4(0.f, 0.f, 0.f, 0.f));
     }
+    STEP_T(A.dbg, 4);       // update pass
     if (blockIdx.x == 0 && threadIdx.x == 0 && A.loss_acc && A.loss_sum) {
         const float step_loss = *A.loss_acc;
         *A.loss_sum += step_loss;

@@ -65,6 +65,10 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
 //  2. Code before the wait reads only data written before the step began or by kernels at least two launches back on
 //     the same stream (parameters, knot tables, weight images, activations of earlier blocks), and writes only
 //     shared and tensor memory.  Every thread that reads a predecessor's output or writes global memory waits first.
+//     Epilogue inputs count too: where the caller states that an input is that old (stdadk_bwd_args.settled for the
+//     dropout step counter and for a saved x image and its stats, stdadk_adamw_args.state_early for the fused tail's
+//     optimizer state, hyper-parameters and step counter), the one-wave backward's keep bits, x^ and activation bits
+//     and the tail's state are formed or loaded before the wait.
 //  3. A grid-wide barrier (the fused step tail) sits after the wait, where the prerequisites have exited.
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }

@@ -11,6 +11,7 @@ mirroring STInterpMLP.forward (stnf/models/st_interp.py:827-882) and its autogra
 """
 from __future__ import annotations
 
+import os
 import ctypes as C
 from dataclasses import dataclass
 from typing import Dict, List, Optional, Sequence, Tuple
@@ -136,6 +137,10 @@ class Executor:
         self._knots_ready = False
         self._side = None
         self.fused_predict = True      # forward-only calls use the whole-network kernel when the shape fits
+        # the one-wave backward and the fused step tail read settled inputs (dropout step, saved x images, optimizer
+        # state) before their programmatic-launch wait; STDADK_PREWAIT=0 makes them read everything after it (same
+        # results, for comparison)
+        self.prewait = os.environ.get("STDADK_PREWAIT", "1") != "0"
         self._fused_ok = None
         self._field_ok = None
         self._cell_ws = None
@@ -609,6 +614,11 @@ class Executor:
             a.drop = drop
             if ws.x is not None:
                 a.x_img = ws.x[l].data_ptr()
+                # The launch just before a backward is another backward (or, for the head, the last forward), and the
+                # dropout step counter advances in the previous step's tail.  Below the head x and stats come from the
+                # forward, further back.
+                if self.prewait:
+                    a.settled = L.SETTLED_STEP | (L.SETTLED_X if l < nh - 1 else 0)
             if ws.stats[l] is not None:
                 a.stats = ws.stats[l].data_ptr()
                 a.d_gamma = g["gammas"][l].data_ptr()

@@ -227,15 +227,16 @@ def grad_sqnorm(g: torch.Tensor, group_end: Sequence[int], out: torch.Tensor, wo
 
 def adamw_ema_step(p, g, m, v, shadow, group_end: Sequence[int], hyper: torch.Tensor, sqnorms, step_count,
                    beta1=0.9, beta2=0.999, eps=1e-8, ema_decay=0.0, zero_grad=False, loss_acc=None, loss_sum=None,
-                   loss_last=None, norm_ws=None):
+                   loss_last=None, norm_ws=None, state_early=False):
     """zero_grad: the kernel leaves `g` zeroed (next step's zero_grad); loss_acc/loss_sum: device scalars,
     loss_sum += loss_acc; loss_acc = 0 inside the same launch.  norm_ws (zero-initialised (148*8+8) floats): ONE launch for
     the whole step tail -- the kernel computes the squared gradient norms itself (into `sqnorms`, which stays None when
-    clipping is off) and advances the step counter."""
+    clipping is off) and advances the step counter.  state_early (with norm_ws): the kernel launched just before writes
+    none of p / m / v / shadow / hyper / step_count, so the tail loads them while that kernel still runs."""
     arr = (C.c_int64 * len(group_end))(*group_end)
     a = L.AdamWArgs(_ptr(p), _ptr(g), _ptr(m), _ptr(v), _ptr(shadow), p.numel(), len(group_end), int(bool(zero_grad)),
                     arr, _ptr(hyper), _ptr(sqnorms), _ptr(step_count), beta1, beta2, eps, ema_decay, _ptr(loss_acc),
-                    _ptr(loss_sum), _ptr(loss_last), int(norm_ws is not None), 0, _ptr(norm_ws))
+                    _ptr(loss_sum), _ptr(loss_last), int(norm_ws is not None), int(bool(state_early)), _ptr(norm_ws))
     L.check(L.lib().stdadk_adamw_ema_step(C.byref(a), _stream()), "adamw_ema_step")
 
 

@@ -432,7 +432,7 @@ class Trainer:
         ops.adamw_ema_step(fl.p, fl.g[:fl.n], fl.m, fl.v, fl.shadow, fl.group_end, self.hyper,
                            self.sqnorms if self.clip > 0 else None, self.step_count, ema_decay=self.ema_decay,
                            zero_grad=True, loss_acc=ex.loss_acc, loss_sum=self.loss_sum, loss_last=self.loss_last,
-                           norm_ws=self._tail_ws if fused_tail else None)
+                           norm_ws=self._tail_ws if fused_tail else None, state_early=fused_tail and ex.prewait)
         if scratch_tail:
             fl.g[fl.n:fl.n + fl.n_scratch].zero_()
         self._g_clean = True
