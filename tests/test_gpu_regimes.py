@@ -131,16 +131,17 @@ def _add(a, b):
 
 
 def chunked_oracle(m, X, coords, t, y, loss="mse", taus=None, nc_weight=0.0, nc_power=1, key_offset=0,
-                   knot_grads=False, rnd=None, chunk=CHUNK):
+                   knot_grads=False, rnd=None, chunk=CHUNK, seed=SEED, step=STEP):
     """(yhat, loss, gradients) of one training step, memory bounded by `chunk` rows: forward per chunk (dropout masks
-    keyed from key_offset + chunk start), the loss and dL/dyhat once over all rows (its 1/(n Q) and the non-crossing
-    term see the whole batch), then per chunk a forward again and the backward of its slice of dL/dyhat, summed."""
+    of `seed` and `step` keyed from key_offset + chunk start), the loss and dL/dyhat once over all rows (its 1/(n Q) and
+    the non-crossing term see the whole batch), then per chunk a forward again and the backward of its slice of
+    dL/dyhat, summed."""
     n = coords.shape[0]
     hidden = m.weights[:len(m.ln_gamma)]
     spans = [(lo, min(lo + chunk, n)) for lo in range(0, n, chunk)]
 
     def fwd(lo, hi, **kw):
-        masks = [orc.dropout_keep_mask(hi - lo, w.shape[0], m.dropout, SEED, STEP, l, key_offset + lo)
+        masks = [orc.dropout_keep_mask(hi - lo, w.shape[0], m.dropout, seed, step, l, key_offset + lo)
                  for l, w in enumerate(hidden)]
         return orc.forward(m, None if X is None else X[lo:hi], coords[lo:hi], t[lo:hi], train=True, keep_masks=masks,
                            rnd=rnd, **kw)
