@@ -55,7 +55,11 @@ typedef struct {
     const int64_t* index;   /* optional gather: row r reads sample index[row_begin + r] of the arrays (and of y):
                                a mini-batch is a slice of a device-resident permutation, no collate copy
                                (replaces train_st_interp.py:453-460) */
-    int32_t grid_nx, grid_ny, grid_nt, _pad;
+    int32_t grid_nx, grid_ny, grid_nt;
+    int32_t settled;        /* read by stdadk_layer_fwd only (stdadk_fwd_args has no spare word): STDADK_SETTLED_STEP
+                               when the kernel launched just before this one does not write the dropout step counter,
+                               so a one-wave forward of block 2+ (a_img) forms its keep bits while that kernel
+                               still runs (same results) */
     int64_t row_begin;
     int64_t n_rows;
 } stdadk_points;
@@ -127,7 +131,8 @@ typedef struct {
     float* out_img_lo;       /* tf32x3: residual image of out_img (written together with it) */
 } stdadk_fwd_args;
 
-/* stdadk_bwd_args.settled: the dropout step counter (drop.step_ptr) / the saved x image and its stats */
+/* stdadk_points.settled (read by stdadk_layer_fwd) / stdadk_bwd_args.settled: the dropout step counter (drop.step_ptr)
+ * / the saved x image and its stats (backward only) */
 #define STDADK_SETTLED_STEP 1
 #define STDADK_SETTLED_X 2
 

@@ -18,7 +18,7 @@ CALIBRATION = {"wendland": 1.0, "gaussian": 0.223477, "triangular": 0.654714}
 fp = C.c_void_p  # device pointers travel as integers
 
 
-SETTLED_STEP, SETTLED_X = 1, 2       # stdadk_bwd_args.settled bits (STDADK_SETTLED_*)
+SETTLED_STEP, SETTLED_X = 1, 2       # stdadk_points / stdadk_bwd_args.settled bits (STDADK_SETTLED_*)
 
 
 class Basis(C.Structure):
@@ -28,7 +28,7 @@ class Basis(C.Structure):
 
 class Points(C.Structure):
     _fields_ = [("coords", fp), ("t", fp), ("xcov", fp), ("index", fp), ("grid_nx", C.c_int32), ("grid_ny", C.c_int32),
-                ("grid_nt", C.c_int32), ("_pad", C.c_int32), ("row_begin", C.c_int64), ("n_rows", C.c_int64)]
+                ("grid_nt", C.c_int32), ("settled", C.c_int32), ("row_begin", C.c_int64), ("n_rows", C.c_int64)]
 
 
 class Layer(C.Structure):

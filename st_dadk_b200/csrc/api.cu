@@ -287,14 +287,18 @@ static int check_layer(const stdadk_layer& l, const char* who) {
 constexpr uint32_t SMEM_LIMIT = 227 * 1024;
 constexpr int BWD_CG = 2, BWD_NS = 4;
 // cg = 4 (latency configuration, 4 stages) or 2 (two CTAs per SM, 2 stages); tab_chunks = k_slabs * 8 with a basis
+static SmemPlan fwd_plan(int n_pad, int q, int k_s, int k_t, int tab_chunks, int cg) {
+    return plan_smem(n_pad, q, k_s, k_t, false, cg, cg == 2 ? 2 : 4, tab_chunks);
+}
 static uint32_t fwd_smem(int n_pad, int q, int k_s, int k_t, int tab_chunks, int cg) {
-    return plan_smem(n_pad, q, k_s, k_t, false, cg, cg == 2 ? 2 : 4, tab_chunks).total;
+    return fwd_plan(n_pad, q, k_s, k_t, tab_chunks, cg).total;
 }
 static uint32_t bwd_smem(int n_pad, int q, int k_s, int k_t, int tab_chunks) {
     return plan_smem(n_pad, q, k_s, k_t, true, BWD_CG, BWD_NS, tab_chunks).total;
 }
 
 static unsigned long long* g_predict_dbg = nullptr;   // stdadk_debug_counters (profiling builds)
+static unsigned long long* g_step_dbg = nullptr;      // stdadk_debug_step_counters (profiling builds)
 int stdadk_layer_fwd(const stdadk_fwd_args* a, void* stream) {
     if (int r = check_device()) return r;
     REQUIRE(a, "layer_fwd: NULL args");
@@ -333,7 +337,7 @@ int stdadk_layer_fwd(const stdadk_fwd_args* a, void* stream) {
     K.addend = a->addend;
     K.x_img = a->x_img;
     K.feat_img = a->basis ? a->feat_img : nullptr;
-    K.dbg = g_predict_dbg;
+    K.dbg = g_step_dbg ? (a->layer.layer_id < 4 ? g_step_dbg + 64 + 16 * a->layer.layer_id : nullptr) : g_predict_dbg;
     K.out_img = a->out_img;
     K.stats = a->stats;
     K.has_head = a->head ? 1 : 0;
@@ -354,10 +358,20 @@ int stdadk_layer_fwd(const stdadk_fwd_args* a, void* stream) {
     if (half_tiles) tiles *= 2;
     K.tmem_cols = half_tiles ? tmem_cols_m64(K.n_pad) : pow2_cols(K.n_pad);
     // 1 CTA/SM in the latency configuration: spend the shared memory on pipeline depth (4 stages, else 2)
-    const uint32_t smem = fwd_smem(K.n_pad, K.has_head ? K.head.q : 0, basis ? K.basis.k_s : 0, basis ? K.basis.k_t : 0,
-                                   basis ? K.k_slabs * 8 : 0, cg);
+    const SmemPlan plan = fwd_plan(K.n_pad, K.has_head ? K.head.q : 0, basis ? K.basis.k_s : 0,
+                                   basis ? K.basis.k_t : 0, basis ? K.k_slabs * 8 : 0, cg);
+    uint32_t smem = plan.total;
     REQUIRE(smem <= SMEM_LIMIT, "layer_fwd: needs %u B of shared memory (> 227 KB): too many knots for the dense path",
             smem);
+    // Keep bits before the wait: blocks 2+ on one-wave tiles, dropout on, a settled step counter, and room for them.
+    // Not block 1: its predecessor, pack_images, has ended by the time block 1's workers reach the wait, so the early
+    // Philox calls (2.9 us per CTA) lengthened the chain by more than they took off the epilogue (1.4 us; B200, batch
+    // 4,096, tools/prof_step_phases.py).
+    if (!basis && half_tiles && a->drop.p > 0.0f && (a->pts.settled & STDADK_SETTLED_STEP) &&
+        smem + fwd_keep_bytes(K.n_pad) <= SMEM_LIMIT) {
+        K.keep_off = plan.keep_off;
+        smem += fwd_keep_bytes(K.n_pad);
+    }
     K.n_tiles = tiles;
 #define LAUNCH_FWD(B, TM, C)                                                                                 \
     do {                                                                                                     \
@@ -380,11 +394,10 @@ int stdadk_layer_fwd(const stdadk_fwd_args* a, void* stream) {
 // Development aid (not part of include/stdadk.h): 16 device counters of cycles the fused prediction kernel's roles spend
 // waiting; see tools/prof_predict.py.
 extern "C" void stdadk_debug_counters(void* dev_u64x16) { g_predict_dbg = static_cast<unsigned long long*>(dev_u64x16); }
-// Phase stamps of the training step (STEP_T, profiling builds): 8 counters per kernel, layer_bwd of layer l at 8 l
-// (l < 7), the fused tail at 56.  Launches read the pointer when they are made, so a graph keeps the one it was
-// captured with.
-static unsigned long long* g_step_dbg = nullptr;
-extern "C" void stdadk_debug_step_counters(void* dev_u64x64) { g_step_dbg = static_cast<unsigned long long*>(dev_u64x64); }
+// Phase stamps of the training step (profiling builds), 128 counters: STEP_T's 8 per kernel for layer_bwd of layer l
+// at 8 l (l < 7) and the fused tail at 56; FWD_T's 16 for layer_fwd of layer l at 64 + 16 l (l < 4).  Launches read
+// the pointer when they are made, so a graph keeps the one it was captured with.
+extern "C" void stdadk_debug_step_counters(void* dev_u64x128) { g_step_dbg = static_cast<unsigned long long*>(dev_u64x128); }
 
 // The hidden blocks of the whole-network kernels: each block's n_in must be the previous block's n_out.
 static int fill_pred_layers(const stdadk_layer* layers, int n_layers, PredLayerP* out, const char* who) {

@@ -80,7 +80,8 @@ __device__ __forceinline__ void colsum_chunk(float* cs, int c0, bool cvalid, flo
 
 // ---------------------------------------------------------------- shared-memory carve-up
 struct SmemPlan {
-    uint32_t a_off, b_off, bar_off, tmem_off, vec_off, headw_off, knots_off, tknots_off, colsum_off, red_off, total;
+    uint32_t a_off, b_off, bar_off, tmem_off, vec_off, headw_off, knots_off, tknots_off, colsum_off, red_off, keep_off,
+        total;
 };
 // tab_chunks > 0 (forward kernel of block 1): the knot tables are the chunk-indexed SoA tables of gen_basis_slab_soa
 // (64 bytes per 4-feature chunk) instead of the knots4 / tknots2 copies.
@@ -101,6 +102,7 @@ __host__ __device__ inline SmemPlan plan_smem(int n_pad, int q, int k_s, int k_t
     s.colsum_off = o; o += bwd ? (uint32_t)((3 + q) * n_pad + STDADK_MAX_Q) * 4u : 0u;
     s.red_off = s.a_off;   // epilogue scratch reuses the operand stages, which are dead once the last MMA committed
     (void)cg;
+    s.keep_off = o;        // layer_fwd's keep bits (fwd_keep_bytes), when the launch has them, go last
     s.total = o + 1024;                                   // slack for manual 1024-byte alignment
     return s;
 }
@@ -122,10 +124,19 @@ struct FwdK {
     unsigned int thresh16;
     float drop_scale;
     int n_tiles, passes;        // passes: 1 (TF32) or 3 (tf32x3)
-    unsigned long long* dbg;    // optional phase timers of -DSTDADK_PF_DEBUG builds (stdadk_debug_counters), else NULL
+    uint32_t keep_off;          // blocks 2+ at TM = 64, dropout, a settled step counter: offset of the keep bits
+                                // formed before the wait (fwd_keep_bytes at sp.keep_off), else 0
+    unsigned long long* dbg;    // optional phase timers of -DSTDADK_PF_DEBUG builds (stdadk_debug_counters, or in a
+                                // training step stdadk_debug_step_counters), else NULL
 };
+// Keep bits that the one-wave forward of block 2+ (TM = 64, CG = 4) forms before its wait: one word per worker thread
+// and chunk of its column loop, in shared memory behind the rest of the plan (sp.keep_off)
+__host__ __device__ constexpr uint32_t fwd_keep_bytes(int n_pad) {
+    return (uint32_t)n_work(4) * 4u * (uint32_t)((n_pad + 4 * 64 - 1) / (4 * 64));
+}
 // Development aid: globaltimer nanoseconds between the phases of a tile's life, summed over CTAs by one worker thread
-// (dbg[0..7] phase sums, dbg[8] = CTAs).  Production builds carry none of it.
+// (dbg[0..4] and dbg[9..10] phase sums, dbg[5..7] waits of single threads, dbg[8] = CTAs).  Production builds carry
+// none of it.
 #ifdef STDADK_PF_DEBUG
 #define FWD_T(slot)                                                       \
     do {                                                                  \
@@ -688,7 +699,9 @@ struct EpiCtx {
     long long lrow, grow;
     bool rvalid, tile_valid;
 };
-template <int CG, int TM>
+// EARLY: the kernel form that may have formed the keep bits before the wait (P.keep_off).  They are found from the
+// kernel parameter rather than a pointer, which would hold two registers across pass 1.
+template <int CG, int TM, bool EARLY>
 __device__ __forceinline__ void fwd_epilogue(const FwdK& P, const EpiCtx& E) {
     using G = TileGeo<TM>;
     constexpr int NW = n_work(CG), NG = G::groups(CG), WSTEP = G::WARP_COLS * CG;
@@ -760,15 +773,22 @@ __device__ __forceinline__ void fwd_epilogue(const FwdK& P, const EpiCtx& E) {
 #pragma unroll
     for (int k = 0; k < STDADK_MAX_Q; ++k) yh[k] = 0.0f;
     const bool drop = P.L.drop_p > 0.0f;
-    const unsigned int drop_step = drop ? dropout_step(P.L) : 0u;
+    const bool keep_early = EARLY && P.keep_off != 0;
+    const unsigned int drop_step = (drop && !keep_early) ? dropout_step(P.L) : 0u;
     // pass 2: x -> LayerNorm -> ReLU -> dropout -> operand image (+ head partials, + x image for the backward)
-    for (int wc = G::WARP_COLS * cg; wc < n_pad; wc += WSTEP) {
+    int ch = 0;
+    for (int wc = G::WARP_COLS * cg; wc < n_pad; wc += WSTEP, ++ch) {
         const int c0 = wc + coff;
         const bool cvalid = TM == 128 || c0 < n_pad;
         uint32_t keep = 0xFFFFFFFFu;
-        if (drop && cvalid)   // masks first: the Philox calls neither sit behind the TMEM load nor hold 32 live values
-            keep = pf_keep_mask(P.L.seed, drop_step, (uint32_t)P.L.layer_id, P.L.key_offset + (unsigned long long)lrow, c0,
-                                P.thresh16);
+        if (drop && cvalid) {  // masks first: the Philox calls neither sit behind the TMEM load nor hold 32 live values
+            if (keep_early) {
+                extern __shared__ uint8_t smem_raw[];
+                keep = reinterpret_cast<const uint32_t*>(align_smem(smem_raw) + P.keep_off)[ch * NW + (int)threadIdx.x];
+            }
+            else keep = pf_keep_mask(P.L.seed, drop_step, (uint32_t)P.L.layer_id, P.L.key_offset + (unsigned long long)lrow,
+                                     c0, P.thresh16);
+        }
         acc_ld<TM>(trow + wc, v);
         if (arow) add_addend_chunk(v, arow, c0, n_out);
 #pragma unroll
@@ -951,14 +971,31 @@ __global__ void __launch_bounds__(n_threads(CG), CG <= 2 ? 2 : 1) layer_fwd_kern
         __syncwarp();
     } else {
         // ---------------- workers: thread = (row, column group)
-        // The points may have been written by the launch just before this one (a prediction call's inputs), the
-        // addend by the support walk just before block 1, and the epilogue writes global memory: wait first.
-        pdl_wait();
         const int q4 = warp & 3, cg = warp >> 2;
         const int row = G::row(q4, lane), grp = G::group(cg, lane);     // grp: the thread's 8 / NG chunks of each slab
         const long long lrow = (long long)tile * TM + row;
         const bool rvalid = tile_valid && lrow < P.pts.n_rows;
         const long long grow = P.pts.row_begin + lrow;
+        // A one-wave training forward of block 2+ whose dropout step counter is settled (the previous step's tail
+        // advanced it; ptx.cuh, rule 2) forms the keep bits of the thread's chunks here, while the previous launch still
+        // runs, and parks them in shared memory for pass 2 of the epilogue: held in registers across the LayerNorm pass
+        // they spill.  Block 1 (api.cu says why) and the 128-row forms keep the Philox calls in pass 2.
+        if (!BASIS && TM == 64 && P.keep_off) {
+            uint32_t* kw = reinterpret_cast<uint32_t*>(smem + P.keep_off) + tid;
+            const unsigned int step = dropout_step(P.L);
+            int ch = 0;
+            for (int wc = G::WARP_COLS * cg; wc < n_pad; wc += G::WARP_COLS * CG, ++ch) {
+                const int c0 = wc + G::chunk_off(lane);
+                if (c0 < n_pad)
+                    kw[ch * NW] = pf_keep_mask(P.L.seed, step, (uint32_t)P.L.layer_id,
+                                               P.L.key_offset + (unsigned long long)lrow, c0, P.thresh16);
+            }
+        }
+        FWD_T(9);   // work before the wait
+        // The points may have been written by the launch just before this one (a prediction call's inputs), the
+        // addend by the support walk just before block 1, and the epilogue writes global memory: wait first.
+        pdl_wait();
+        FWD_T(10);  // wait for the previous launch
         if (BASIS) {
             float x = 0.f, y = 0.f, t = 0.f;
             const float* xrow = nullptr;
@@ -1003,7 +1040,7 @@ __global__ void __launch_bounds__(n_threads(CG), CG <= 2 ? 2 : 1) layer_fwd_kern
         FWD_T(2);   // wait for the accumulator
         EpiCtx E{sbias, sgam, sbet, shw, shb, red, tmem_base + ((uint32_t)(q4 * 32) << 16), itile, row, irow0 + row, cg, lane,
                  lrow, grow, rvalid, tile_valid};
-        fwd_epilogue<CG, TM>(P, E);
+        fwd_epilogue<CG, TM, !BASIS && TM == 64>(P, E);
         tc_fence_before();
         FWD_T(3);   // epilogue
     }

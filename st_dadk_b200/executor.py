@@ -137,8 +137,8 @@ class Executor:
         self._knots_ready = False
         self._side = None
         self.fused_predict = True      # forward-only calls use the whole-network kernel when the shape fits
-        # the one-wave backward and the fused step tail read settled inputs (dropout step, saved x images, optimizer
-        # state) before their programmatic-launch wait; STDADK_PREWAIT=0 makes them read everything after it (same
+        # the one-wave training forward and backward and the fused step tail read settled inputs (dropout step, saved x
+        # images, optimizer state) before their programmatic-launch wait; STDADK_PREWAIT=0 makes them read everything after it (same
         # results, for comparison)
         self.prewait = os.environ.get("STDADK_PREWAIT", "1") != "0"
         self._fused_ok = None
@@ -350,6 +350,8 @@ class Executor:
         for l in range(s.n_hidden):
             a = L.FwdArgs()
             a.pts = pts
+            if train and self.prewait:      # the step counter advances in the previous step's tail
+                a.pts.settled = L.SETTLED_STEP
             if l == 0:
                 a.basis = C.pointer(basis)
                 if self.sparse:

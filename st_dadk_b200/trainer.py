@@ -171,9 +171,14 @@ class Trainer:
         m = self.model
         self.learnable = bool(m.spatial_basis.learnable)
         self.q = m.output_dim
-        # static effective-head buffers (delta parameterisation recomputes them each step)
-        self.head_w = torch.empty(self.q, m.last_hidden_dim, device=self.device)
-        self.head_b = torch.empty(self.q, device=self.device)
+        # Effective head the kernels read.  The Linear head is read straight from its parameters, which live (Q, d)
+        # row-major in the flat buffer and are only ever rewritten in place (AdamW, the EMA swap).  The delta
+        # parameterisation has static buffers that _refresh_head recomputes each step.
+        if m.delta_params is not None:
+            self.head_w = torch.empty(self.q, m.last_hidden_dim, device=self.device)
+            self.head_b = torch.empty(self.q, device=self.device)
+        else:
+            self.head_w, self.head_b = m.mlp[-1].weight.detach(), m.mlp[-1].bias.detach()
         self.ex = Executor(self._spec())
         self.ex.loss_acc = self.flat.loss_slot      # the loss accumulator travels with the gradient all-reduce
         # captured graphs hold raw pointers into the executor's workspaces: drop them when one is evicted
@@ -214,14 +219,11 @@ class Trainer:
 
     def _refresh_head(self):
         m = self.model
-        with torch.no_grad():
-            if m.delta_params is not None:
+        if m.delta_params is not None:
+            with torch.no_grad():
                 beta = torch.cumsum(torch.stack([d.detach() for d in m.delta_params]), dim=0)
                 self.head_w.copy_(beta[:, 1:])
                 self.head_b.copy_(beta[:, 0])
-            else:
-                self.head_w.copy_(m.mlp[-1].weight.detach())
-                self.head_b.copy_(m.mlp[-1].bias.detach())
 
     def _init_loss(self):
         c = self.cfg

@@ -29,4 +29,5 @@ if os.environ.get("FWD_DBG"):
     names = ["prologue", "generate operand (+ stage waits)", "wait accumulator", "epilogue", "tail (barrier, dealloc)"]
     print("CTAs", v[8], "mean ns per CTA:", {k: round(v[i] / n_cta) for i, k in enumerate(names)}, "sum", round(sum(v[:5]) / n_cta),
           "| worker thread 0 waiting for a free stage:", round(v[5] / n_cta), " MMA thread waiting for operands:", round(v[6] / n_cta),
-          " producer waiting for a free stage:", round(v[7] / n_cta))
+          " producer waiting for a free stage:", round(v[7] / n_cta), "| before / in the launch wait:", round(v[9] / n_cta),
+          round(v[10] / n_cta))

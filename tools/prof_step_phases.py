@@ -1,8 +1,10 @@
 #!/usr/bin/env python
-"""Where the time of the training step's backward kernels and fused tail goes after their programmatic-launch wait.
+"""Where the time of the training step's forward and backward kernels and fused tail goes around their
+programmatic-launch wait.
 
-Needs the profiling build (tools/build_dbg.sh) through STDADK_LIB=st_dadk_b200/libstdadk_dbg.so: its layer_bwd and
-adamw_ema kernels stamp globaltimer phases (STEP_T in common.cuh) into stdadk_debug_step_counters.  Two trainers of the
+Needs the profiling build (tools/build_dbg.sh) through STDADK_LIB=st_dadk_b200/libstdadk_dbg.so: its layer_fwd
+(FWD_T in layer.cuh), layer_bwd and adamw_ema kernels (STEP_T in common.cuh) stamp globaltimer phases into
+stdadk_debug_step_counters.  Two trainers of the
 bench workload (bench.py's model, data and batch), one that reads settled inputs before the wait (Executor.prewait,
 the default) and one that reads everything after it (the order of the parent commit), replay their captured steps
 alternately, L2 flushed between steps as in the bench.  Printed: mean ns per CTA and step of each phase, per kernel.
@@ -18,6 +20,8 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tools"))
 
+# layer_fwd's counters in phase order (slot, name); slot 8 counts the CTAs
+FWD = [(0, "prologue"), (9, "before wait"), (10, "wait"), (1, "operand"), (2, "accumulator"), (3, "epilogue"), (4, "tail")]
 BWD = ["prologue", "before wait", "wait", "accumulator", "pass A", "pass B + flush"]
 TAIL = ["early loads", "wait", "g + norm partials", "grid barrier", "update"]
 
@@ -37,7 +41,7 @@ def main():
     flush = torch.empty(256 * 1024 * 1024 // 4, dtype=torch.float32, device=dev)
     runs = {}
     for mode in ("after wait", "before wait"):
-        cnt = torch.zeros(64, dtype=torch.int64, device=dev)
+        cnt = torch.zeros(128, dtype=torch.int64, device=dev)
         L.lib().stdadk_debug_step_counters(ctypes.c_void_p(cnt.data_ptr()))   # captured into the graph
         os.environ["STDADK_PREWAIT"] = "1" if mode == "before wait" else "0"
         step = build_trainer(bench.BATCH, "tf32", dev)
@@ -59,6 +63,12 @@ def main():
     for mode, (_, cnt) in runs.items():
         v = cnt.cpu().tolist()
         lines.append(f"-- inputs read {mode}")
+        for l in range(4):
+            c = v[64 + 16 * l + 8]
+            if c:
+                ph = [v[64 + 16 * l + k] / c for k, _ in FWD]
+                lines.append(f"  layer_fwd block {l + 1:d}: " + ", ".join(f"{n} {x:.0f}" for (_, n), x in zip(FWD, ph)) +
+                             f" | after wait {sum(ph[3:]):.0f}")
         for l in range(7):
             c = v[8 * l + 7]
             if c:
