@@ -651,7 +651,10 @@ class Executor:
                 side.wait_stream(main)
                 with torch.cuda.stream(side):
                     self._wgrad_block(l, pts, ws, basis, g)
-        main.wait_stream(side)      # join: every weight gradient is complete before the caller continues
+        if nh > 1:
+            # join: every weight gradient is complete before the caller continues.  With one hidden block the side stream
+            # ran nothing, and inside a graph capture a wait on it would depend on work outside the capture.
+            main.wait_stream(side)
         if s.learnable_basis and not self.sparse:
             a = L.KnotGradArgs()
             a.basis = C.pointer(basis)

@@ -13,6 +13,7 @@ Replaces the upstream Python loop `train_model` / `evaluate_model` (scripts/trai
 """
 from __future__ import annotations
 
+import gc
 import math
 import os
 import warnings
@@ -473,6 +474,9 @@ class Trainer:
                 # Captures are serialised across the threads of a process (several configurations train concurrently on
                 # separate streams of one GPU, scripts/run_grid_search.py) and use thread-local capture mode, so what
                 # the other threads enqueue meanwhile neither enters nor invalidates this capture.
+                # The cyclic garbage collector stays off while this thread captures.  Trainers sit in reference
+                # cycles, so the graphs of an abandoned one are freed whenever the collector happens to run; freeing a
+                # graph is not permitted while the same thread captures, and it invalidates the capture.
                 with _CAPTURE_LOCK:
                     self._step_body(table, self._stage_idx, 0, n_rows, global_rows, key_offset)
                     torch.cuda.current_stream().synchronize()
@@ -480,18 +484,24 @@ class Trainer:
                     # Data parallel: the peer-memory exchange is a plain kernel and is captured with the rest of the
                     # step; an NCCL all-reduce stays between two graphs (the collective outside stream capture).
                     one_graph = self.world == 1 or self._peer is not None
-                    if one_graph:
-                        g1 = torch.cuda.CUDAGraph()
-                        with torch.cuda.graph(g1, **mode):
-                            self._step_body(table, self._stage_idx, 0, n_rows, global_rows, key_offset)
-                        g = (g1, None)
-                    else:
-                        g1, g2 = torch.cuda.CUDAGraph(), torch.cuda.CUDAGraph()
-                        with torch.cuda.graph(g1, **mode):
-                            self._step_compute(table, self._stage_idx, 0, n_rows, global_rows, key_offset)
-                        with torch.cuda.graph(g2, **mode):
-                            self._step_update()
-                        g = (g1, g2)
+                    gc_on = gc.isenabled()          # read under the lock: no other capture has switched it off
+                    gc.disable()
+                    try:
+                        if one_graph:
+                            g1 = torch.cuda.CUDAGraph()
+                            with torch.cuda.graph(g1, **mode):
+                                self._step_body(table, self._stage_idx, 0, n_rows, global_rows, key_offset)
+                            g = (g1, None)
+                        else:
+                            g1, g2 = torch.cuda.CUDAGraph(), torch.cuda.CUDAGraph()
+                            with torch.cuda.graph(g1, **mode):
+                                self._step_compute(table, self._stage_idx, 0, n_rows, global_rows, key_offset)
+                            with torch.cuda.graph(g2, **mode):
+                                self._step_update()
+                            g = (g1, g2)
+                    finally:
+                        if gc_on:
+                            gc.enable()
                 self._graphs[gkey] = g
             else:
                 g[0].replay()

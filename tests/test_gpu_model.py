@@ -281,6 +281,42 @@ def test_step_tail_bookkeeping_gradient_zeroing_and_loss_sum():
     assert np.allclose(l0, l2, rtol=2e-3) and close(p0, p2)
 
 
+def test_step_capture_runs_no_garbage_collection():
+    """Freeing a CUDA graph while the same thread captures another invalidates that capture.  Trainers sit in reference
+    cycles, so the graphs of an abandoned trainer are freed whenever the cyclic garbage collector runs: the trainer keeps
+    the collector off while it captures.  With a collection threshold of 1 nearly every allocation starts a collection;
+    none may start while the stream captures, and the captured step replays."""
+    import gc
+    from stnf.models import STInterpMLP
+    from stnf.dataio import ObservationTable
+    from st_dadk_b200.trainer import Trainer
+    rng = np.random.default_rng(6)
+    n, B = 2048, 1024
+    c, t = rng.random((n, 2)).astype(np.float32), rng.random(n).astype(np.float32)
+    table = ObservationTable(torch.from_numpy(c), torch.from_numpy(t), torch.from_numpy(t.copy())).to(DEV)
+    perm = torch.arange(n, device=DEV)
+    cfg = dict(lr=1e-3, weight_decay=0.0, regression_type="mean")
+    capturing = []
+
+    def seen(phase, info):
+        if phase == "start":
+            capturing.append(torch.cuda.is_current_stream_capturing())
+
+    threshold = gc.get_threshold()
+    gc.callbacks.append(seen)
+    try:
+        gc.set_threshold(1)
+        tr = Trainer(STInterpMLP(hidden_dims=[64, 32]), cfg, DEV, batches_per_epoch=2, use_cuda_graph=True)
+        for s in range(4):
+            tr.train_step(table, perm, (s % 2) * B, B)
+        torch.cuda.synchronize()
+    finally:
+        gc.set_threshold(*threshold)
+        gc.callbacks.remove(seen)
+    assert len(tr._graphs) == 1 and np.isfinite(float(tr.loss_last.item()))
+    assert capturing and not any(capturing), f"{sum(capturing)} of {len(capturing)} collections started during capture"
+
+
 def test_host_buffer_step_sync_and_lagged_match_device_step():
     """Trainer.train_step_host (pinned host batch -> H2D -> step -> D2H loss, double-buffered staging): the
     synchronous form returns each step's loss, the lagged form the previous step's (then flush); both equal the

@@ -60,7 +60,7 @@ class Net:
 
     @property
     def q(self):
-        return self.m.weights[-1].shape[0]
+        return len(self.m.delta) if self.m.delta is not None else self.m.weights[-1].shape[0]
 
     def nc_power(self, regime):
         # N2 takes the linear penalty in the one regime of its own (its row count is not shared with another regime)
@@ -185,10 +185,16 @@ def test_chunked_oracle_matches_whole_batch():
 _ORACLE = {}
 
 
-def oracle(name, n, regime):
-    """FP64 and TF32-emulating oracle results of network `name` on the batch of n rows, shared by both precisions."""
-    nt = net(name)
-    key = (name, n, nt.nc_power(regime))
+def _as_net(nt):
+    """A Net, or the name of one in the net() registry."""
+    return net(nt) if isinstance(nt, str) else nt
+
+
+def oracle(nt, n, regime):
+    """FP64 and TF32-emulating oracle results of network `nt` (a Net or a registry name) on the batch of n rows, shared
+    by both precisions."""
+    nt = _as_net(nt)
+    key = (nt, n, nt.nc_power(regime))
     if key not in _ORACLE:
         coords, t, y, X, perm = table(n, nt.m.p)
         idx = perm[ROW_BEGIN:ROW_BEGIN + n]
@@ -200,10 +206,11 @@ def oracle(name, n, regime):
 
 
 # ---------------------------------------------------------------------------------------------------- one step
-def train_step(name, n, regime, precision="tf32"):
-    """forward(train, save) + backward of network `name` on n gathered rows; returns (executor, yhat, loss, grads)."""
+def train_step(nt, n, regime, precision="tf32"):
+    """forward(train, save) + backward of network `nt` (a Net or a registry name) on n gathered rows; returns
+    (executor, yhat, loss, grads)."""
     L, ops, Executor, NetSpec, LossSpec = _mods()
-    nt = net(name)
+    nt = _as_net(nt)
     spec = spec_from_oracle(nt.m, learnable=nt.learnable, dropout=nt.m.dropout, precision=precision)
     if nt.sizes is not None:
         spec.level_sizes = nt.sizes
@@ -232,7 +239,12 @@ def _grad_pairs(grads, ref, nt):
         if nt.m.ln_gamma[l] is not None:
             out += [(f"dgamma{l}", grads["gammas"][l], ref["ln_gamma"][l]),
                     (f"dbeta{l}", grads["betas"][l], ref["ln_beta"][l])]
-    out += [("dhead_w", grads["head_w"], ref["weights"][-1]), ("dhead_b", grads["head_b"], ref["biases"][-1])]
+    if nt.m.delta is not None:
+        # the kernels give the effective head's gradient; d delta_l = sum_{k >= l} [d head_b | d head_w]_k
+        dbeta = np.concatenate([grads["head_b"][:, None], grads["head_w"]], axis=1)
+        out.append(("ddelta", np.cumsum(dbeta[::-1], axis=0)[::-1], np.stack(ref["delta"])))
+    else:
+        out += [("dhead_w", grads["head_w"], ref["weights"][-1]), ("dhead_b", grads["head_b"], ref["biases"][-1])]
     if nt.learnable:
         out += [("dcenters", grads["centers"], ref["centers"]),
                 ("dlog_bw", grads["log_bandwidths"], ref["log_bandwidths"])]

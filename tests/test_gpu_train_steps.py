@@ -192,11 +192,15 @@ def test_train_steps_vs_oracle_at_matched_weights(name):
     3e-4 of the step (at most 0.62 of these bounds).  Negative control: the masks of steps 0 and 2 miss step 1 by
     2.3e-4 / 2.7e-3 in the loss and 5.1e-2 / 4.4e-2 in the gradients.  The clip is engaged on 4 of A's 8 steps (from
     step 0) and on none of C's and D's."""
+    run_case(name, _cases()[name])
+
+
+def run_case(name, cs):
+    """Run the Trainer through every step of Case `cs` and check each step against the oracle (module docstring)."""
     from stnf.dataio import ObservationTable
     from stnf.models import STInterpMLP
     from st_dadk_b200.trainer import Trainer
 
-    cs = _cases()[name]
     x3 = cs.cfg.get("precision", "tf32x3") == "tf32x3"
     cfg = dict(cs.cfg, precision="tf32x3" if x3 else "tf32")
     sizes = [b for ep in cs.batches for b in ep]
