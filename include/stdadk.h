@@ -64,6 +64,13 @@ typedef struct {
     int64_t n_rows;
 } stdadk_points;
 
+/* Widest hidden block (n_out) of the per-block entry points (stdadk_layer_fwd / _bwd, stdadk_wgrad, stdadk_knot_grad,
+ * stdadk_sparse_l1_*, stdadk_dense_*): a block's LayerNorm needs its whole row in one CTA, whose FP32 accumulator takes
+ * one of the 512 tensor-memory columns of an SM per output unit.  A block wider than 256 runs in the wide forms of the
+ * block kernels; stdadk_layer_bwd then needs the x image of its forward (x_img).  The whole-network and field kernels
+ * take blocks of at most 256. */
+#define STDADK_MAX_WIDTH 512
+
 /* One hidden block Linear -> LayerNorm -> ReLU -> Dropout (st_interp.py:659-666). */
 typedef struct {
     const float* w_img;  /* image of W (n_out x n_in), K-major forward operand */
@@ -301,7 +308,8 @@ int stdadk_sparse_l1_wgrad(const stdadk_sparse_args* a, void* stream);
  * train_st_interp.py:884-961, :1233-1248, :1380-1394; STInterpMLP.forward in eval mode, st_interp.py:827-882):
  * basis -> hidden blocks -> head in ONE persistent kernel; activations stay in shared / tensor memory, the only
  * per-point HBM traffic is the point (12 B, or 0 for a generated grid) and y_hat (4Q B).  Dropout is the identity.
- * Limits: 1..STDADK_MAX_HIDDEN hidden blocks of width <= 256, dense basis (all knots resident in shared memory);
+ * Limits: 1..STDADK_MAX_HIDDEN hidden blocks of width <= 256 (not STDADK_MAX_WIDTH: the kernel's weight ring and
+ * tensor-memory halves are laid out for 256), dense basis (all knots resident in shared memory);
  * stdadk_predict_supported() tells whether a shape fits, otherwise chain stdadk_layer_fwd calls. */
 #define STDADK_MAX_HIDDEN 4
 typedef struct {

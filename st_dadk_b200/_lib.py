@@ -8,6 +8,8 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 # STDADK_LIB: an alternative build of the same library (e.g. the -DSTDADK_PF_DEBUG profiling build of tools/)
 LIB_PATH = os.environ.get("STDADK_LIB") or os.path.join(_HERE, "libstdadk.so")
 MAX_Q = 8
+MAX_WIDTH = 512          # STDADK_MAX_WIDTH: widest hidden block of the per-block kernels
+MAX_N = 256              # widest block of the whole-network and field kernels; wider blocks run the wide block kernels
 
 WENDLAND, GAUSSIAN, TRIANGULAR = 0, 1, 2
 LOSS_NONE, LOSS_MSE, LOSS_PINBALL = 0, 1, 2

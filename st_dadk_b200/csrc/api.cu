@@ -273,8 +273,8 @@ int stdadk_unpack_image(const float* img, int64_t rows, int64_t cols, float* dst
 
 static int check_layer(const stdadk_layer& l, const char* who) {
     REQUIRE(l.w_img && l.bias, "%s: weight image / bias is NULL", who);
-    REQUIRE(l.n_out >= 1 && l.n_out <= MAX_N, "%s: n_out=%d outside [1,%d] (one UMMA N / LayerNorm row per thread)", who,
-            l.n_out, MAX_N);
+    REQUIRE(l.n_out >= 1 && l.n_out <= MAX_W, "%s: n_out=%d outside [1,%d] (one LayerNorm row per CTA, one tensor-memory "
+            "column per output)", who, l.n_out, MAX_W);
     REQUIRE(l.n_in >= 1, "%s: n_in=%d", who, l.n_in);
     REQUIRE((l.gamma == nullptr) == (l.beta == nullptr), "%s: gamma and beta must both be given or both NULL", who);
     REQUIRE(((reinterpret_cast<uintptr_t>(l.w_img) | reinterpret_cast<uintptr_t>(l.w_img_lo)) & 127) == 0,
@@ -286,15 +286,18 @@ static int check_layer(const stdadk_layer& l, const char* who) {
 // these same functions (and wgrad_smem_bytes), so the executor's regime choice and the launch checks cannot disagree.
 constexpr uint32_t SMEM_LIMIT = 227 * 1024;
 constexpr int BWD_CG = 2, BWD_NS = 4;
+// A block wider than MAX_N runs the wide forms: layer_fwd_kernel<B, TM, 4, 2> and layer_bwd_kernel<false, TM, 2, 2, ...>
+// (x-image backward only), 2 stages each.
+static bool wide(int n_pad) { return n_pad > MAX_N; }
 // cg = 4 (latency configuration, 4 stages) or 2 (two CTAs per SM, 2 stages); tab_chunks = k_slabs * 8 with a basis
 static SmemPlan fwd_plan(int n_pad, int q, int k_s, int k_t, int tab_chunks, int cg) {
-    return plan_smem(n_pad, q, k_s, k_t, false, cg, cg == 2 ? 2 : 4, tab_chunks);
+    return plan_smem(n_pad, q, k_s, k_t, false, cg, (cg == 2 || wide(n_pad)) ? 2 : 4, tab_chunks);
 }
 static uint32_t fwd_smem(int n_pad, int q, int k_s, int k_t, int tab_chunks, int cg) {
     return fwd_plan(n_pad, q, k_s, k_t, tab_chunks, cg).total;
 }
 static uint32_t bwd_smem(int n_pad, int q, int k_s, int k_t, int tab_chunks) {
-    return plan_smem(n_pad, q, k_s, k_t, true, BWD_CG, BWD_NS, tab_chunks).total;
+    return plan_smem(n_pad, q, k_s, k_t, true, BWD_CG, wide(n_pad) ? 2 : BWD_NS, tab_chunks).total;
 }
 
 static unsigned long long* g_predict_dbg = nullptr;   // stdadk_debug_counters (profiling builds)
@@ -350,7 +353,8 @@ int stdadk_layer_fwd(const stdadk_fwd_args* a, void* stream) {
     // few tiles (a training batch): 16 worker warps per CTA hide the latency of the serial phases; many tiles
     // (dense prediction): 8 worker warps and two CTAs per SM so one tile's epilogue overlaps the other's MMAs
     const int sms = g_sm_count > 0 ? g_sm_count : 148;
-    const int cg = tiles >= 2 * sms ? 2 : 4;
+    const bool wd = wide(K.n_pad);       // one CTA per SM at any batch: the 4-group configuration
+    const int cg = tiles >= 2 * sms && !wd ? 2 : 4;
     // a batch that fits in one wave of 64-row tiles runs on twice the SMs, each walking half the rows.  Both halves of
     // every 128-row image tile get a CTA, so the padding rows of the last tile are written (zeros) as on the 128-row
     // path: wgrad and the knot gradient read whole 128-row tiles.
@@ -378,7 +382,17 @@ int stdadk_layer_fwd(const stdadk_fwd_args* a, void* stream) {
         if (int r = set_smem(layer_fwd_kernel<B, TM, C, (C == 2 ? 2 : 4)>, smem)) return r;                  \
         launch_chained(layer_fwd_kernel<B, TM, C, (C == 2 ? 2 : 4)>, dim3(tiles), n_threads(C), smem, stream, K); \
     } while (0)
-    if (basis) {
+#define LAUNCH_FWD_WIDE(B, TM)                                                                               \
+    do {                                                                                                     \
+        if (int r = set_smem(layer_fwd_kernel<B, TM, 4, 2>, smem)) return r;                                 \
+        launch_chained(layer_fwd_kernel<B, TM, 4, 2>, dim3(tiles), n_threads(4), smem, stream, K);          \
+    } while (0)
+    if (wd) {
+        if (basis && half_tiles) LAUNCH_FWD_WIDE(true, 64);
+        else if (basis) LAUNCH_FWD_WIDE(true, 128);
+        else if (half_tiles) LAUNCH_FWD_WIDE(false, 64);
+        else LAUNCH_FWD_WIDE(false, 128);
+    } else if (basis) {
         if (half_tiles) LAUNCH_FWD(true, 64, 4);
         else if (cg == 2) LAUNCH_FWD(true, 128, 2);
         else LAUNCH_FWD(true, 128, 4);
@@ -388,6 +402,7 @@ int stdadk_layer_fwd(const stdadk_fwd_args* a, void* stream) {
         else LAUNCH_FWD(false, 128, 4);
     }
 #undef LAUNCH_FWD
+#undef LAUNCH_FWD_WIDE
     return check_launch("layer_fwd");
 }
 
@@ -404,6 +419,8 @@ static int fill_pred_layers(const stdadk_layer* layers, int n_layers, PredLayerP
     for (int l = 0; l < n_layers; ++l) {
         const stdadk_layer& y = layers[l];
         if (int r = check_layer(y, who)) return r;
+        REQUIRE(y.n_out <= MAX_N, "%s: block %d of width %d: the whole-network kernels take blocks of at most %d (chain "
+                "stdadk_layer_fwd calls)", who, l, y.n_out, MAX_N);
         REQUIRE(l == 0 || y.n_in == layers[l - 1].n_out, "%s: block %d n_in=%d != previous n_out=%d", who, l, y.n_in,
                 layers[l - 1].n_out);
         PredLayerP& L = out[l];
@@ -568,7 +585,7 @@ int stdadk_layer_bwd(const stdadk_bwd_args* a, void* stream) {
                     a->d_head_b,
                 "layer_bwd: head arguments incomplete");
     } else {
-        REQUIRE(a->wt_next_img && a->n_next >= 1 && a->n_next <= MAX_N, "layer_bwd: wt_next_img / n_next invalid");
+        REQUIRE(a->wt_next_img && a->n_next >= 1 && a->n_next <= MAX_W, "layer_bwd: wt_next_img / n_next invalid");
     }
     const bool x3 = a->layer.w_img_lo != nullptr;
     if (x3) {
@@ -576,6 +593,9 @@ int stdadk_layer_bwd(const stdadk_bwd_args* a, void* stream) {
         REQUIRE(a->head || (a->dz_next_img_lo && a->wt_next_img_lo), "layer_bwd: tf32x3 needs dz_next_img_lo / wt_next_img_lo");
         REQUIRE(a->dz_img_lo, "layer_bwd: tf32x3 needs dz_img_lo");
     }
+    const bool wd = wide(pad32(a->layer.n_out));
+    REQUIRE(!wd || a->x_img, "layer_bwd: a block wider than %d needs the forward's x_img (its backward has no recompute GEMM)",
+            MAX_N);
     if (a->pts.n_rows <= 0) return 0;
     BwdK K{};
     K.basis = to_basis(a->basis);
@@ -620,14 +640,32 @@ int stdadk_layer_bwd(const stdadk_bwd_args* a, void* stream) {
     const int sms = g_sm_count > 0 ? g_sm_count : 148;
     const bool half_tiles = a->x_img && 2 * tiles <= sms;
     if (half_tiles) tiles *= 2;
-    K.tmem_cols = 2 * (half_tiles ? tmem_cols_m64(K.n_pad) : pow2_cols(K.n_pad));
+    // narrow: recompute accumulator and dh in two halves; wide: dh alone, at column 0
+    K.tmem_cols = (wd ? 1 : 2) * (half_tiles ? tmem_cols_m64(K.n_pad) : pow2_cols(K.n_pad));
     const bool ln = a->layer.gamma != nullptr, hd = a->head != nullptr;
 #define LAUNCH_BWD(B, TM, LNV, HD)                                                                          \
     do {                                                                                                    \
         if (int r = set_smem(layer_bwd_kernel<B, TM, BCG, BNS, LNV, HD>, smem)) return r;                   \
         launch_chained(layer_bwd_kernel<B, TM, BCG, BNS, LNV, HD>, dim3(tiles), n_threads(BCG), smem, stream, K); \
     } while (0)
-    if (half_tiles) {
+#define LAUNCH_BWD_WIDE(TM, LNV, HD)                                                                            \
+    do {                                                                                                        \
+        if (int r = set_smem(layer_bwd_kernel<false, TM, BCG, 2, LNV, HD>, smem)) return r;                     \
+        launch_chained(layer_bwd_kernel<false, TM, BCG, 2, LNV, HD>, dim3(tiles), n_threads(BCG), smem, stream, K); \
+    } while (0)
+    if (wd) {
+        if (half_tiles) {
+            if (ln && hd) LAUNCH_BWD_WIDE(64, true, true);
+            else if (ln) LAUNCH_BWD_WIDE(64, true, false);
+            else if (hd) LAUNCH_BWD_WIDE(64, false, true);
+            else LAUNCH_BWD_WIDE(64, false, false);
+        } else {
+            if (ln && hd) LAUNCH_BWD_WIDE(128, true, true);
+            else if (ln) LAUNCH_BWD_WIDE(128, true, false);
+            else if (hd) LAUNCH_BWD_WIDE(128, false, true);
+            else LAUNCH_BWD_WIDE(128, false, false);
+        }
+    } else if (half_tiles) {
         if (ln && hd) LAUNCH_BWD(false, 64, true, true);
         else if (ln) LAUNCH_BWD(false, 64, true, false);
         else if (hd) LAUNCH_BWD(false, 64, false, true);
@@ -644,6 +682,7 @@ int stdadk_layer_bwd(const stdadk_bwd_args* a, void* stream) {
         else LAUNCH_BWD(false, 128, false, false);
     }
 #undef LAUNCH_BWD
+#undef LAUNCH_BWD_WIDE
     return check_launch("layer_bwd");
 }
 
@@ -652,7 +691,7 @@ int stdadk_wgrad(const stdadk_wgrad_args* a, void* stream) {
     REQUIRE(a, "wgrad: NULL args");
     REQUIRE((a->basis != nullptr) != (a->a_img != nullptr), "wgrad: give exactly one of basis / a_img");
     REQUIRE(a->dz_img && a->dw, "wgrad: dz_img / dw NULL");
-    REQUIRE(a->n_out >= 1 && a->n_out <= MAX_N && a->n_in >= 1, "wgrad: bad sizes n_in=%d n_out=%d", a->n_in, a->n_out);
+    REQUIRE(a->n_out >= 1 && a->n_out <= MAX_W && a->n_in >= 1, "wgrad: bad sizes n_in=%d n_out=%d", a->n_in, a->n_out);
     if (a->basis)
         if (int r = check_basis_points(a->basis, a->pts, a->n_in)) return r;
     if (a->pts.n_rows <= 0) return 0;
@@ -699,18 +738,20 @@ int stdadk_wgrad(const stdadk_wgrad_args* a, void* stream) {
 }
 
 // The block-1 launches of the dense path: layer_fwd in both CTA configurations (every forward), and with `training`
-// also layer_bwd regenerating the basis (batches the forward saves no x for) and the basis-form wgrad.
+// also layer_bwd regenerating the basis (batches the forward saves no x for) and the basis-form wgrad.  A wide block 1
+// has one forward configuration, and its backward reads the x image at every batch size (no knot tables).
 static int dense_basis_check(int n_in, int n_out, int k_s, int k_t, int q_head, int training) {
-    REQUIRE(n_out >= 1 && n_out <= MAX_N && k_s >= 0 && k_t >= 0 && n_in >= k_s + k_t && q_head >= 0 &&
+    REQUIRE(n_out >= 1 && n_out <= MAX_W && k_s >= 0 && k_t >= 0 && n_in >= k_s + k_t && q_head >= 0 &&
                 q_head <= STDADK_MAX_Q,
             "dense_basis_supported: bad sizes n_in=%d n_out=%d k_s=%d k_t=%d q_head=%d", n_in, n_out, k_s, k_t, q_head);
     const int n_pad = pad32(n_out), tab_chunks = pad32(n_in) / SLAB_K * 8;
     for (int cg : {4, 2}) {
+        if (cg == 2 && wide(n_pad)) continue;
         const uint32_t b = fwd_smem(n_pad, q_head, k_s, k_t, tab_chunks, cg);
         REQUIRE(b <= SMEM_LIMIT, "layer_fwd: needs %u B of shared memory (> 227 KB): too many knots for the dense path", b);
     }
     if (!training) return 0;
-    const uint32_t bb = bwd_smem(n_pad, q_head, k_s, k_t, tab_chunks);
+    const uint32_t bb = wide(n_pad) ? bwd_smem(n_pad, q_head, 0, 0, 0) : bwd_smem(n_pad, q_head, k_s, k_t, tab_chunks);
     REQUIRE(bb <= SMEM_LIMIT, "layer_bwd: needs %u B of shared memory (> 227 KB)", bb);
     const uint32_t wb = wgrad_smem_bytes(k_s, k_t);
     REQUIRE(wb <= SMEM_LIMIT, "wgrad: needs %u B of shared memory (> 227 KB)", wb);
@@ -738,7 +779,7 @@ int stdadk_knot_grad(const stdadk_knotgrad_args* a, void* stream) {
     if (int r = check_device()) return r;
     REQUIRE(a && a->basis && a->dz_img && a->w1s_img && a->d_centers && a->d_log_bw, "knot_grad: NULL argument");
     if (int r = check_basis_points(a->basis, a->pts, -1)) return r;
-    REQUIRE(a->n_out >= 1 && a->n_out <= MAX_N, "knot_grad: n_out=%d", a->n_out);
+    REQUIRE(a->n_out >= 1 && a->n_out <= MAX_W, "knot_grad: n_out=%d", a->n_out);
     if (a->pts.n_rows <= 0 || a->basis->k_s == 0) return 0;
     KnotGradK K{};
     K.basis = to_basis(a->basis);
@@ -766,8 +807,8 @@ static int sparse_fill(const stdadk_sparse_args* a, SparseK* K, bool wgrad) {
             a->n_levels);
     REQUIRE(a->basis_fn == STDADK_WENDLAND || a->basis_fn == STDADK_TRIANGULAR,
             "sparse_l1: only compactly supported bases can be walked (the gaussian basis is dense)");
-    REQUIRE(a->n_out >= 4 && a->n_out <= MAX_N && a->n_out % 4 == 0, "sparse_l1: n_out=%d must be a multiple of 4 <= %d",
-            a->n_out, MAX_N);
+    REQUIRE(a->n_out >= 4 && a->n_out <= MAX_W && a->n_out % 4 == 0, "sparse_l1: n_out=%d must be a multiple of 4 <= %d",
+            a->n_out, MAX_W);
     REQUIRE(a->knots4, "sparse_l1: knots4 is NULL");
     REQUIRE(a->pts.grid_nx > 0 || a->pts.coords != nullptr, "sparse_l1: no point source");
     REQUIRE(a->pts.grid_nx > 0 || (reinterpret_cast<uintptr_t>(a->pts.coords) & 7) == 0, "sparse_l1: coords alignment");
@@ -879,7 +920,8 @@ int stdadk_sparse_l1_fwd(const stdadk_sparse_args* a, void* stream) {
     if (int r = sparse_fill(a, &K, false)) return r;
     if (a->pts.n_rows <= 0) return 0;
     int blocks = grid_for(a->pts.n_rows, SP_WARPS, 8);
-    sparse_spatial_fwd_kernel<<<blocks, SP_WARPS * 32, 0, (cudaStream_t)stream>>>(K);
+    if (a->n_out > MAX_N) sparse_spatial_fwd_wide_kernel<<<blocks, SP_WARPS * 32, 0, (cudaStream_t)stream>>>(K);
+    else sparse_spatial_fwd_kernel<<<blocks, SP_WARPS * 32, 0, (cudaStream_t)stream>>>(K);
     return check_launch("sparse_l1_fwd");
 }
 
@@ -889,7 +931,8 @@ int stdadk_sparse_l1_wgrad(const stdadk_sparse_args* a, void* stream) {
     if (int r = sparse_fill(a, &K, true)) return r;
     if (a->pts.n_rows <= 0) return 0;
     int blocks = grid_for(a->pts.n_rows, SP_WARPS, 8);
-    sparse_spatial_wgrad_kernel<<<blocks, SP_WARPS * 32, 0, (cudaStream_t)stream>>>(K);
+    if (a->n_out > MAX_N) sparse_spatial_wgrad_wide_kernel<<<blocks, SP_WARPS * 32, 0, (cudaStream_t)stream>>>(K);
+    else sparse_spatial_wgrad_kernel<<<blocks, SP_WARPS * 32, 0, (cudaStream_t)stream>>>(K);
     return check_launch("sparse_l1_wgrad");
 }
 

@@ -37,7 +37,11 @@ constexpr int TILE_M = 128;                  // rows (points) per tile = TMEM la
 constexpr int SLAB_K = 32;                   // fp32/tf32 elements per 128-byte operand row
 constexpr int SLAB_FLOATS = TILE_M * SLAB_K; // 4096 floats = 16 KB
 constexpr int SLAB_BYTES = SLAB_FLOATS * 4;
-constexpr int MAX_N = 256;                   // widest hidden layer (one UMMA N, one LayerNorm row per thread)
+constexpr int MAX_N = 256;                   // widest block of the whole-network and field kernels (one UMMA N); layout
+                                             // constant of their weight ring and tensor-memory halves
+constexpr int MAX_W = STDADK_MAX_WIDTH;      // widest block of the per-block kernels: one FP32 accumulator column per
+                                             // output unit in the 512 tensor-memory columns of an SM
+static_assert(MAX_W == 2 * MAX_N, "a wide block is two MMAs of N <= MAX_N per K slab");
 
 __host__ __device__ inline int pad32(int x) { return (x + 31) & ~31; }
 __host__ __device__ inline int64_t ceil_div64(int64_t a, int64_t b) { return (a + b - 1) / b; }

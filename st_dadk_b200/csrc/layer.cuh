@@ -18,6 +18,8 @@
 // take alternate 32-column chunks, so thread = (row, 1/(2 CG) of the columns).  Then one producer warp (bulk copies)
 // and one MMA issuer warp (one elected thread).  CG = 4 for latency (few tiles), CG = 2 with two CTAs per SM for
 // throughput.  TM = 64 is for batches that fit in one wave of 64-row tiles: twice the SMs, half the rows per CTA.
+// Blocks wider than MAX_N (up to MAX_W) run the wide forms, CG = 4 with 2 stages forward and 2 stages backward: two
+// MMAs per K slab fill one accumulator of up to 512 tensor-memory columns.
 #pragma once
 #include "common.cuh"
 
@@ -848,9 +850,15 @@ __device__ __forceinline__ void fwd_epilogue(const FwdK& P, const EpiCtx& E) {
     }
 }
 
+// The wide form, CG = 4 with NS = 2 (MAX_N < n_pad <= MAX_W; 2 stages of up to 80 KB, one CTA per SM by its shared
+// memory and by its tensor memory, all 512 columns at width 512): one UMMA takes N <= MAX_N, so every K slab is two
+// MMAs, B rows [0, MAX_N) into accumulator columns [0, MAX_N) and the rest into [MAX_N, n_pad).  The accumulator is then
+// the same n_pad contiguous columns the epilogue reads at any width.  The narrow forms are <CG = 4, NS = 4> and
+// <CG = 2, NS = 2>.
 template <bool BASIS, int TM, int CG, int NS>
 __global__ void __launch_bounds__(n_threads(CG), CG <= 2 ? 2 : 1) layer_fwd_kernel(const __grid_constant__ FwdK P) {
     using G = TileGeo<TM>;
+    constexpr bool WIDE = CG == 4 && NS == 2;
     constexpr int NW = n_work(CG), NT = n_threads(CG), NSTAGE = NS, NG = G::groups(CG);
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = align_smem(smem_raw);
@@ -956,7 +964,8 @@ __global__ void __launch_bounds__(n_threads(CG), CG <= 2 ? 2 : 1) layer_fwd_kern
     } else if (warp == 4 * CG + 1) {
         // ---------------- MMA issuer
         if (lane == 0) {
-            const uint32_t idesc = umma_idesc_tf32((uint32_t)n_pad, 0, 0, TM);
+            const uint32_t idesc = umma_idesc_tf32((uint32_t)(WIDE ? MAX_N : n_pad), 0, 0, TM);
+            const uint32_t idesc_hi = WIDE ? umma_idesc_tf32((uint32_t)(n_pad - MAX_N), 0, 0, TM) : 0u;
             const int n_virt = P.k_slabs * P.passes;
             for (int s = 0; s < n_virt; ++s) {
                 int stage = s % NSTAGE, it = s / NSTAGE;
@@ -964,6 +973,9 @@ __global__ void __launch_bounds__(n_threads(CG), CG <= 2 ? 2 : 1) layer_fwd_kern
                 tc_fence_after();
                 issue_slab_mma(tmem_base, sA + (size_t)stage * SLAB_FLOATS, sB + stage * b_stage_floats, idesc,
                                s == 0);
+                if (WIDE)
+                    issue_slab_mma(tmem_base + MAX_N, sA + (size_t)stage * SLAB_FLOATS,
+                                   sB + stage * b_stage_floats + (size_t)MAX_N * SLAB_K, idesc_hi, s == 0);
                 umma_commit(&empty[stage]);
             }
             umma_commit(accf);
@@ -1072,12 +1084,16 @@ __device__ __forceinline__ void head_dh_chunk(float (&g)[32], const float (&dyh)
 // =============================================================================================
 // LN / HEAD are compile-time so that each instantiation carries only its own epilogue: the generic kernel was
 // 150 KB of SASS and a one-wave launch (32 tiles) spent ~30% of its stall samples on instruction fetch.
+// The wide form, NS = 2 (MAX_N < n_pad <= MAX_W; the narrow form has NS = 4): x comes from the forward's image only (no
+// recompute GEMM, BASIS is false), so the dh accumulator starts at column 0 and spans up to MAX_W columns, two MMAs per
+// K slab as in the wide forward.  There is no free half of tensor memory for x^: x_early stays off.
 template <bool BASIS, int TM, int CG, int NS, bool LN, bool HEAD>
 __global__ void __launch_bounds__(n_threads(CG), 1) layer_bwd_kernel(const __grid_constant__ BwdK P) {
     using G = TileGeo<TM>;
+    constexpr bool WIDE = NS == 2;
     constexpr int NW = n_work(CG), NT = n_threads(CG), NSTAGE = NS, NG = G::groups(CG);
     constexpr int WSTEP = G::WARP_COLS * CG;
-    constexpr int MAXCH = MAX_N / WSTEP;            // column chunks per thread
+    constexpr int MAXCH = (WIDE ? MAX_W : MAX_N) / WSTEP;   // column chunks per thread
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = align_smem(smem_raw);
     const int q = HEAD ? P.head.q : 0;
@@ -1110,7 +1126,7 @@ __global__ void __launch_bounds__(n_threads(CG), 1) layer_bwd_kernel(const __gri
     const size_t b_stage_floats = (size_t)n_pad * SLAB_K;
     const int virt1 = P.k_slabs * P.passes;                 // GEMM 1 (recompute), then GEMM 2 (dgrad): virtual slabs
     const int total_slabs = virt1 + P.k_slabs2 * P.passes;
-    const uint32_t acc1_off = (uint32_t)(P.tmem_cols / 2);
+    const uint32_t acc1_off = WIDE ? 0u : (uint32_t)(P.tmem_cols / 2);
 
     if (tid == NW) {
         for (int s = 0; s < NSTAGE; ++s) {
@@ -1184,7 +1200,8 @@ __global__ void __launch_bounds__(n_threads(CG), 1) layer_bwd_kernel(const __gri
         __syncwarp();
     } else if (warp == 4 * CG + 1) {
         if (lane == 0) {
-            const uint32_t idesc = umma_idesc_tf32((uint32_t)n_pad, 0, 0, TM);
+            const uint32_t idesc = umma_idesc_tf32((uint32_t)(WIDE ? MAX_N : n_pad), 0, 0, TM);
+            const uint32_t idesc_hi = WIDE ? umma_idesc_tf32((uint32_t)(n_pad - MAX_N), 0, 0, TM) : 0u;
             for (int s = 0; s < total_slabs; ++s) {
                 int stage = s % NSTAGE, it = s / NSTAGE;
                 mbar_wait(&full[stage], it & 1);
@@ -1192,6 +1209,9 @@ __global__ void __launch_bounds__(n_threads(CG), 1) layer_bwd_kernel(const __gri
                 bool second = s >= virt1;
                 issue_slab_mma(tmem_base + (second ? acc1_off : 0u), sA + (size_t)stage * SLAB_FLOATS,
                                sB + stage * b_stage_floats, idesc, s == 0 || s == virt1);
+                if (WIDE)
+                    issue_slab_mma(tmem_base + MAX_N, sA + (size_t)stage * SLAB_FLOATS,
+                                   sB + stage * b_stage_floats + (size_t)MAX_N * SLAB_K, idesc_hi, s == 0);
                 umma_commit(&empty[stage]);
             }
             umma_commit(accf);
@@ -1254,7 +1274,7 @@ __global__ void __launch_bounds__(n_threads(CG), 1) layer_bwd_kernel(const __gri
         // activation bits.  x^ goes to the half of tensor memory that the recompute GEMM would use (an x-image backward
         // has none): the warp's chunk at column wc sits in columns wc / 2 .. +31, one 32x32b lane per thread, so the
         // epilogue reads it back with one tcgen05.ld instead of two dependent trips to L2.
-        constexpr bool X_EARLY_OK = TM == 64 && !HEAD;
+        constexpr bool X_EARLY_OK = TM == 64 && !HEAD && !WIDE;
         const bool keeps_early = P.step_settled != 0;
         const bool x_early = X_EARLY_OK && keeps_early && P.x_settled != 0;
         if (keeps_early) chunk_keep_masks<TM, CG, MAXCH>(P.L, P.thresh16, lrow, cg, lane, n_pad, actbits);
@@ -1314,7 +1334,7 @@ __global__ void __launch_bounds__(n_threads(CG), 1) layer_bwd_kernel(const __gri
             const bool cvalid = TM == 128 || c0 < n_pad;
             if (x_early) {
                 tmem_ld32(trow + (uint32_t)(wc / 2), z);       // x^
-            } else if (P.x_img) {
+            } else if (WIDE || P.x_img) {
                 if (cvalid) image_load_chunk(P.x_img, itile, n_pad / SLAB_K, c0, (uint32_t)irow, z);    // x saved by the forward
             } else {
                 acc_ld<TM>(trow + wc, z);
@@ -1415,7 +1435,7 @@ __global__ void __launch_bounds__(n_threads(CG), 1) layer_bwd_kernel(const __gri
                 const bool cvalid = TM == 128 || c0 < n_pad;
                 if (x_early) {
                     tmem_ld32(trow + (uint32_t)(wc / 2), z);   // x^
-                } else if (P.x_img) {
+                } else if (WIDE || P.x_img) {
                     if (cvalid) image_load_chunk(P.x_img, itile, n_pad / SLAB_K, c0, (uint32_t)irow, z);
                 } else {
                     acc_ld<TM>(trow + wc, z);

@@ -71,6 +71,13 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
 //     one-wave backward's keep bits, x^ and activation bits, the keep bits of the one-wave forward of blocks 2+ and the
 //     tail's state are formed or loaded before the wait.
 //  3. A grid-wide barrier (the fused step tail) sits after the wait, where the prerequisites have exited.
+// Tensor memory: a CTA of a block wider than MAX_N (as a 256-wide recompute backward) holds all 512 columns of its SM,
+// so an early CTA of the next kernel, or a wgrad CTA of the side stream, that lands on that SM blocks in tcgen05.alloc
+// until the wide CTA exits.  This cannot deadlock.  The CTA that holds columns waits only on kernels launched before it
+// (pdl_wait) and on its own pipeline, never on a later launch, so it runs to its end and frees them; by rule 1 every CTA
+// of the previous kernel has its columns before a dependent CTA can ask for any.  And shared memory bounds what is
+// resident beside a wide CTA (two stages of its weight slabs: over 100 KB), while launch_chained starts a grid early only when the grid
+// has at most one CTA per SM: at most one early CTA waits on an SM.
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 

@@ -304,4 +304,86 @@ __global__ void __launch_bounds__(SP_WARPS * 32) sparse_spatial_wgrad_kernel(con
     }
 }
 
+// Blocks 1 wider than MAX_N (up to MAX_W outputs): the columns of a row are LANE_SETS = 4 float4 groups per lane,
+// lane + 32 k, where the kernels above take two.  Kept apart from them so that their code stays as it is.
+template <int LANE_SETS>
+__device__ __forceinline__ void sparse_fwd_rows(const SparseK& P) {
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const long long n_warps = (long long)gridDim.x * SP_WARPS;
+    const int ngroups = P.n_out >> 2;
+    for (long long r = (long long)blockIdx.x * SP_WARPS + warp; r < P.pts.n_rows; r += n_warps) {
+        float x, y, t;
+        load_point(P.pts, P.pts.row_begin + r, x, y, t);
+        float4 acc[LANE_SETS];
+#pragma unroll
+        for (int k = 0; k < LANE_SETS; ++k) acc[k] = make_float4(0.f, 0.f, 0.f, 0.f);
+        sparse_for_each_active(P, x, y, lane, [&](int j, float f, float, float, float, float) {
+            const float4* row = reinterpret_cast<const float4*>(P.w1t + (size_t)(P.p_cov + j) * P.n_out);
+#pragma unroll
+            for (int k = 0; k < LANE_SETS; ++k)
+                if (lane + 32 * k < ngroups) {
+                    float4 w = __ldg(row + lane + 32 * k);
+                    acc[k].x = fmaf(f, w.x, acc[k].x); acc[k].y = fmaf(f, w.y, acc[k].y);
+                    acc[k].z = fmaf(f, w.z, acc[k].z); acc[k].w = fmaf(f, w.w, acc[k].w);
+                }
+        });
+        float4* out = reinterpret_cast<float4*>(P.zs + (size_t)r * P.n_out);
+#pragma unroll
+        for (int k = 0; k < LANE_SETS; ++k)
+            if (lane + 32 * k < ngroups) out[lane + 32 * k] = acc[k];
+    }
+}
+__global__ void __launch_bounds__(SP_WARPS * 32) sparse_spatial_fwd_wide_kernel(const __grid_constant__ SparseK P) {
+    sparse_fwd_rows<4>(P);
+}
+
+template <int LANE_SETS>
+__device__ __forceinline__ void sparse_wgrad_rows(const SparseK& P) {
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const long long n_warps = (long long)gridDim.x * SP_WARPS;
+    const int ngroups = P.n_out >> 2;
+    const int slabs = pad32(P.n_out) / SLAB_K;
+    const bool knot_grads = P.d_centers != nullptr;
+    for (long long r = (long long)blockIdx.x * SP_WARPS + warp; r < P.pts.n_rows; r += n_warps) {
+        float x, y, t;
+        load_point(P.pts, P.pts.row_begin + r, x, y, t);
+        float4 d[LANE_SETS];
+#pragma unroll
+        for (int k = 0; k < LANE_SETS; ++k)
+            d[k] = lane + 32 * k < ngroups ? image_load4(P.dz_img, slabs, r, lane + 32 * k) : make_float4(0.f, 0.f, 0.f, 0.f);
+        sparse_for_each_active(P, x, y, lane, [&](int j, float f, float dx, float dy, float d2, float inv_th) {
+            float4* row = reinterpret_cast<float4*>(P.dw1t + (size_t)(P.p_cov + j) * P.n_out);
+#pragma unroll
+            for (int k = 0; k < LANE_SETS; ++k)
+                if (lane + 32 * k < ngroups)
+                    atomicAdd(row + lane + 32 * k, make_float4(f * d[k].x, f * d[k].y, f * d[k].z, f * d[k].w));
+            if (knot_grads) {
+                // G = dz1[n, :] . W1t[p + j, :]; then dL/dc_j += G phi'(r) (-(s - c)/(d theta')), dL/dlog theta_j += G phi'(r) (-r)
+                const float4* wr = reinterpret_cast<const float4*>(P.w1t + (size_t)(P.p_cov + j) * P.n_out);
+                float g = 0.0f;
+#pragma unroll
+                for (int k = 0; k < LANE_SETS; ++k)
+                    if (lane + 32 * k < ngroups) {
+                        const float4 w = __ldg(wr + lane + 32 * k);
+                        const float gk = fmaf(d[k].x, w.x, fmaf(d[k].y, w.y, fmaf(d[k].z, w.z, d[k].w * w.w)));
+                        g = k == 0 ? gk : g + gk;
+                    }
+                g = warp_sum(g);
+                if (lane == 0 && d2 > 0.0f) {
+                    const float d = sqrtf(d2), rr = d * inv_th;
+                    const float coef = g * phi_dr(P.fn, rr);
+                    const float s = coef * inv_th / d;
+                    atomicAdd(&P.d_centers[2 * j], -dx * s);
+                    atomicAdd(&P.d_centers[2 * j + 1], -dy * s);
+                    atomicAdd(&P.d_log_bw[j], -rr * coef);
+                }
+            }
+        });
+    }
+}
+// at least two CTAs per SM, i.e. up to 128 registers: with the default bound ptxas held the kernel to 64 and spilled
+__global__ void __launch_bounds__(SP_WARPS * 32, 2) sparse_spatial_wgrad_wide_kernel(const __grid_constant__ SparseK P) {
+    sparse_wgrad_rows<4>(P);
+}
+
 }  // namespace stdadk

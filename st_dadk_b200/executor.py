@@ -78,8 +78,12 @@ class _Workspace:
         self.dz_lo = [ops.new_image(n_rows, w.shape[0], device) for w in spec.weights] if x3 else None
         self.stats = [torch.empty(n_rows, 2, dtype=torch.float32, device=device) if g is not None else None
                       for g in spec.gammas]
-        # pre-LayerNorm x of every block, kept only for single-wave batches (see Executor.SAVE_X_MAX_ROWS)
-        self.x = [ops.new_image(n_rows, w.shape[0], device) for w in spec.weights] if save_x else None
+        # pre-LayerNorm x per block: every block of a single-wave batch (see Executor.SAVE_X_MAX_ROWS), and a block wider
+        # than L.MAX_N at every batch size, as its backward has no recompute GEMM (2 KB/row at width 512).  None for a
+        # block that does not keep it, and as a whole when no block does.
+        keep = [save_x or w.shape[0] > L.MAX_N for w in spec.weights]
+        self.x = [ops.new_image(n_rows, w.shape[0], device) if k else None
+                  for w, k in zip(spec.weights, keep)] if any(keep) else None
         self.yhat = torch.empty(n_rows, spec.q, dtype=torch.float32, device=device)
         self.dyhat = torch.empty(n_rows, spec.q, dtype=torch.float32, device=device)
 
@@ -366,7 +370,7 @@ class Executor:
             a.drop = drop
             if save and ws.stats[l] is not None:
                 a.stats = ws.stats[l].data_ptr()
-            if save and ws.x is not None:
+            if save and ws.x is not None and ws.x[l] is not None:
                 a.x_img = ws.x[l].data_ptr()
             if l < s.n_hidden - 1:
                 a.out_img = ws.h[l].data_ptr()
@@ -614,7 +618,7 @@ class Executor:
                     a.a_img_lo = ws.h_lo[l - 1].data_ptr()
             a.layer = self._layer(l)
             a.drop = drop
-            if ws.x is not None:
+            if ws.x is not None and ws.x[l] is not None:
                 a.x_img = ws.x[l].data_ptr()
                 # The launch just before a backward is another backward (or, for the head, the last forward), and the
                 # dropout step counter advances in the previous step's tail.  Below the head x and stats come from the

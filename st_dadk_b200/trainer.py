@@ -182,8 +182,12 @@ class Trainer:
             self.head_w, self.head_b = m.mlp[-1].weight.detach(), m.mlp[-1].bias.detach()
         self.ex = Executor(self._spec())
         self.ex.loss_acc = self.flat.loss_slot      # the loss accumulator travels with the gradient all-reduce
-        # captured graphs hold raw pointers into the executor's workspaces: drop them when one is evicted
-        self.ex.on_evict = lambda: self._graphs.clear()
+        # Captured graphs hold raw pointers into the executor's workspaces: drop them when one is evicted.  The callback
+        # holds the graph dictionary, not the trainer: a trainer in a reference cycle with its executor is only freed
+        # when the cyclic garbage collector runs, and freeing its graphs then, inside another capture on this thread
+        # (a global-mode capture: any thread), invalidates that capture.
+        self._graphs: Dict[tuple, torch.cuda.CUDAGraph] = {}
+        self.ex.on_evict = self._graphs.clear
         self.ex.alloc_grads(self.flat.g, self.flat.grad_views_for(m))
         self._init_loss()
         self._init_optimizer(batches_per_epoch)
@@ -198,7 +202,6 @@ class Trainer:
         self.loss_last = torch.zeros(1, device=self.device)     # loss of the most recent step (written by AdamW)
         self._g_clean = False     # True while the flat gradient and loss_acc are known to be zero (left so by AdamW)
         self.use_cuda_graph = use_cuda_graph
-        self._graphs: Dict[tuple, torch.cuda.CUDAGraph] = {}
         self._stage_idx = None
         self._host_stage = None
         self._host_perm = None
@@ -474,9 +477,9 @@ class Trainer:
                 # Captures are serialised across the threads of a process (several configurations train concurrently on
                 # separate streams of one GPU, scripts/run_grid_search.py) and use thread-local capture mode, so what
                 # the other threads enqueue meanwhile neither enters nor invalidates this capture.
-                # The cyclic garbage collector stays off while this thread captures.  Trainers sit in reference
-                # cycles, so the graphs of an abandoned one are freed whenever the collector happens to run; freeing a
-                # graph is not permitted while the same thread captures, and it invalidates the capture.
+                # The cyclic garbage collector stays off while this thread captures.  Graphs held by any object in a
+                # reference cycle are freed whenever the collector happens to run; freeing a graph is not permitted
+                # while the same thread captures, and it invalidates the capture.
                 with _CAPTURE_LOCK:
                     self._step_body(table, self._stage_idx, 0, n_rows, global_rows, key_offset)
                     torch.cuda.current_stream().synchronize()

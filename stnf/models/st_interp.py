@@ -272,9 +272,9 @@ class STInterpMLP(nn.Module):
     def _executor(self, head_w=None, head_b=None):
         spec = self.net_spec(head_w, head_b)
         for hdim in self._hidden_dims:
-            if hdim > 256:
-                raise RuntimeError(f"hidden width {hdim} > 256 is not supported by the tcgen05 block kernel "
-                                   "(one UMMA N / one LayerNorm row per thread)")
+            if hdim > _L.MAX_WIDTH:
+                raise RuntimeError(f"hidden width {hdim} > {_L.MAX_WIDTH} is not supported by the tcgen05 block kernels "
+                                   f"(one LayerNorm row per CTA, one of the {_L.MAX_WIDTH} tensor-memory columns per unit)")
         if self._ex is None or self._ex.device != spec.centers.device:
             self._ex = Executor(spec)
         else:
